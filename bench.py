@@ -10,6 +10,7 @@ and -- for N > 1 -- the data-parallel gradient all-reduce over NCCL.  `value` = 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's sm_100a engine
     python bench.py --impl reference ...                            # the reference's CPU PyTorch path (oracle port)
     python bench.py --impl eager_gpu ...                            # informational: torch eager + cuDNN on the same GPU
+    python bench.py --dump-outputs DIR ...                          # also write the last timed step's loss and gradients
 
 Keys follow the driver contract: value (inputs resident in HBM), e2e (inputs copied from pinned host memory inside the
 timed region through the public nn.Module API, loss read back), roofline (dominant kernel, measured live with CUDA
@@ -24,6 +25,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -144,6 +146,27 @@ class ClockSampler:
                 "reasons": sorted(reasons)}
 
 
+DUMP_MAX_ELEMS = 1 << 18   # per gradient: the 3d_fullres UNet's 101 gradients come to ~20 MB in all
+
+
+def dump_outputs(out_dir: str, loss: torch.Tensor, named_params) -> None:
+    """Write what a training step hands its caller -- the loss and every parameter gradient -- as float32 `loss.npy` and
+    `grad.<parameter name>.npy`, so that two builds can be compared output for output.  A gradient of more than
+    DUMP_MAX_ELEMS elements is written flattened, as the same sorted sample of its elements on every run (a generator seeded
+    by the parameter's name)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    for name, p in named_params:
+        if p.grad is None:       # without deep supervision only the last seg layer reaches the loss
+            continue
+        g = p.grad.detach().float()
+        if g.numel() > DUMP_MAX_ELEMS:
+            idx = np.random.default_rng(zlib.crc32(name.encode())).choice(g.numel(), DUMP_MAX_ELEMS, replace=False)
+            g = g.reshape(-1)[torch.from_numpy(np.sort(idx)).to(g.device)]
+        np.save(os.path.join(out_dir, f"grad.{name}.npy"), g.cpu().numpy())
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # reference arm / cpu baseline: the oracle port of the reference's PlainConvUNet on the host cores
 # ----------------------------------------------------------------------------------------------------------------
@@ -227,15 +250,20 @@ def reference_arm(args) -> None:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the flagship workload (`value` and `e2e`); the extra configs time their own fixed counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "eager_gpu"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--no-extras", action="store_true", help="skip the C2-C5 / cuDNN-eager entries (bench_extras.py)")
+    ap.add_argument("--no-extras", action="store_true", help="skip the C2-C5 / cuDNN-eager entries (bench_extras.py, each timed over its own fixed count)")
     ap.add_argument("--launch", default="graph", choices=["graph", "eager"],
                     help="b200 arm: replay the step from one CUDA graph (rehrseg_b200.graphs.GraphedTrainStep) or launch it from Python")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and parameter gradients of the last one to DIR/*.npy (rank 0)")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU arms")
         return reference_arm(args)
 
     import torch.distributed as dist
@@ -349,7 +377,7 @@ def main() -> None:
         l0 = Fn.launches()
         e0.record()
         for _ in range(steps):
-            step_fn()
+            out = step_fn()
         e1.record()
         torch.cuda.synchronize()
         launches = Fn.launches() - l0
@@ -358,14 +386,16 @@ def main() -> None:
         if world > 1:
             dist.barrier()
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms), launches, clocks
+        return float(ms), launches, clocks, out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
     phys = int(os.environ.get("CUDA_VISIBLE_DEVICES", "").split(",")[local]) if os.environ.get("CUDA_VISIBLE_DEVICES") else local
-    ms, launches, clocks = timed(step_resident, args.steps, ClockSampler(phys) if rank == 0 else None)
+    ms, launches, clocks, loss = timed(step_resident, args.steps, ClockSampler(phys) if rank == 0 else None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model.named_parameters())
     step_e2e()
-    ms_e2e, _, _ = timed(step_e2e, args.steps)
+    ms_e2e, _, _, _ = timed(step_e2e, args.steps)
 
     # roofline of the dominant kernel: one instrumented step, CUDA events around every conv-engine launch
     roof = None

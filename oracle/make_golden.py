@@ -372,9 +372,50 @@ def stage2_sample_fixture() -> None:
     np.savez_compressed(os.path.join(OUT, "stage2_sample.npz"), **out)
 
 
+FBA_PS = ("infinity", "inf", 0.5, 2, "3")
+
+
+def reference_helpers_fixture() -> None:
+    """The reference's find_integer_p / projected_size / get_pads / compute_steps_for_sliding_window over the ranges
+    tests/test_oracle_vs_reference.py sweeps, and rotate_vol_2d / fba on its seeded arrays -> tests/golden/reference_helpers.json
+    + .npz, which that test compares against wherever no reference checkout is present.  The committed files were recorded
+    through the oracle restatements (oracle/volume.py), which the live comparison had found bit-identical to the reference
+    on every one of these inputs; with a checkout, this function records them from the reference itself."""
+    po, pad, su = refimport.load("utils.patch_ops"), refimport.load("utils.pad"), refimport.load("utils.seg_utils")
+    rot, fb = refimport.load("utils.rotate"), refimport.load("utils.fba")
+    cases = {"find_integer_p": [], "get_pads": [], "steps": []}
+    for n in range(1, 70):
+        for s in (1.0, 1.25, 1.5, 2.0, 2.4, 3.0, 3.2, 4.0, 4.5, 6.0):
+            cases["find_integer_p"].append([n, s, po.find_integer_p(n, s), po.projected_size(n, 3, s)])
+    for t in range(0, 40):
+        for d in range(0, 40):
+            cases["get_pads"].append([t, d, *pad.get_pads(t, d)])
+    rng = np.random.default_rng(0)
+    for _ in range(200):
+        tile = [int(v) for v in rng.integers(4, 40, 3)]
+        img = [t + int(v) for t, v in zip(tile, rng.integers(0, 90, 3))]
+        step = float(rng.choice([0.25, 0.5, 0.75, 1.0]))
+        cases["steps"].append([img, tile, step, su.compute_steps_for_sliding_window(img, tile, step)])
+    with open(os.path.join(OUT, "reference_helpers.json"), "w") as f:
+        json.dump(cases, f)
+    g = torch.Generator().manual_seed(3)
+    v = torch.randn((4, 6, 5), generator=g)
+    arrs = {"rot_in": v.numpy()}
+    for a in (0, 90, -90, 180, -180, 270, -270, 360):
+        arrs[f"rot_{a}"] = rot.rotate_vol_2d(v, a).contiguous().numpy()
+    vols = [torch.randn((8, 6, 10), generator=g).numpy() for _ in range(4)]
+    arrs["fba_in"] = np.stack(vols)
+    for p in FBA_PS:
+        arrs[f"fba_{p}"] = fb.fba(vols, p)
+    np.savez_compressed(os.path.join(OUT, "reference_helpers.npz"), **arrs)
+
+
 def main() -> None:
     os.makedirs(OUT, exist_ok=True)
     import sys
+    if "--only-helpers" in sys.argv:
+        reference_helpers_fixture()
+        return
     if "--only-stage2" in sys.argv:
         stage2_sample_fixture()
         return
@@ -516,6 +557,7 @@ def main() -> None:
     sr_degrade_fixture()
     spatial_aug_fixture()
     stage2_sample_fixture()
+    reference_helpers_fixture()
     print("golden fixtures written to", OUT, {k: os.path.getsize(os.path.join(OUT, k)) for k in sorted(os.listdir(OUT))})
 
 
