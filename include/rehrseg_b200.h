@@ -64,7 +64,9 @@ typedef enum { REHR_ACT_NONE = 0, REHR_ACT_RELU = 1, REHR_ACT_LRELU = 2 } rehr_a
 
 const char* rehr_strerror(int status);
 int rehr_last_cuda_error(void);     /* cudaError_t of the last failing CUDA call on this thread */
-int rehr_version(void);             /* ABI version, currently 5 (4: rehr_tensor.dtype, dtype arguments of the weight packers; 5: batched re-pack, *_dgrad_inred, *_bwd_finalize_raw added -- additive) */
+int rehr_version(void);             /* ABI version, currently 6 (4: rehr_tensor.dtype, dtype arguments of the weight packers; 5: batched
+                                     * re-pack and fused InstanceNorm-backward sums added -- additive; 6: the normalise-on-load and fused
+                                     * InstanceNorm-backward-sum entry points removed) */
 int rehr_device_sm_count(void);
 
 /* ------------------------------------------------------------------------------------------------
@@ -154,28 +156,6 @@ int rehr_pack_weight_march(const float* src, void* dst16, int cout, int cin, int
 int rehr_conv3d_march_stats_tiles(const rehr_tensor* x, const rehr_tensor* y, int ks);
 int rehr_conv3d_march_fwd(const rehr_tensor* x, const void* w_march, const float* bias, const rehr_tensor* y, int ks, int y_is_f32,
                           int act, float slope, float* stats, rehr_stream stream);
-/* "Normalise on load": x is the RAW (pre-InstanceNorm) conv output of the producing layer; extra warps rewrite every landed
- * input plane in shared memory as  operand = lrelu_c(x * scale[n,c] + shift[n,c])  before the MMA reads it, so the normalised
- * activation of ConvDropoutNormReLU (models/seg_model.py:174-191) never makes a round trip through HBM.  norm = f32
- * [n][3][cin] (scale, shift, slope rows; slope 1 = no activation) from rehr_instnorm_finalize_norm; op_dtype = 16-bit format the
- * operand is written in = format of the packed weights.  Supported for output-channel tiles <= 32 (..._norm_supported). */
-int rehr_conv3d_march_norm_supported(const rehr_conv_desc* desc, int cin, int cout);
-int rehr_conv3d_march_fwd_norm(const rehr_tensor* x, const float* norm, int op_dtype, const void* w_march, const float* bias,
-                               const rehr_tensor* y, int ks, int y_is_f32, int act, float slope, float* stats, rehr_stream stream);
-
-/* Input gradient of a stride-1 k3 marching layer whose INPUT is the activation of a Conv -> InstanceNorm -> LeakyReLU block
- * (ConvDropoutNormReLU, models/seg_model.py:174-191): besides dx = conv^T(dy) the epilogue accumulates that block's InstanceNorm
- * backward sums from the fp32 accumulators -- S1 = sum g, S2raw = sum g*y with g = (scale*y + shift > 0 ? 1 : slope) * dx, y_prod =
- * the block's pre-normalisation tensor (shape of dx), norm_prod = its f32 [n][3][c] (scale, shift, slope) table from
- * rehr_instnorm_finalize_norm -- into stats [n][rehr_conv3d_march_stats_tiles(dy, dx, ks)][c][2].  The block's stand-alone reduce
- * pass (rehr_instnorm_lrelu_bwd_reduce) is then not needed: rehr_instnorm_lrelu_bwd_finalize_raw converts the raw sums
- * (sum g*xhat = rstd * (sum g*y - mean * sum g)).  cin_dy / cout_dx: channels of dy / dx. */
-int rehr_conv3d_march_dgrad_inred_supported(const rehr_conv_desc* desc, int cin_dy, int cout_dx);
-int rehr_conv3d_march_dgrad_inred(const rehr_tensor* dy, const void* w_march, const rehr_tensor* dx, int ks, const rehr_tensor* y_prod,
-                                  const float* norm_prod, float* stats, rehr_stream stream);
-int rehr_instnorm_lrelu_bwd_finalize_raw(const float* partial, int n, int tiles, int c, const float* mean, const float* rstd,
-                                         float* sums, float* dgamma, float* dbeta, int accumulate, rehr_stream stream);
-
 /* Batched weight re-pack (csrc/pack_batch.cu).  Between rehr_pack_batch_begin() and rehr_pack_batch_launch() every
  * rehr_pack_weight / rehr_pack_weight_march / rehr_pack_weight_march_s2dgrad call ON THIS THREAD is recorded instead of launched;
  * rehr_pack_batch_launch issues all of them as ONE kernel (one per 128 recorded calls) whose job table travels in the kernel
@@ -206,9 +186,6 @@ int rehr_conv3d_wgrad_march_supported(const rehr_conv_desc* desc, const rehr_ten
 size_t rehr_conv3d_wgrad_march_workspace(const rehr_tensor* x, const rehr_tensor* dy, int ks);
 int rehr_conv3d_wgrad_march(const rehr_tensor* x, const rehr_tensor* dy, int ks, int cout, float* dw, int accumulate, void* ws,
                             size_t ws_bytes, rehr_stream stream);
-/* Same with x = the producer's RAW conv output (either 16-bit format) normalised on load to a bf16 operand (norm as above). */
-int rehr_conv3d_wgrad_march_norm(const rehr_tensor* x, const float* norm, const rehr_tensor* dy, int ks, int cout, float* dw,
-                                 int accumulate, void* ws, size_t ws_bytes, rehr_stream stream);
 
 /* Weight gradient of a k3 / pad 1 conv with strides in {1, 2}: one marching pass per parity class of X (a strided TMA view),
  * restricted to the 1-2 offsets per strided dimension that class contributes to; dw f32 [Cout][Cin][27]. */
@@ -216,8 +193,6 @@ int rehr_conv3d_wgrad_march_s2_supported(const rehr_conv_desc* desc, const rehr_
 size_t rehr_conv3d_wgrad_march_s2_workspace(const rehr_conv_desc* desc, const rehr_tensor* x, const rehr_tensor* dy);
 int rehr_conv3d_wgrad_march_s2(const rehr_conv_desc* desc, const rehr_tensor* x, const rehr_tensor* dy, float* dw, int accumulate,
                                void* ws, size_t ws_bytes, rehr_stream stream);
-int rehr_conv3d_wgrad_march_s2_norm(const rehr_conv_desc* desc, const rehr_tensor* x, const float* norm, const rehr_tensor* dy,
-                                    float* dw, int accumulate, void* ws, size_t ws_bytes, rehr_stream stream);
 
 /* Direct convolution for tiny input-channel counts (Cin <= 4: the 1-channel nnU-Net stem, the 2-channel
  * FLAVR stem k(3,7,7)); x is NCDHW f32 exactly as the caller hands it (train_all.py:524), y NDHWC bf16.
@@ -244,16 +219,6 @@ int rehr_instnorm_stats(const rehr_tensor* x, float* partial, rehr_stream stream
 /* partial [n][tiles][c][2] -> mean[n][c], rstd[n][c] (biased variance, double accumulation). */
 int rehr_instnorm_finalize(const float* partial, int n, int tiles, int c, long long count, float eps,
                            float* mean, float* rstd, rehr_stream stream);
-/* rehr_instnorm_finalize that also emits the normalise-on-load triples of this InstanceNorm + LeakyReLU:
- *   norm[(n*3 + 0)*c_total + c_off + c] = gamma*rstd, [(n*3 + 1)..] = beta - mean*gamma*rstd, [(n*3 + 2)..] = slope;
- * channels [0, c_off) are set to the identity (1, 0, 1) -- the up-sampled half of a decoder concat buffer [up | skip].
- * norm_own (optional): the same triples again as a dense [n][3][c] table, for consumers of this tensor alone. */
-int rehr_instnorm_finalize_norm(const float* partial, int n, int tiles, int c, long long count, float eps, const float* gamma,
-                                const float* beta, float slope, float* mean, float* rstd, float* norm, int c_total, int c_off,
-                                float* norm_own, rehr_stream stream);
-/* a = lrelu_c(y * scale + shift) from such triples (norm = f32 [n][3][y->c]): materialises a deferred activation for consumers
- * without an on-load path; a2 optional second copy in another 16-bit format. */
-int rehr_norm_apply(const rehr_tensor* y, const float* norm, const rehr_tensor* a, const rehr_tensor* a2, rehr_stream stream);
 /* a = lrelu(gamma * (y - mean) * rstd + beta)   (slope = 1 -> no activation).  a2 (optional, may be NULL): a second copy of
  * the result in another 16-bit format / buffer, written in the same pass (the bf16 twin of an fp16 activation that the
  * weight-gradient GEMM of the consumer contracts with bf16 gradients). */

@@ -89,18 +89,9 @@ def _declare(L: C.CDLL) -> None:
         "rehr_pack_weight_march": (i, [vp, vp, i, i, i, ll, ll, i, i, vp]),
         "rehr_conv3d_march_stats_tiles": (i, [T, T, i]),
         "rehr_conv3d_march_fwd": (i, [T, vp, vp, T, i, i, i, f, vp, vp]),
-        "rehr_conv3d_march_norm_supported": (i, [D, i, i]),
-        "rehr_conv3d_march_fwd_norm": (i, [T, vp, i, vp, vp, T, i, i, i, f, vp, vp]),
-        "rehr_conv3d_wgrad_march_norm": (i, [T, vp, T, i, i, vp, i, vp, sz, vp]),
-        "rehr_conv3d_wgrad_march_s2_norm": (i, [D, T, vp, T, vp, i, vp, sz, vp]),
-        "rehr_instnorm_finalize_norm": (i, [vp, i, i, i, ll, f, vp, vp, f, vp, vp, vp, i, i, vp, vp]),
-        "rehr_norm_apply": (i, [T, vp, T, T, vp]),
         "rehr_conv3d_march_s2dgrad_supported": (i, [D, i, i]),
         "rehr_conv3d_march_s2dgrad_weight_bytes": (sz, [D, i, i]),
         "rehr_pack_weight_march_s2dgrad": (i, [D, vp, vp, i, i, vp]),
-        "rehr_conv3d_march_dgrad_inred_supported": (i, [D, i, i]),
-        "rehr_conv3d_march_dgrad_inred": (i, [T, vp, T, i, T, vp, vp, vp]),
-        "rehr_instnorm_lrelu_bwd_finalize_raw": (i, [vp, i, i, i, vp, vp, vp, vp, vp, i, vp]),
         "rehr_pack_batch_begin": (i, []),
         "rehr_pack_batch_launch": (i, [vp]),
         "rehr_pack_batch_abort": (i, []),

@@ -64,7 +64,7 @@ const char* rehr_strerror(int status) {
   }
 }
 int rehr_last_cuda_error(void) { return g_last_cuda_error; }
-int rehr_version(void) { return 5; }
+int rehr_version(void) { return 6; }
 int rehr_device_sm_count(void) { return sm_count(); }
 
 int rehr_pack_weight(const float* src, void* dst16, int R, int C, int T, long long sr, long long sc, long long st, int dtype,

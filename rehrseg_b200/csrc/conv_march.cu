@@ -35,12 +35,6 @@ int encode_tiled_bf16(CUtensorMap* m, const void* base, int rank, const unsigned
                       const unsigned long long* gstride_bytes, const unsigned* box, int swizzle_bytes);
 
 static constexpr int kMarchThreads = 192;  // warp0 TMA, warp1 MMA (+TMEM alloc), warps 2..5 epilogue
-// "normalise on load" variant (template XF): 3 more warps rewrite every landed input plane in place before the MMA reads it,
-//   operand = lrelu(x * scale[n,c] + shift[n,c])  (per-channel slope; slope 1 = identity),
-// so the InstanceNorm + LeakyReLU of the PRODUCING layer is applied on this layer's operand path and the normalised activation
-// never exists in HBM (x is the producer's raw, pre-normalisation conv output).  288 threads keep 224 registers per thread.
-static constexpr int kXfWarps = 3;
-static constexpr int kMarchThreadsXf = kMarchThreads + 32 * kXfWarps;
 static constexpr int kTileH = 16, kTileW = 8;
 // kernel size KS (3 or 5, cubic, stride 1, pad (KS-1)/2): halo'd input tile of (16 + KS - 1) x (8 + KS - 1) voxels
 template <int KS>
@@ -75,25 +69,15 @@ struct alignas(64) MarchParams {
   void* out;
   int out_f32;
   int out_f16;  // 16-bit output format (rehr_dtype of y) when !out_f32
-  int in_f16;   // MMA operand format: of the packed weights and of the activation tile the MMA reads (one format per tcgen05.mma)
-  int src_f16;  // storage format of x in HBM (differs from in_f16 only when the transform warps convert on load)
-  const float* norm;  // [N][3][Cin]: scale, shift, slope of the normalise-on-load transform (XF variants), else null
+  int in_f16;   // MMA operand format: of x and of the packed weights (one format per tcgen05.mma)
   long long out_ld;
   const float* bias;
   int act;
   float slope;
   float* stats;  // [N][tiles_per_sample][Cout][2] or null
-  // RED variants (input gradient whose result is the gradient of an InstanceNorm + LeakyReLU activation): y = the pre-normalisation
-  // tensor of THAT block (same voxels / channels as the output), red_norm = its f32 [N][3][Cout] table (scale, shift, slope).  The
-  // statistics slots then receive  S1 = sum g,  S2raw = sum g*y  with  g = (scale*y + shift > 0 ? 1 : slope) * output
-  const unsigned short* red_y;
-  const float* red_norm;
-  long long red_ld;
-  int red_f16;
   int* err;
   long long* prof;  // development only: per-role cycle counters of CTA 0 (env REHR_MARCH_PROF)
-  int debug;  // development only (env REHR_MARCH_DEBUG): bit0 skip input TMA, bit1 skip epilogue body, bit2 skip MMAs,
-              // bit3 skip the normalise-on-load body (barriers only), bit4 normalise-on-load copies without arithmetic
+  int debug;  // development only (env REHR_MARCH_DEBUG): bit0 skip input TMA, bit1 skip epilogue body, bit2 skip MMAs
 };
 
 __device__ __forceinline__ float march_act(float v, int act, float slope) {
@@ -129,14 +113,17 @@ __device__ __forceinline__ bool elect_one_sync() {
 // the MMA issue sequence of one input plane (9 * CHUNKS * BKT/16 instructions) is fully unrolled with constant
 // descriptor increments: a single thread must issue one tcgen05.mma every ~50 clk (tools/umma_rate2.cu measures
 // 40 clk/MMA for this code shape vs 120-280 clk/MMA with run-time descriptor arithmetic).
-// REHR_MARCH_MAXNREG (build-time, default = no cap): register cap of the 192-thread variants.  A 128-register build lets two
-// blocks of an InstanceNorm pass become resident next to a conv CTA (tools/overlap_probe.py: 55 % of a co-scheduled pass hides
-// behind a forward conv instead of 12 %) but costs the conv itself 5 % (spilled column sums); measured on the C1 step: a net loss.
+// REHR_MARCH_MAXNREG (build-time, default = no cap): register cap of the kernel.  A 128-register build lets two blocks of an
+// InstanceNorm pass become resident next to a conv CTA (tools/overlap_probe.py: 55 % of a co-scheduled pass hides behind a
+// forward conv instead of 12 %) but costs the conv itself 5 % (spilled column sums); measured on the C1 step: a net loss.
+// The kernel carries both .maxntid and .maxnreg: ptxas allocates registers differently with the explicit cap than without it
+// (94 instead of 80 for the 16-channel tile), and the kernels were measured that way.  nvcc accepts __launch_bounds__ together
+// with __maxnreg__ only when an argument depends on a template parameter, hence the KS term.
 #ifndef REHR_MARCH_MAXNREG
 #define REHR_MARCH_MAXNREG 255
 #endif
-template <int BKT, int CHUNKS, int CT, int KS, bool XF, bool RED = false>
-__global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnreg__(XF ? 224 : REHR_MARCH_MAXNREG) conv_march_kernel(const __grid_constant__ MarchParams p) {
+template <int BKT, int CHUNKS, int CT, int KS>
+__global__ void __launch_bounds__(kMarchThreads) __maxnreg__(KS > 0 ? REHR_MARCH_MAXNREG : 0) conv_march_kernel(const __grid_constant__ MarchParams p) {
   constexpr int R = MarchGeo<KS>::R;
   constexpr int kHaloW = MarchGeo<KS>::kHaloW;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -150,8 +137,7 @@ __global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnre
   uint64_t* tempty_bar = tfull_bar + kMaxSlots;            // [slots]
   uint64_t* wfull_bar = tempty_bar + kMaxSlots;            // [1]
   uint64_t* wfree_bar = wfull_bar + 1;                     // [1]
-  uint64_t* ready_bar = wfree_bar + 1;                     // [ring]  (XF: plane transformed, MMA may read)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(ready_bar + kMaxRing);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wfree_bar + 1);
   float* part = reinterpret_cast<float*>(tmem_slot + 4);   // [4 warps][2][64]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -164,7 +150,6 @@ __global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnre
     for (int i = 0; i < p.ring; ++i) {
       mbar_init(&full_bar[i], 1);
       mbar_init(&empty_bar[i], 1);
-      mbar_init(&ready_bar[i], kXfWarps);
     }
     for (int i = 0; i < p.slots; ++i) {
       mbar_init(&tfull_bar[i], 1);
@@ -263,7 +248,7 @@ __global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnre
           ++next_open;
         }
         const long long tm1 = clock64();
-        mbar_wait(XF ? &ready_bar[stage] : &full_bar[stage], phase, p.err, 33);
+        mbar_wait(&full_bar[stage], phase, p.err, 33);
         tc_fence_after();
         const long long tm2 = clock64();
         const uint32_t a_lo = sring_lo + (uint32_t)stage * slot_lo;
@@ -322,81 +307,7 @@ __global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnre
         __syncwarp();
       }
     }
-  } else if (XF && warp >= 6) {
-    // ============================== normalise-on-load (warps 6..8) ==============================
-    // thread = (16-byte channel group g, row lane): its 8 channels per chunk are fixed, so scale / shift / slope live in registers
-    constexpr int G = BKT / 8;               // 16-byte groups per tile row
-    constexpr int RL = 32 * kXfWarps / G;    // row lanes
-    constexpr uint32_t kRowB = BKT * 2;
-    constexpr int kHaloRows = MarchGeo<KS>::kHaloRows;
-    const int tt = (int)threadIdx.x - 192;
-    const int g = tt % G, rl = tt / G;
-    float sc[CHUNKS][8], sf[CHUNKS][8], sl[CHUNKS][8];
-    int cur_n = -1;
-    int stage = 0;
-    uint32_t phase = 0;
-    const int src16 = p.src_f16, dst16 = p.in_f16;
-    for (int item = blockIdx.x; item < p.total_items; item += gridDim.x) {
-      const ItemCoord c = decode_item(p, item);
-      if (c.n != cur_n) {
-        cur_n = c.n;
-#pragma unroll
-        for (int ch = 0; ch < CHUNKS; ++ch) {
-          const float* np = p.norm + (size_t)c.n * 3 * p.Cin + ch * BKT + g * 8;
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            sc[ch][i] = __ldg(np + i);
-            sf[ch][i] = __ldg(np + p.Cin + i);
-            sl[ch][i] = __ldg(np + 2 * p.Cin + i);
-          }
-        }
-      }
-      const int d0 = c.seg * p.Ds, d1 = min(p.D, d0 + p.Ds);
-      const int pa = max(d0 + p.kd_lo - R, 0), pb = min(d1 - 1 + p.kd_hi - R, p.D - 1);
-      const int h0 = c.th * kTileH - R, w0 = c.tw * kTileW - R;
-      for (int pl = pa; pl <= pb; ++pl) {
-        mbar_wait(&full_bar[stage], phase, p.err, 61);
-        uint8_t* base = s_ring + (size_t)stage * p.slot_stride;
-        // U rows per pass and thread: all loads of a pass are issued before the arithmetic (latency, not issue rate, bounds this
-        // stage: it must stay below the MMA time of a plane)
-        constexpr int U = CHUNKS == 1 ? 4 : 2;
-        for (int r0 = rl; r0 < kHaloRows && !(p.debug & 8); r0 += RL * U) {
-          uint4 v[U][CHUNKS];
-          uint32_t off[U];
-          bool ok[U];
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            const int r = r0 + u * RL;
-            const int hh = r / kHaloW, ww = r - hh * kHaloW;
-            // rows outside the volume hold the TMA zero fill and must STAY zero: the conv pads the normalised activation
-            ok[u] = r < kHaloRows && (unsigned)(h0 + hh) < (unsigned)p.H && (unsigned)(w0 + ww) < (unsigned)p.W;
-            off[u] = (uint32_t)r * kRowB + (uint32_t)g * 16u;
-            off[u] ^= ((off[u] >> 7) & (uint32_t)(G - 1)) << 4;  // TMA swizzle: 16-byte unit index XOR (128-byte line index mod G)
-            if (ok[u]) {
-#pragma unroll
-              for (int ch = 0; ch < CHUNKS; ++ch) v[u][ch] = *reinterpret_cast<const uint4*>(base + (size_t)ch * p.chunk_stride + off[u]);
-            }
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            if (ok[u]) {
-#pragma unroll
-              for (int ch = 0; ch < CHUNKS; ++ch)
-                *reinterpret_cast<uint4*>(base + (size_t)ch * p.chunk_stride + off[u]) =
-                    (p.debug & 16) ? v[u][ch] : xform16(v[u][ch], sc[ch], sf[ch], sl[ch], src16, dst16);
-            }
-          }
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the MMA (async proxy)
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&ready_bar[stage]);
-        if (++stage == p.ring) {
-          stage = 0;
-          phase ^= 1u;
-        }
-      }
-    }
-  } else if (warp < 6) {
+  } else {
     // ============================== epilogue (warps 2..5) ==============================
     const int q4 = warp & 3;
     const int row = q4 * 32 + lane;
@@ -430,16 +341,6 @@ __global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnre
       for (int q = d0; q < d1; ++q) {
         const int s = (q - d0) & kSlotMask;
         const long long te0 = clock64();
-        // RED: this voxel's y row is requested BEFORE the wait for the plane's accumulators, so its global-memory latency
-        // overlaps the MMAs still running (issued after the wait it sat on the critical path of every plane: +65 % kernel time)
-        uint4 ypre[RED ? CT / 8 : 1];
-        if constexpr (RED) {
-          if (valid_hw && q < p.OD) {
-            const long long yoff = ((((long long)c.n * p.D + q) * p.H + oh) * p.W + ow) * p.red_ld + cbase;
-#pragma unroll
-            for (int i = 0; i < CT / 8; ++i) ypre[i] = __ldg(reinterpret_cast<const uint4*>(p.red_y + yoff + 8 * i));
-          }
-        }
         mbar_wait(&tfull_bar[s], (tfull_par >> s) & 1u, p.err, 41);
         tfull_par ^= 1u << s;
         tc_fence_after();
@@ -470,40 +371,7 @@ __global__ void __launch_bounds__(XF ? kMarchThreadsXf : kMarchThreads) __maxnre
                 if (i < nvalid) f[i] += __ldg(p.bias + cbase + c0 + i);
             }
           }
-          if constexpr (RED) {
-            // InstanceNorm + LeakyReLU backward sums of the block that produced this conv's input, taken from the fp32
-            // accumulators on their way out (saves that block's stand-alone reduce pass over dA and y)
-            if (valid) {
-              const float* nt = p.red_norm + (long long)c.n * 3 * p.Cout + cbase + c0;
-#pragma unroll
-              for (int i = 0; i < kW; i += 8) {
-                const uint4 yu = ypre[(c0 + i) / 8];
-                const uint32_t yw[4] = {yu.x, yu.y, yu.z, yu.w};
-                float yv[8];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const float2 t2 = unpack16x2(yw[k], p.red_f16);
-                  yv[2 * k] = t2.x;
-                  yv[2 * k + 1] = t2.y;
-                }
-#pragma unroll
-                for (int h4 = 0; h4 < 8; h4 += 4) {
-                  const float4 A4 = __ldg(reinterpret_cast<const float4*>(nt + i + h4));
-                  const float4 B4 = __ldg(reinterpret_cast<const float4*>(nt + p.Cout + i + h4));
-                  const float4 S4 = __ldg(reinterpret_cast<const float4*>(nt + 2 * p.Cout + i + h4));
-                  const float Ai[4] = {A4.x, A4.y, A4.z, A4.w}, Bi[4] = {B4.x, B4.y, B4.z, B4.w}, Si[4] = {S4.x, S4.y, S4.z, S4.w};
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) {
-                    const float yy = yv[h4 + k];
-                    const float z = fmaf(Ai[k], yy, Bi[k]);
-                    const float gi = z > 0.f ? f[i + h4 + k] : f[i + h4 + k] * Si[k];
-                    s1[c0 + i + h4 + k] += gi;
-                    s2[c0 + i + h4 + k] = fmaf(gi, yy, s2[c0 + i + h4 + k]);
-                  }
-                }
-              }
-            }
-          } else if (p.stats != nullptr && valid) {
+          if (p.stats != nullptr && valid) {
 #pragma unroll
             for (int i = 0; i < kW; ++i) {
               s1[c0 + i] += f[i];
@@ -643,6 +511,8 @@ struct MarchPlan {
   int grid;
 };
 
+// barriers (full / empty ring, tfull / tempty slots, wfull, wfree), TMEM address, epilogue partials.  One more ring of barriers
+// (8 * kMaxRing bytes) stays reserved: the plane-ring depths of the tuned layer shapes were measured with a tail of this size.
 static size_t march_tail_bytes() { return (3 * kMaxRing + 2 * kMaxSlots + 2) * 8 + 16 + 4 * 2 * 64 * 4; }
 
 static int plan_march(const rehr_tensor& x, const rehr_tensor& y, int ks_code, MarchPlan* out, int ds_override) {
@@ -711,8 +581,7 @@ struct MarchExt {
 };
 
 int launch_march(const rehr_tensor& x, const void* w_march, const float* bias, const rehr_tensor& y, int ks_code, int y_is_f32, int act,
-                 float slope, float* stats, cudaStream_t stream, const MarchExt* ext = nullptr, const float* norm = nullptr,
-                 int op_dtype = REHR_BF16, const rehr_tensor* red_y = nullptr, const float* red_norm = nullptr) {
+                 float slope, float* stats, cudaStream_t stream, const MarchExt* ext = nullptr) {
   MarchPlan pl;
   int rc = plan_march(x, y, ks_code, &pl, 0);
   if (rc != REHR_OK) return rc;
@@ -723,9 +592,7 @@ int launch_march(const rehr_tensor& x, const void* w_march, const float* bias, c
   p.out = y.ptr;
   p.out_f32 = y_is_f32;
   p.out_f16 = y.dtype == REHR_F16;
-  p.src_f16 = x.dtype == REHR_F16;
-  p.in_f16 = norm ? (op_dtype == REHR_F16) : p.src_f16;
-  p.norm = norm;
+  p.in_f16 = x.dtype == REHR_F16;
   p.out_ld = y.ld;
   p.o_pw = y.ld;
   p.o_ph = (long long)y.w * y.ld;
@@ -746,18 +613,6 @@ int launch_march(const rehr_tensor& x, const void* w_march, const float* bias, c
   p.act = act;
   p.slope = slope;
   p.stats = stats;
-  p.red_y = nullptr;
-  p.red_norm = nullptr;
-  if (red_y != nullptr) {
-    // same voxels and channels as the output, whole channel tiles, plain stride-1 layer
-    if (ext || norm || !stats || !red_norm || y_is_f32 || red_y->n != y.n || red_y->d != y.d || red_y->h != y.h || red_y->w != y.w ||
-        red_y->c != y.c || y.c % p.Ct != 0 || red_y->ld % 8 != 0 || (reinterpret_cast<uintptr_t>(red_y->ptr) & 15) != 0)
-      return REHR_UNSUPPORTED;
-    p.red_y = reinterpret_cast<const unsigned short*>(red_y->ptr);
-    p.red_norm = red_norm;
-    p.red_ld = red_y->ld;
-    p.red_f16 = red_y->dtype == REHR_F16;
-  }
   p.err = nullptr;
   {
     const char* dbg = getenv("REHR_MARCH_DEBUG");
@@ -795,28 +650,8 @@ int launch_march(const rehr_tensor& x, const void* w_march, const float* bias, c
 
 template <int BKT, int CHUNKS, int CT, int KS>
 static int launch_variant(const MarchPlan& pl, cudaStream_t stream) {
-  if (pl.p.norm != nullptr) {
-    if constexpr (CT <= 32 && KS == 3) {   // the transform warps cost registers: 64-column epilogues keep the 192-thread shape
-      REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS, true>), 227 * 1024);
-      conv_march_kernel<BKT, CHUNKS, CT, KS, true><<<pl.grid, kMarchThreadsXf, pl.smem, stream>>>(pl.p);
-      REHR_CHECK_LAUNCH();
-      return REHR_OK;
-    } else {
-      return REHR_UNSUPPORTED;
-    }
-  }
-  if (pl.p.red_y != nullptr) {
-    if constexpr (KS == 3 && CT <= 32) {   // the layers whose input is a Conv -> InstanceNorm -> LeakyReLU block at 16 .. 128 channels
-      REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS, false, true>), 227 * 1024);
-      conv_march_kernel<BKT, CHUNKS, CT, KS, false, true><<<pl.grid, kMarchThreads, pl.smem, stream>>>(pl.p);
-      REHR_CHECK_LAUNCH();
-      return REHR_OK;
-    } else {
-      return REHR_UNSUPPORTED;
-    }
-  }
-  REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS, false>), 227 * 1024);
-  conv_march_kernel<BKT, CHUNKS, CT, KS, false><<<pl.grid, kMarchThreads, pl.smem, stream>>>(pl.p);
+  REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS>), 227 * 1024);
+  conv_march_kernel<BKT, CHUNKS, CT, KS><<<pl.grid, kMarchThreads, pl.smem, stream>>>(pl.p);
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }
@@ -975,38 +810,6 @@ int rehr_conv3d_march_fwd(const rehr_tensor* x, const void* w_march, const float
                           int act, float slope, float* stats, rehr_stream stream) {
   if (!x || !y || !x->ptr || !y->ptr || !w_march) return REHR_BAD_SHAPE;
   return launch_march(*x, w_march, bias, *y, ks, y_is_f32, act, slope, stats, (cudaStream_t)stream);
-}
-
-// Input gradient dx = conv^T(dy) of a stride-1 marching layer whose INPUT was the activation of a Conv -> InstanceNorm -> LeakyReLU
-// block: y_prod = that block's pre-normalisation tensor (same shape as dx), norm_prod = its f32 [n][3][c] table (scale, shift,
-// slope) from rehr_instnorm_finalize_norm.  Besides dx the epilogue leaves the block's backward sums (S1 = sum g, S2raw = sum g*y)
-// in stats [n][rehr_conv3d_march_stats_tiles][c][2]; rehr_instnorm_lrelu_bwd_finalize_raw turns them into (sum g, sum g*xhat).
-int rehr_conv3d_march_dgrad_inred_supported(const rehr_conv_desc* d, int cin_dy, int cout_dx) {
-  const int ks = march_ks_of(d);
-  if (ks != 3) return 0;
-  const int ct = march_ct(cin_dy, cout_dx, 3, false);
-  return ct > 0 && ct <= 32 && cout_dx % ct == 0 ? 1 : 0;
-}
-int rehr_conv3d_march_dgrad_inred(const rehr_tensor* dy, const void* w_march, const rehr_tensor* dx, int ks, const rehr_tensor* y_prod,
-                                  const float* norm_prod, float* stats, rehr_stream stream) {
-  if (!dy || !dx || !dy->ptr || !dx->ptr || !w_march || !y_prod || !y_prod->ptr || !norm_prod || !stats) return REHR_BAD_SHAPE;
-  return launch_march(*dy, w_march, nullptr, *dx, ks, 0, REHR_ACT_NONE, 0.f, stats, (cudaStream_t)stream, nullptr, nullptr, REHR_BF16,
-                      y_prod, norm_prod);
-}
-
-// Same, with the producer's InstanceNorm + LeakyReLU applied on the operand path: x is the RAW conv output of the producing
-// layer, norm = f32 [n][3][cin] (scale = gamma * rstd, shift = beta - mean * scale, slope) from rehr_instnorm_norm_params; the
-// transformed tile is written in the 16-bit format `op_dtype`, which is also the format of the packed weights.
-int rehr_conv3d_march_norm_supported(const rehr_conv_desc* d, int cin, int cout) {
-  const int ks = march_ks_of(d);
-  if (ks != 3 && ks != 1) return 0;
-  const int ct = march_ct(cin, cout, 3, ks == 1);
-  return ct > 0 && ct <= 32 ? 1 : 0;
-}
-int rehr_conv3d_march_fwd_norm(const rehr_tensor* x, const float* norm, int op_dtype, const void* w_march, const float* bias,
-                               const rehr_tensor* y, int ks, int y_is_f32, int act, float slope, float* stats, rehr_stream stream) {
-  if (!x || !y || !x->ptr || !y->ptr || !w_march || !norm) return REHR_BAD_SHAPE;
-  return launch_march(*x, w_march, bias, *y, ks, y_is_f32, act, slope, stats, (cudaStream_t)stream, nullptr, norm, op_dtype);
 }
 
 // ---- stride-2 (per dimension 1 or 2) input gradient of a k3 / pad 1 conv through the marching kernel, one launch per parity class

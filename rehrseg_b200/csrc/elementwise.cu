@@ -213,16 +213,11 @@ static int launch_in_reduce(const StatArgs& a, int N, cudaStream_t st) {
 // so a 1024-tile list costs ~32 dependent-free loads per thread instead of 1024 serial ones.
 static constexpr int kFinLanes = 32;
 
-// norm (optional): the affine + activation of this InstanceNorm as per-(n, channel) triples for "normalise on load" consumers,
-//   norm[(n*3 + 0) * c_total + c_off + c] = gamma*rstd,  [.. + 1 ..] = beta - mean*gamma*rstd,  [.. + 2 ..] = slope;
-// channels [0, c_off) of the same rows are set to the identity (1, 0, 1): the up-sampled half of a decoder concat buffer.
 // CPB = channels per block (32, or 8 for long partial lists: four times as many blocks and tile lanes -- the stage-entry convs
 // leave 2048 partials per sample, which 4 blocks of 32 lanes took 25 us to walk)
 template <int CPB>
 __global__ void __launch_bounds__(32 * kFinLanes) in_finalize_kernel(const float* partial, int N, int tiles, int C,
-                                                                      double inv_count, float eps, float* mean, float* rstd,
-                                                                      const float* gamma, const float* beta, float slope,
-                                                                      float* norm, int c_total, int c_off, float* norm_own) {
+                                                                      double inv_count, float eps, float* mean, float* rstd) {
   constexpr int kLanes = 32 * kFinLanes / CPB;
   __shared__ double sh1[kLanes][CPB + 1], sh2[kLanes][CPB + 1];
   const int cl = threadIdx.x % CPB, tl = threadIdx.x / CPB;
@@ -253,65 +248,13 @@ __global__ void __launch_bounds__(32 * kFinLanes) in_finalize_kernel(const float
     const float rs = (float)(1.0 / sqrt(var + (double)eps));
     mean[n * C + c] = (float)m;
     rstd[n * C + c] = rs;
-    if (norm != nullptr) {
-      const float ga = gamma ? gamma[c] : 1.f, be = beta ? beta[c] : 0.f;
-      float* row = norm + (size_t)n * 3 * c_total + c_off + c;
-      row[0] = ga * rs;
-      row[c_total] = be - (float)m * ga * rs;
-      row[2 * c_total] = slope;
-      if (norm_own != nullptr) {  // the same triples as a dense [n][3][C] table (consumers of this tensor alone)
-        float* own = norm_own + (size_t)n * 3 * C + c;
-        own[0] = row[0];
-        own[C] = row[c_total];
-        own[2 * C] = slope;
-      }
-    }
-  }
-  if (norm != nullptr && blockIdx.x == 0) {
-    for (int i = threadIdx.x; i < c_off; i += blockDim.x) {
-      float* row = norm + (size_t)n * 3 * c_total + i;
-      row[0] = 1.f;
-      row[c_total] = 0.f;
-      row[2 * c_total] = 1.f;
-    }
-  }
-}
-
-// a = lrelu_c(y * scale[n,c] + shift[n,c]) from norm triples (see in_finalize_kernel); optional second copy a2 in another format
-struct NormApplyArgs {
-  const __nv_bfloat16* y;
-  __nv_bfloat16 *out, *out2;
-  long long ld_y, ld_o, ld_o2, V;
-  const float* norm;
-  int C, y_f16, out_f16, out2_f16;
-};
-__global__ void __launch_bounds__(256) norm_apply_kernel(const NormApplyArgs a) {
-  extern __shared__ float sh[];  // [3][C]
-  const int n = blockIdx.y, C = a.C;
-  for (int i = threadIdx.x; i < 3 * C; i += blockDim.x) sh[i] = a.norm[(size_t)n * 3 * C + i];
-  __syncthreads();
-  const int groups = C / 8;
-  const long long items = a.V * groups;
-  for (long long it = blockIdx.x * (long long)blockDim.x + threadIdx.x; it < items; it += (long long)gridDim.x * blockDim.x) {
-    const int g = (int)(it % groups);
-    const long long vox = (long long)n * a.V + it / groups;
-    float y[8], o[8];
-    x16x8_to_float(__ldcs(reinterpret_cast<const uint4*>(a.y + vox * a.ld_y + g * 8)), y, a.y_f16);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const int c = g * 8 + i;
-      const float z = fmaf(y[i], sh[c], sh[C + c]);
-      o[i] = z > 0.f ? z : z * sh[2 * C + c];
-    }
-    *reinterpret_cast<uint4*>(a.out + vox * a.ld_o + g * 8) = float_to_x16x8(o, a.out_f16);
-    if (a.out2 != nullptr) *reinterpret_cast<uint4*>(a.out2 + vox * a.ld_o2 + g * 8) = float_to_x16x8(o, a.out2_f16);
   }
 }
 
 // partial [n][tiles][c][2] -> sums [n][c][2]; dgamma[c] = sum_n S2, dbeta[c] = sum_n S1.  Same thread layout; grid = C/32.
 __global__ void __launch_bounds__(32 * kFinLanes) in_bwd_finalize_kernel(const float* partial, int N, int tiles, int C,
                                                                           float* sums, float* dgamma, float* dbeta,
-                                                                          int accumulate, const float* raw_mean, const float* raw_rstd) {
+                                                                          int accumulate) {
   __shared__ double sh1[kFinLanes][33], sh2[kFinLanes][33];
   const int cl = threadIdx.x & 31, tl = threadIdx.x >> 5;
   const int c = blockIdx.x * 32 + cl;
@@ -346,8 +289,6 @@ __global__ void __launch_bounds__(32 * kFinLanes) in_bwd_finalize_kernel(const f
           a2 += sh2[l][cl];
         }
         const int n = n0 + k;
-        // raw partials (sum g, sum g*y) from a conv epilogue: sum g*xhat = rstd * (sum g*y - mean * sum g)
-        if (raw_mean != nullptr) a2 = (double)raw_rstd[n * C + c] * (a2 - (double)raw_mean[n * C + c] * a1);
         sums[((long long)n * C + c) * 2] = (float)a1;
         sums[((long long)n * C + c) * 2 + 1] = (float)a2;
         b += a1;
@@ -1673,44 +1614,10 @@ int rehr_instnorm_finalize(const float* partial, int n, int tiles, int c, long l
   if (!partial || !mean || !rstd || count <= 0) return REHR_BAD_SHAPE;
   if (tiles >= 256)
     in_finalize_kernel<8><<<dim3((c + 7) / 8, n), 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, 1.0 / (double)count, eps, mean,
-                                                                            rstd, nullptr, nullptr, 1.f, nullptr, 0, 0, nullptr);
+                                                                            rstd);
   else
     in_finalize_kernel<32><<<dim3((c + 31) / 32, n), 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, 1.0 / (double)count, eps, mean,
-                                                                              rstd, nullptr, nullptr, 1.f, nullptr, 0, 0, nullptr);
-  REHR_CHECK_LAUNCH();
-  return REHR_OK;
-}
-
-int rehr_instnorm_finalize_norm(const float* partial, int n, int tiles, int c, long long count, float eps, const float* gamma,
-                                const float* beta, float slope, float* mean, float* rstd, float* norm, int c_total, int c_off,
-                                float* norm_own, rehr_stream stream) {
-  if (!partial || !mean || !rstd || !norm || count <= 0 || c_off < 0 || c_off + c > c_total) return REHR_BAD_SHAPE;
-  if (tiles >= 256)
-    in_finalize_kernel<8><<<dim3((c + 7) / 8, n), 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, 1.0 / (double)count, eps, mean,
-                                                                            rstd, gamma, beta, slope, norm, c_total, c_off, norm_own);
-  else
-    in_finalize_kernel<32><<<dim3((c + 31) / 32, n), 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, 1.0 / (double)count, eps, mean,
-                                                                              rstd, gamma, beta, slope, norm, c_total, c_off, norm_own);
-  REHR_CHECK_LAUNCH();
-  return REHR_OK;
-}
-
-int rehr_norm_apply(const rehr_tensor* y, const float* norm, const rehr_tensor* a, const rehr_tensor* a2, rehr_stream stream) {
-  if (!bf16_tensor_ok(y) || !bf16_tensor_ok(a) || !norm || y->c != a->c || y->n != a->n || voxels_per_sample(y) != voxels_per_sample(a))
-    return REHR_BAD_SHAPE;
-  if (a2 && (!bf16_tensor_ok(a2) || a2->c != y->c || a2->n != y->n || voxels_per_sample(a2) != voxels_per_sample(y))) return REHR_BAD_SHAPE;
-  NormApplyArgs p{};
-  p.y = reinterpret_cast<const __nv_bfloat16*>(y->ptr);
-  p.out = reinterpret_cast<__nv_bfloat16*>(a->ptr);
-  p.out2 = a2 ? reinterpret_cast<__nv_bfloat16*>(a2->ptr) : nullptr;
-  p.ld_y = y->ld; p.ld_o = a->ld; p.ld_o2 = a2 ? a2->ld : 0;
-  p.V = voxels_per_sample(y);
-  p.norm = norm;
-  p.C = y->c;
-  p.y_f16 = y->dtype == REHR_F16; p.out_f16 = a->dtype == REHR_F16; p.out2_f16 = a2 ? a2->dtype == REHR_F16 : 0;
-  const long long items = p.V * (p.C / 8);
-  int gx = std::max(1, grid_for(items, 256, 8) / std::max(1, y->n));
-  norm_apply_kernel<<<dim3(gx, y->n), 256, (size_t)3 * p.C * sizeof(float), (cudaStream_t)stream>>>(p);
+                                                                              rstd);
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }
@@ -1771,17 +1678,7 @@ int rehr_instnorm_lrelu_bwd_finalize(const float* partial, int n, int tiles, int
                                      float* dgamma, float* dbeta, int accumulate, rehr_stream stream) {
   (void)rstd;
   if (!partial || !sums) return REHR_BAD_SHAPE;
-  in_bwd_finalize_kernel<<<(c + 31) / 32, 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, sums, dgamma, dbeta, accumulate,
-                                                                                     nullptr, nullptr);
-  REHR_CHECK_LAUNCH();
-  return REHR_OK;
-}
-
-int rehr_instnorm_lrelu_bwd_finalize_raw(const float* partial, int n, int tiles, int c, const float* mean, const float* rstd, float* sums,
-                                         float* dgamma, float* dbeta, int accumulate, rehr_stream stream) {
-  if (!partial || !sums || !mean || !rstd) return REHR_BAD_SHAPE;
-  in_bwd_finalize_kernel<<<(c + 31) / 32, 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, sums, dgamma, dbeta, accumulate,
-                                                                                     mean, rstd);
+  in_bwd_finalize_kernel<<<(c + 31) / 32, 32 * kFinLanes, 0, (cudaStream_t)stream>>>(partial, n, tiles, c, sums, dgamma, dbeta, accumulate);
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }
@@ -1886,8 +1783,7 @@ int rehr_channel_sum(const rehr_tensor* x, float* out, int accumulate, void* ws,
 int rehr_upsample_linear_d(const rehr_tensor* x, const rehr_tensor* y, rehr_stream stream) {
   if (!bf16_tensor_ok(x) || !bf16_tensor_ok(y) || x->c != y->c || x->n != y->n || x->h != y->h || x->w != y->w) return REHR_BAD_SHAPE;
   const long long HW = (long long)x->h * x->w;
-  static const bool legacy = getenv("REHR_UPSAMPLE_LEGACY") != nullptr;  // the output-centric kernel, for A/B runs
-  if (y->d >= x->d && !legacy) {
+  if (y->d >= x->d) {
     const long long items = (long long)x->n * x->d * HW * (x->c / 8);
     upsample_d_src_kernel<<<grid_for(items, 256, 8), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const __nv_bfloat16*>(x->ptr), x->ld, reinterpret_cast<__nv_bfloat16*>(y->ptr), y->ld, x->n, x->d, y->d, HW, x->c,

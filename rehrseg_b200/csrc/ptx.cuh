@@ -185,24 +185,6 @@ __device__ __forceinline__ float2 unpack16x2(uint32_t u, int fp16) {
 }
 __device__ __forceinline__ float unpack16(unsigned short u, int fp16) { return unpack16x2((uint32_t)u, fp16).x; }
 
-// "Normalise on load" of ONE 16-byte unit (8 channels) of a landed tile: v -> lrelu(v*sc + sf) per channel, re-packed in the
-// operand format.  LeakyReLU in max form (z, z*slope): valid for slopes in [0, 1] (ReLU, LeakyReLU, identity = 1).
-__device__ __forceinline__ uint4 xform16(const uint4 u, const float (&sc)[8], const float (&sf)[8], const float (&sl)[8], int src16,
-                                         int dst16) {
-  const uint32_t w4[4] = {u.x, u.y, u.z, u.w};
-  uint32_t o4[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    float2 v = unpack16x2(w4[k], src16);
-    v.x = fmaf(v.x, sc[2 * k], sf[2 * k]);
-    v.y = fmaf(v.y, sc[2 * k + 1], sf[2 * k + 1]);
-    v.x = fmaxf(v.x, v.x * sl[2 * k]);
-    v.y = fmaxf(v.y, v.y * sl[2 * k + 1]);
-    o4[k] = pack16x2(v.x, v.y, dst16);
-  }
-  return make_uint4(o4[0], o4[1], o4[2], o4[3]);
-}
-
 }  // namespace rehr
 
 namespace rehr {

@@ -68,13 +68,6 @@ struct alignas(64) WgmParams {
   int cls_begin[9];
   int cls_gmask[8], cls_jmin[8], cls_jmax[8];
   CUtensorMap h_maps[8];
-  // "normalise on load" of the X operand (see conv_march.cu): the otherwise idle drain warps rewrite every landed X tile in place,
-  //   operand = bf16( lrelu(x * scale[n,c] + shift[n,c]) ),   norm = f32 [N][3][x_c] (scale, shift, slope),
-  // so X may be the producer's RAW conv output in either 16-bit storage format.  xf_role: 0 off, 1 X is the halo operand, 2 X is
-  // the plain operand.  Rows outside the X volume (TMA zero fill) stay zero; xd / xh / xw = extents of the X view a class reads.
-  int xf_role, x_f16, x_c;
-  const float* norm;
-  int xd[8], xh[8], xw[8];
 };
 
 // Geometry of one (CH halo channels, PC plain channels, KS kernel size) variant.
@@ -151,9 +144,7 @@ __global__ void __launch_bounds__(kWgmThreads, 1) wgrad_march_kernel(const __gri
   uint64_t* empty_p = full_p + kPRing;
   uint64_t* zero_bar = empty_p + kPRing;
   uint64_t* done_bar = zero_bar + 1;
-  uint64_t* ready_h = done_bar + 1;       // [kHStages]  halo tile transformed
-  uint64_t* ready_p = ready_h + kMaxHStages;  // [kPRing]    plain tile transformed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(ready_p + kPRing);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(done_bar + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0 && lane == 0) {
@@ -162,12 +153,10 @@ __global__ void __launch_bounds__(kWgmThreads, 1) wgrad_march_kernel(const __gri
     for (int i = 0; i < kMaxHStages; ++i) {
       mbar_init(&full_h[i], 1);
       mbar_init(&empty_h[i], 1);
-      mbar_init(&ready_h[i], 3);
     }
     for (int i = 0; i < kPRing; ++i) {
       mbar_init(&full_p[i], 1);
       mbar_init(&empty_p[i], 1);
-      mbar_init(&ready_p[i], 3);
     }
     mbar_init(zero_bar, 4);
     mbar_init(done_bar, 1);
@@ -252,10 +241,10 @@ __global__ void __launch_bounds__(kWgmThreads, 1) wgrad_march_kernel(const __gri
         while (waited < need) {
           ++waited;
           const uint32_t cc = cnt0 + (uint32_t)(waited - pa);
-          mbar_wait(p.xf_role == 2 ? &ready_p[cc % kPRing] : &full_p[cc % kPRing], (cc / kPRing) & 1u, p.err, 62);
+          mbar_wait(&full_p[cc % kPRing], (cc / kPRing) & 1u, p.err, 62);
         }
         const uint32_t st = kh % kHStages;
-        mbar_wait(p.xf_role == 1 ? &ready_h[st] : &full_h[st], (kh / kHStages) & 1u, p.err, 63);
+        mbar_wait(&full_h[st], (kh / kHStages) & 1u, p.err, 63);
         tc_fence_after();
         // plain planes q - R + j, j in [jlo, jhi], exist inside the volume
         const int jlo = max(max(0, R - q), j_min), jhi = min(min(KS - 1, p.D - 1 - q + R), j_max);
@@ -307,97 +296,6 @@ __global__ void __launch_bounds__(kWgmThreads, 1) wgrad_march_kernel(const __gri
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(zero_bar);
-    }
-    if (p.xf_role != 0 && warp < 5) {
-      // ---------------- normalise-on-load of the X tiles (these warps are idle until the final drain) ----------------
-      // warps 2..4 only: warp 5 shares its scheduler with the MMA-issuing warp 1, whose issue slots bound the kernel
-      const int tt = (int)threadIdx.x - 64;           // 0..95
-      const bool halo = p.xf_role == 1;
-      const int G = halo ? CH / 8 : PC / 8;            // 16-byte groups per tile row
-      const int g = tt % G, rl = tt / G, RL = 96 / G;
-      const uint32_t rowb = halo ? Cfg::kRowB : Cfg::kPRowB;
-      const int c0 = (halo ? hs * CH : ps * PC) + g * 8;
-      const int XD = p.xd[cls], XH = p.xh[cls], XW = p.xw[cls];
-      float sc[8], sf[8], sl[8];
-      int cur_n = -1;
-      uint32_t kh = 0, kp = 0;
-      constexpr int U = 4;   // rows in flight per thread: all loads of a pass are issued before the arithmetic
-      for (int item = rank; item < p.items_per_combo; item += ctas_per_combo) {
-        const WgmItem c = wgm_decode(p, item);
-        if (c.n != cur_n) {
-          cur_n = c.n;
-          const float* np = p.norm + (size_t)c.n * 3 * p.x_c + c0;
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            sc[i] = __ldg(np + i);
-            sf[i] = __ldg(np + p.x_c + i);
-            sl[i] = __ldg(np + 2 * p.x_c + i);
-          }
-        }
-        const int d0 = c.seg * p.Ds, d1 = min(p.D, d0 + p.Ds);
-        const int pa = max(d0 - R, 0), pb = min(d1 - 1 + R, p.D - 1);
-        const int h0 = c.th * kWTileH, w0 = c.tw * kWTileW;
-        if (halo) {
-          for (int q = d0; q < d1; ++q) {
-            const uint32_t st = kh % kHStages;
-            mbar_wait(&full_h[st], (kh / kHStages) & 1u, p.err, 81);
-            if (q < XD) {
-              uint8_t* base = s_h + (size_t)st * p.h_stride;
-              for (int r0 = rl; r0 < Cfg::kHaloRows; r0 += RL * U) {
-                uint4 v[U];
-                uint32_t off[U];
-                bool ok[U];
-#pragma unroll
-                for (int u = 0; u < U; ++u) {
-                  const int r = r0 + u * RL;
-                  const int hh = r / Cfg::kHaloW, ww = r - hh * Cfg::kHaloW;
-                  // rows outside the X volume hold the TMA zero fill and stay zero (the conv pads the normalised activation)
-                  ok[u] = r < Cfg::kHaloRows && (unsigned)(h0 - R + hh) < (unsigned)XH && (unsigned)(w0 - R + ww) < (unsigned)XW;
-                  off[u] = (uint32_t)r * rowb + (uint32_t)g * 16u;
-                  off[u] ^= ((off[u] >> 7) & (uint32_t)(G - 1)) << 4;
-                  if (ok[u]) v[u] = *reinterpret_cast<const uint4*>(base + off[u]);
-                }
-#pragma unroll
-                for (int u = 0; u < U; ++u)
-                  if (ok[u]) *reinterpret_cast<uint4*>(base + off[u]) = xform16(v[u], sc, sf, sl, p.x_f16, 0);
-              }
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&ready_h[st]);
-            ++kh;
-          }
-        } else {
-          for (int pl = pa; pl <= pb; ++pl) {
-            const uint32_t slot = kp % kPRing;
-            mbar_wait(&full_p[slot], (kp / kPRing) & 1u, p.err, 82);
-            const int copies = slot < (uint32_t)Cfg::kMirror ? 2 : 1;
-            for (int cp = 0; cp < copies; ++cp) {
-              uint8_t* base = s_p + (size_t)(slot + cp * kPRing) * kPSlotBytes;
-              for (int r0 = rl; r0 < kWTileH * kWTileW; r0 += RL * U) {
-                uint4 v[U];
-                uint32_t off[U];
-                bool ok[U];
-#pragma unroll
-                for (int u = 0; u < U; ++u) {
-                  const int r = r0 + u * RL;
-                  ok[u] = r < kWTileH * kWTileW && h0 + r / kWTileW < XH && w0 + r % kWTileW < XW;
-                  off[u] = (uint32_t)r * rowb + (uint32_t)g * 16u;
-                  off[u] ^= ((off[u] >> 7) & (uint32_t)(G - 1)) << 4;
-                  if (ok[u]) v[u] = *reinterpret_cast<const uint4*>(base + off[u]);
-                }
-#pragma unroll
-                for (int u = 0; u < U; ++u)
-                  if (ok[u]) *reinterpret_cast<uint4*>(base + off[u]) = xform16(v[u], sc, sf, sl, p.x_f16, 0);
-              }
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&ready_p[slot]);
-            ++kp;
-          }
-        }
-      }
     }
     mbar_wait(done_bar, 0, p.err, 71);
     tc_fence_after();
@@ -632,6 +530,8 @@ static int plan_wgm(const rehr_tensor& x, const rehr_tensor& dy, int ks_code, Wg
   p.h_stride = ((uint32_t)(halo_rows + 16) * CH * 2 + 1023u) & ~1023u;  // + slack rows read by discarded atoms
   out->grid = p.n_combo * p.ctas_per_combo;
   const size_t pslot = (size_t)kWTileH * kWTileW * PC * 2;
+  // barriers (full / empty of both rings, zero, done) and the TMEM address.  One more barrier per slot of each ring stays reserved:
+  // the halo-ring depths of the tuned layer shapes were measured with a tail of this size.
   const size_t tailb = (3 * kMaxHStages + 3 * (ks + kPSpare) + 2) * 8 + 16;
   const size_t fixed = 1024 + (((size_t)(ks + kPSpare + ks - 1) * pslot + 1023) & ~size_t(1023)) + tailb;
   {
@@ -750,10 +650,10 @@ size_t rehr_conv3d_wgrad_march_workspace(const rehr_tensor* x, const rehr_tensor
 }
 
 // dw: f32 [cout][x->c][ks^3] (ks = 1: planar k(1,3,3) layer, dw [cout][x->c][9]); `cout` <= dy->c lets the caller pass a dy zero-padded to a multiple of 16 channels.
-static int wgrad_march_impl(const rehr_tensor* x, const float* norm, const rehr_tensor* dy, int ks, int cout, float* dw, int accumulate,
-                            void* ws, size_t ws_bytes, rehr_stream stream_) {
+int rehr_conv3d_wgrad_march(const rehr_tensor* x, const rehr_tensor* dy, int ks, int cout, float* dw, int accumulate, void* ws,
+                            size_t ws_bytes, rehr_stream stream_) {
   if (!x || !dy || !x->ptr || !dy->ptr || !dw || cout <= 0 || cout > dy->c) return REHR_BAD_SHAPE;
-  if (dy->dtype != REHR_BF16 || (!norm && x->dtype != REHR_BF16)) return REHR_UNSUPPORTED;  // one MMA, one 16-bit format
+  if (dy->dtype != REHR_BF16 || x->dtype != REHR_BF16) return REHR_UNSUPPORTED;  // one MMA, one 16-bit format
   cudaStream_t stream = (cudaStream_t)stream_;
   WgmPlan pl;
   int rc = plan_wgm(*x, *dy, ks, &pl);
@@ -762,11 +662,6 @@ static int wgrad_march_impl(const rehr_tensor* x, const float* norm, const rehr_
   WgmParams& p = pl.p;
   p.ws = reinterpret_cast<float*>(ws);
   p.err = nullptr;
-  p.norm = norm;
-  p.xf_role = norm ? (pl.role == 0 ? 1 : 2) : 0;
-  p.x_f16 = x->dtype == REHR_F16;
-  p.x_c = x->c;
-  p.xd[0] = x->d; p.xh[0] = x->h; p.xw[0] = x->w;
   const rehr_tensor& hh = pl.role == 0 ? *x : *dy;
   const rehr_tensor& pp = pl.role == 0 ? *dy : *x;
   {
@@ -788,18 +683,6 @@ static int wgrad_march_impl(const rehr_tensor* x, const float* norm, const rehr_
     if (rc != REHR_OK) return rc;
   }
   return wgm_run(pl, x->c, cout, dw, accumulate, nullptr, nullptr, stream);
-}
-
-int rehr_conv3d_wgrad_march(const rehr_tensor* x, const rehr_tensor* dy, int ks, int cout, float* dw, int accumulate, void* ws,
-                            size_t ws_bytes, rehr_stream stream) {
-  return wgrad_march_impl(x, nullptr, dy, ks, cout, dw, accumulate, ws, ws_bytes, stream);
-}
-// x = the producing layer's RAW conv output (either 16-bit format); its InstanceNorm + LeakyReLU (norm = f32 [n][3][x->c]: scale,
-// shift, slope) is applied while the tiles sit in shared memory and the operand is written as bf16 (see csrc/conv_march.cu)
-int rehr_conv3d_wgrad_march_norm(const rehr_tensor* x, const float* norm, const rehr_tensor* dy, int ks, int cout, float* dw,
-                                 int accumulate, void* ws, size_t ws_bytes, rehr_stream stream) {
-  if (!norm) return REHR_BAD_SHAPE;
-  return wgrad_march_impl(x, norm, dy, ks, cout, dw, accumulate, ws, ws_bytes, stream);
 }
 
 // ---- weight gradient of a k3 / pad 1 conv with strides in {1, 2}: one marching pass per parity class of X -------------------
@@ -832,10 +715,10 @@ size_t rehr_conv3d_wgrad_march_s2_workspace(const rehr_conv_desc* d, const rehr_
   if (wgm_s2_plan(d, x, dy, &pl) != REHR_OK) return 0;
   return pl.ws_bytes;
 }
-static int wgrad_march_s2_impl(const rehr_conv_desc* d, const rehr_tensor* x, const float* norm, const rehr_tensor* dy, float* dw,
-                               int accumulate, void* ws, size_t ws_bytes, rehr_stream stream_) {
+int rehr_conv3d_wgrad_march_s2(const rehr_conv_desc* d, const rehr_tensor* x, const rehr_tensor* dy, float* dw, int accumulate,
+                               void* ws, size_t ws_bytes, rehr_stream stream_) {
   if (!x || !dy || !x->ptr || !dy->ptr || !dw) return REHR_BAD_SHAPE;
-  if (dy->dtype != REHR_BF16 || (!norm && x->dtype != REHR_BF16)) return REHR_UNSUPPORTED;
+  if (dy->dtype != REHR_BF16 || x->dtype != REHR_BF16) return REHR_UNSUPPORTED;
   cudaStream_t stream = (cudaStream_t)stream_;
   WgmPlan pl;
   int rc = wgm_s2_plan(d, x, dy, &pl);
@@ -856,10 +739,6 @@ static int wgrad_march_s2_impl(const rehr_conv_desc* d, const rehr_tensor* x, co
   }
   pl.p.ws = reinterpret_cast<float*>(ws);
   pl.p.err = nullptr;
-  pl.p.norm = norm;
-  pl.p.xf_role = norm ? 1 : 0;   // the class views of X are always the halo operand (wgm_s2_plan forces role 0)
-  pl.p.x_f16 = x->dtype == REHR_F16;
-  pl.p.x_c = x->c;
   // all parity classes in ONE launch: class c owns the CTAs [cls_begin[c], cls_begin[c + 1]), sized by its MMA count
   WgmParams& p = pl.p;
   int n_cls = 0, cost[8], cls_r[8][3];
@@ -899,7 +778,6 @@ static int wgrad_march_s2_impl(const rehr_conv_desc* d, const rehr_tensor* x, co
             gmask |= 1 << (pl.CH == 64 ? a / 2 : oh);
           }
         p.cls_gmask[n_cls] = gmask;
-        p.xd[n_cls] = ext[0]; p.xh[n_cls] = ext[1]; p.xw[n_cls] = ext[2];
         cost[n_cls] = __builtin_popcount(gmask);
         for (int a = 0; a < 3; ++a) cls_r[n_cls][a] = r[a];
         ++n_cls;
@@ -930,16 +808,6 @@ static int wgrad_march_s2_impl(const rehr_conv_desc* d, const rehr_tensor* x, co
     if (rc != REHR_OK) return rc;
   }
   return REHR_OK;
-}
-
-int rehr_conv3d_wgrad_march_s2(const rehr_conv_desc* d, const rehr_tensor* x, const rehr_tensor* dy, float* dw, int accumulate,
-                               void* ws, size_t ws_bytes, rehr_stream stream) {
-  return wgrad_march_s2_impl(d, x, nullptr, dy, dw, accumulate, ws, ws_bytes, stream);
-}
-int rehr_conv3d_wgrad_march_s2_norm(const rehr_conv_desc* d, const rehr_tensor* x, const float* norm, const rehr_tensor* dy, float* dw,
-                                    int accumulate, void* ws, size_t ws_bytes, rehr_stream stream) {
-  if (!norm) return REHR_BAD_SHAPE;
-  return wgrad_march_s2_impl(d, x, norm, dy, dw, accumulate, ws, ws_bytes, stream);
 }
 
 }  // extern "C"

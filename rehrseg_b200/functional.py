@@ -26,7 +26,7 @@ Triple = Tuple[int, int, int]
 # launch accounting (bench.py reports `gpu_launches`)
 # --------------------------------------------------------------------------------------------------
 _launches = 0
-path_hits = {"tconv_bias_from_epilogue_sums": 0, "tconv_twin_from_epilogue": 0, "in_bwd_sums_from_dgrad_epilogue": 0}   # which fused shortcuts really ran (tests read this)
+path_hits = {"tconv_bias_from_epilogue_sums": 0, "tconv_twin_from_epilogue": 0}   # which fused shortcuts really ran (tests read this)
 
 
 def launches() -> int:
@@ -106,7 +106,6 @@ class _timed:
 # a weight-gradient GEMM (activation x bf16 gradient) needs a bf16 copy of the activation: `_rehr_bf` holds that twin, written
 # by the same pass that writes the fp16 activation.
 FWD_FP16 = os.environ.get("REHR_FWD_DTYPE", "fp16").lower() != "bf16"
-Y_FP16 = True   # storage of the pre-normalisation conv output y (never an MMA operand; consumed by the InstanceNorm kernels)
 
 
 def is_h(t) -> bool:
@@ -123,7 +122,6 @@ def mark_h(t: torch.Tensor, twin: Optional[torch.Tensor] = None) -> torch.Tensor
 
 def to_float(t: torch.Tensor) -> torch.Tensor:
     """fp32 values of an engine activation (channels-last, either storage format) -- for tests and debugging."""
-    t = plain_h(t)
     h = is_h(t)
     t = t.detach()
     return t.view(torch.float16).float() if h else t.float()
@@ -140,64 +138,15 @@ def convert16_raw(x: torch.Tensor, x_h: bool, out_h: bool, out: Optional[torch.T
     return out
 
 
-# Deferred normalisation ("normalise on load").  With DEFER_NORM a Conv -> InstanceNorm -> LeakyReLU block does not run the
-# normalise pass at all: it hands its consumer the RAW fp16 conv output y together with the per-(sample, channel) triples
-# (scale, shift, slope) of its InstanceNorm + LeakyReLU (`_rehr_norm`, f32 [n][3][C]).  Consumers with an on-load path (the marching
-# forward / weight-gradient kernels) apply lrelu(y*scale + shift) to the tile in shared memory; every other consumer calls
-# `operand()`, which materialises the activation once (cached on the tensor object) in the format(s) it asks for.
-# Measured on B200 (profiles/r02_norm_on_load_microbench.txt): the marching kernels are bound by shared-memory operand reads, so
-# the in-place rewrite of every landed plane (one extra read + write of the plane) costs 9-19 % of those kernels and the
-# arithmetic another ~15 %, which cancels the saved normalise passes (C1 step 13.0 ms materialised vs 13.4-13.7 ms deferred).
-# The path stays available (REHR_DEFER_NORM=1; it also halves the activation memory: only y is kept per layer) but is off.
-DEFER_NORM = FWD_FP16 and os.environ.get("REHR_DEFER_NORM", "0") == "1"
-
-
-def norm_of(t) -> Optional[torch.Tensor]:
-    """The (scale, shift, slope) table of a deferred activation, or None if `t` holds plain values."""
-    return getattr(t, "_rehr_norm", None)
-
-
-def operand(t: torch.Tensor, want_h: bool = False, want_bf: bool = False):
-    """(values of `t` as an fp16-payload tensor or None, as a bf16 tensor or None), materialising / converting at most once per
-    format.  `want_h` on a plain bf16 tensor returns it unchanged in the second slot (its consumer then runs bf16 operands)."""
-    norm = norm_of(t)
-    if norm is None:
-        if not is_h(t):
-            return None, as_cl(t)
-        tw = getattr(t, "_rehr_bf", None)
-        if want_bf and tw is None:
-            tw = convert16_raw(t, True, False)
-            t._rehr_bf = tw
-        return (as_cl(t) if want_h else None), (tw if want_bf else None)
-    mat = t.__dict__.setdefault("_rehr_mat", {})
-    need_h, need_bf = want_h and "h" not in mat, want_bf and "bf" not in mat
-    if need_h or need_bf:
-        y = as_cl(t)
-        outs = [torch.empty(y.shape, dtype=torch.bfloat16, device=y.device) for _ in range(int(need_h) + int(need_bf))]
-        fmts = ([True] if need_h else []) + ([False] if need_bf else [])
-        yt = rt(y, True)
-        ots = [rt(o, f) for o, f in zip(outs, fmts)]
-        check(lib().rehr_norm_apply(C.byref(yt), ptr(norm), C.byref(ots[0]), C.byref(ots[1]) if len(ots) > 1 else None, stream_ptr()),
-              "norm_apply")
-        _count()
-        for o, f in zip(outs, fmts):
-            mat["h" if f else "bf"] = o
-    return (mat.get("h") if want_h else None), (mat.get("bf") if want_bf else None)
-
-
 def bf_twin(t: torch.Tensor) -> torch.Tensor:
-    """The bf16 operand of `t` for a weight-gradient GEMM: `t` itself unless its payload is fp16, then its twin (converted /
-    materialised on the spot if the producer did not write one, e.g. a frozen producer feeding a trainable consumer)."""
-    return operand(t, want_bf=True)[1]
-
-
-def plain_h(t: torch.Tensor) -> torch.Tensor:
-    """`t` with plain (normalised) values in its own 16-bit format: deferred activations are materialised (fp16 payload,
-    marked), everything else passes through.  For consumers without an on-load path that read ONE operand."""
-    if norm_of(t) is None:
-        return t
-    h, _ = operand(t, want_h=True)
-    return mark_h(h)
+    """The bf16 operand of `t` for a weight-gradient GEMM: `t` itself unless its payload is fp16, then its twin (converted on
+    the spot and cached on `t` if the producer did not write one, e.g. a frozen producer feeding a trainable consumer)."""
+    if not is_h(t):
+        return as_cl(t)
+    tw = getattr(t, "_rehr_bf", None)
+    if tw is None:
+        tw = t._rehr_bf = convert16_raw(t, True, False)
+    return tw
 
 
 # --------------------------------------------------------------------------------------------------
@@ -525,11 +474,10 @@ def join_pending_wgrad() -> None:
     _wgrad_pending.clear()
 
 
-def _dgrad_and_wgrad(x, dy, weight, wshape, kernel, stride, padding, need_dx: bool, cache: bool = True, norm=None, x_h=False,
-                     want_chsum: bool = False, inred=None):
+def _dgrad_and_wgrad(x, dy, weight, wshape, kernel, stride, padding, need_dx: bool, cache: bool = True, want_chsum: bool = False):
     """(dx or None, dw) of a conv.  The weight-gradient chain runs on a side stream (events only: graph-capturable): joined right
     after the input gradient for small layers (two latency-bound chains side by side), or -- WGRAD_DEFER_JOIN, inside an autograd
-    backward pass -- at the end of the pass.  `norm` / `x_h`: x is a raw conv output normalised on load (conv3d_wgrad_raw)."""
+    backward pass -- at the end of the pass."""
     voxels = dy.shape[0] * dy.shape[1] * dy.shape[2] * dy.shape[3]
     side_ok = need_dx and WGRAD_SIDE_STREAM and _ktimer is None
     if side_ok and (WGRAD_DEFER_JOIN or voxels <= WGRAD_SIDE_MAX_VOXELS):
@@ -540,13 +488,13 @@ def _dgrad_and_wgrad(x, dy, weight, wshape, kernel, stride, padding, need_dx: bo
             # InstanceNorm passes depend on it -- and the weight gradient is made to WAIT for it (fork point after the launch):
             # inside a replayed CUDA graph two independent branches start in no particular order, a dependency is the only
             # way to fix it.  The InstanceNorm passes then run next to the weight gradient.
-            dx = conv3d_dgrad_raw(dy, weight, x.shape, kernel, stride, padding, cache=cache, want_chsum=want_chsum, inred=inred)
+            dx = conv3d_dgrad_raw(dy, weight, x.shape, kernel, stride, padding, cache=cache, want_chsum=want_chsum)
             with fk:
-                conv3d_wgrad_raw(x, dy, wshape, kernel, stride, padding, out=dw, norm=norm, x_h=x_h)
+                conv3d_wgrad_raw(x, dy, wshape, kernel, stride, padding, out=dw)
         else:
             with fk:
-                conv3d_wgrad_raw(x, dy, wshape, kernel, stride, padding, out=dw, norm=norm, x_h=x_h)
-            dx = conv3d_dgrad_raw(dy, weight, x.shape, kernel, stride, padding, cache=cache, want_chsum=want_chsum, inred=inred)
+                conv3d_wgrad_raw(x, dy, wshape, kernel, stride, padding, out=dw)
+            dx = conv3d_dgrad_raw(dy, weight, x.shape, kernel, stride, padding, cache=cache, want_chsum=want_chsum)
         deferred = False
         # a leaf parameter without a .grad: AccumulateGrad adopts dw without touching it (a view of a parameter, e.g. FLAVR's 2-D
         # fuse convs seen as 5-D, sends dw through a ViewBackward first: joined per layer)
@@ -554,15 +502,15 @@ def _dgrad_and_wgrad(x, dy, weight, wshape, kernel, stride, padding, need_dx: bo
             try:
                 if not _wgrad_pending:
                     torch.autograd.Variable._execution_engine.queue_callback(join_pending_wgrad)
-                _wgrad_pending.append((fk, (x, dy, norm)))   # NOT dw: an extra reference would force AccumulateGrad to clone it
+                _wgrad_pending.append((fk, (x, dy)))   # NOT dw: an extra reference would force AccumulateGrad to clone it
                 deferred = True
             except RuntimeError:      # not inside a backward pass: nobody would join later
                 deferred = False
         if not deferred:
             fk.join()
         return dx, dw
-    dx = conv3d_dgrad_raw(dy, weight, x.shape, kernel, stride, padding, cache=cache, want_chsum=want_chsum, inred=inred) if need_dx else None
-    return dx, conv3d_wgrad_raw(x, dy, wshape, kernel, stride, padding, norm=norm, x_h=x_h)
+    dx = conv3d_dgrad_raw(dy, weight, x.shape, kernel, stride, padding, cache=cache, want_chsum=want_chsum) if need_dx else None
+    return dx, conv3d_wgrad_raw(x, dy, wshape, kernel, stride, padding)
 
 
 MARCH_MAX_WIDE = int(os.environ.get("REHR_MARCH_MAX_WIDE", "128"))
@@ -612,11 +560,9 @@ def _ws(nbytes: int, device) -> torch.Tensor:
 # --------------------------------------------------------------------------------------------------
 def conv3d_raw(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], kernel: Triple, stride: Triple,
                padding: Triple, act: int = ACT_NONE, slope: float = 0.0, want_stats: bool = False,
-               out_f32: bool = False, out: Optional[torch.Tensor] = None, x_h: bool = False, y_h: bool = False,
-               norm: Optional[torch.Tensor] = None, op_h: bool = False):
+               out_f32: bool = False, out: Optional[torch.Tensor] = None, x_h: bool = False, y_h: bool = False):
     """y = act(conv3d(x) + bias) on NDHWC 16-bit `x`; optionally per-tile InstanceNorm partial sums.  `x_h` / `y_h`: the payload
-    of x / y is fp16 (the weights are packed in x's format).  `norm`: x is a RAW conv output normalised on load (marching
-    kernel only, see norm_onload_fwd_ok) into an operand of format `op_h`.  Returns (y, stats_partial or None, tiles)."""
+    of x / y is fp16 (the weights are packed in x's format).  Returns (y, stats_partial or None, tiles)."""
     x = as_cl(x)
     n, d, h, w, cin = x.shape
     cout = weight.shape[0]
@@ -634,22 +580,12 @@ def conv3d_raw(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tenso
         if want_stats:
             tiles = lib().rehr_conv3d_march_stats_tiles(C.byref(xt), C.byref(yt), int(kernel[0]))
             stats = torch.empty((n, tiles, cout, 2), dtype=torch.float32, device=x.device)
-        if norm is not None:
-            wp = _packed(weight, "march_fwd", h=op_h)
-            with _timed("conv_march_kernel", flops, tag):
-                check(lib().rehr_conv3d_march_fwd_norm(C.byref(xt), ptr(norm), L.F16 if op_h else L.BF16, ptr(wp), ptr(_f32(bias)),
-                                                       C.byref(yt), int(kernel[0]), int(out_f32), act, float(slope), ptr(stats),
-                                                       stream_ptr()), "conv3d_march_fwd_norm")
-            _count()
-            return out, stats, tiles
         wp = _packed(weight, "march_fwd", h=x_h)
         with _timed("conv_march_kernel", flops, tag):
             check(lib().rehr_conv3d_march_fwd(C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt), int(kernel[0]), int(out_f32), act,
                                               float(slope), ptr(stats), stream_ptr()), "conv3d_march_fwd")
         _count()
         return out, stats, tiles
-    if norm is not None:
-        raise L.RehrError("conv3d_raw(norm=...): this layer has no normalise-on-load path (check norm_onload_fwd_ok first)")
     if want_stats:
         tiles = lib().rehr_conv3d_stats_tiles(C.byref(yt))
         if tiles > 0:
@@ -676,29 +612,8 @@ def instnorm_stats_raw(y: torch.Tensor, y_h: bool = False):
     return stats, tiles
 
 
-# Fused InstanceNorm-backward sums.  When the input of a stride-1 marching conv is the activation of a Conv -> InstanceNorm ->
-# LeakyReLU block, the conv's input-gradient epilogue also accumulates that block's backward sums (sum g, sum g*y) from its fp32
-# accumulators (rehr_conv3d_march_dgrad_inred), so the block's stand-alone reduce pass over dA and y does not run.  The producer
-# advertises what the epilogue needs on its output tensor (`_rehr_prod`), the result carries the partial sums (`_rehr_insums`).
-# Measured on the C1 step (tools/ab_step.py, tools/timeline.py) and left OFF: the extra epilogue work (y row + 24 table loads + 5
-# operations per accumulator) makes the drain of a plane longer than its MMAs on the 32-channel layers -- the 32<-32 @128^3 input
-# gradient goes from 256 to 430 us to save a 113 us reduce pass that mostly hides behind the weight gradient anyway; 64<-64 @64^3
-# 124 -> 150 us for a 31 us pass; step 12.17 ms off vs 12.25-12.35 ms on.  Kept as a tested path (REHR_INRED=1) for layers with
-# long K loops, where the four drain warps have the slack.
-INRED = os.environ.get("REHR_INRED", "0") == "1"
-
-
-class _Prod:
-    """What a ConvNormAct block leaves on its activation for a fusing consumer: y (pre-normalisation), its format, the f32
-    [n][3][c] (scale, shift, slope) table."""
-    __slots__ = ("y", "y_h", "norm")
-
-    def __init__(self, y, y_h, norm):
-        self.y, self.y_h, self.norm = y, y_h, norm
-
-
 def conv3d_dgrad_raw(dy: torch.Tensor, weight: torch.Tensor, in_shape: Sequence[int], kernel: Triple, stride: Triple,
-                     padding: Triple, cache: bool = True, want_chsum: bool = False, inred: Optional[_Prod] = None) -> torch.Tensor:
+                     padding: Triple, cache: bool = True, want_chsum: bool = False) -> torch.Tensor:
     """dx = conv^T(dy).  `want_chsum`: where the marching kernel runs, its epilogue also leaves the per-(sample, tile, channel) sums
     of the fp32 accumulators on the result (`dx._rehr_chsum`, f32 [n][tiles][cin][2]): the bias gradient of a transposed conv
     that produced (part of) the conv's input then needs no pass over dx."""
@@ -712,18 +627,6 @@ def conv3d_dgrad_raw(dy: torch.Tensor, weight: torch.Tensor, in_shape: Sequence[
         wp = _packed(weight, "march_dgrad", cache)
         dyt, dxt = rt(dy), rt(dx)
         stats = None
-        if inred is not None and not want_chsum and tuple(inred.y.shape) == tuple(dx.shape) \
-                and lib().rehr_conv3d_march_dgrad_inred_supported(C.byref(desc), dy.shape[4], cin):
-            tiles = lib().rehr_conv3d_march_stats_tiles(C.byref(dyt), C.byref(dxt), int(kernel[0]))
-            stats = torch.empty((n, tiles, cin, 2), dtype=torch.float32, device=dy.device)
-            ypt = rt(inred.y, inred.y_h)
-            with _timed("conv_march_kernel", flops, tag):
-                check(lib().rehr_conv3d_march_dgrad_inred(C.byref(dyt), ptr(wp), C.byref(dxt), int(kernel[0]), C.byref(ypt),
-                                                          ptr(inred.norm), ptr(stats), stream_ptr()), "conv3d_march_dgrad_inred")
-            _count()
-            dx._rehr_insums = (stats, tiles, inred.y.data_ptr())
-            path_hits["in_bwd_sums_from_dgrad_epilogue"] = path_hits.get("in_bwd_sums_from_dgrad_epilogue", 0) + 1
-            return dx
         if want_chsum:
             tiles = lib().rehr_conv3d_march_stats_tiles(C.byref(dyt), C.byref(dxt), int(kernel[0]))
             stats = torch.empty((n, tiles, cin, 2), dtype=torch.float32, device=dy.device)
@@ -756,64 +659,49 @@ def conv3d_dgrad_raw(dy: torch.Tensor, weight: torch.Tensor, in_shape: Sequence[
     return dx
 
 
-def norm_onload_fwd_ok(kernel: Triple, stride: Triple, padding: Triple, cin: int, cout: int) -> bool:
-    """True if the forward conv of this layer can normalise its input on load (marching kernel, output tile <= 32 channels)."""
-    desc = conv_desc(kernel, stride, padding)
-    return bool(USE_MARCH and lib().rehr_conv3d_march_norm_supported(C.byref(desc), int(cin), int(cout)))
-
-
-def wgrad_route(x_shape, dy_shape, kernel: Triple, stride: Triple, padding: Triple) -> str:
-    """Which kernel conv3d_wgrad_raw will pick for these (channels-last) shapes: 'march' and 'march_s2' can normalise x on load."""
-    desc = conv_desc(kernel, stride, padding)
-    xt = L.RehrTensor(0, *[int(v) for v in x_shape], int(x_shape[4]), 0)
-    dyt = L.RehrTensor(0, *[int(v) for v in dy_shape], int(dy_shape[4]), 0)
+def _wgrad_route(desc, xt, dyt) -> str:
     if USE_MARCH and lib().rehr_conv3d_wgrad_march_supported(C.byref(desc), C.byref(xt), C.byref(dyt)):
         return "march"
-    if USE_MARCH and dy_shape[0] * dy_shape[1] * dy_shape[2] * dy_shape[3] >= S2_WGRAD_MARCH_MIN_VOXELS \
+    # one marching pass per parity class of x; its fixed cost (TMEM drain + partial reduction per class) only pays off on
+    # the full-resolution stage-entry conv (measured: 32->64 @128^3 0.86 -> 0.57 ms, 64->128 @64^3 0.14 -> 0.48 ms)
+    if USE_MARCH and dyt.n * dyt.d * dyt.h * dyt.w >= S2_WGRAD_MARCH_MIN_VOXELS \
             and lib().rehr_conv3d_wgrad_march_s2_supported(C.byref(desc), C.byref(xt), C.byref(dyt)):
         return "march_s2"
     return "generic"
 
 
+def wgrad_route(x_shape, dy_shape, kernel: Triple, stride: Triple, padding: Triple) -> str:
+    """Which kernel conv3d_wgrad_raw picks for these (channels-last, unpitched) shapes: 'march', 'march_s2' or 'generic'."""
+    xt = L.RehrTensor(0, *[int(v) for v in x_shape], int(x_shape[4]), 0)
+    dyt = L.RehrTensor(0, *[int(v) for v in dy_shape], int(dy_shape[4]), 0)
+    return _wgrad_route(conv_desc(kernel, stride, padding), xt, dyt)
+
+
 def conv3d_wgrad_raw(x: torch.Tensor, dy: torch.Tensor, wshape: Sequence[int], kernel: Triple, stride: Triple,
-                     padding: Triple, out: Optional[torch.Tensor] = None, norm: Optional[torch.Tensor] = None,
-                     x_h: bool = False) -> torch.Tensor:
-    """`norm`: x is a RAW conv output (payload format `x_h`) normalised on load -- marching kernels only (see wgrad_route)."""
+                     padding: Triple, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     x, dy = as_cl(x), as_cl(dy)
     dw = out if out is not None else torch.empty(tuple(wshape), dtype=torch.float32, device=x.device)
     desc = conv_desc(kernel, stride, padding)
-    xt, dyt = rt(x, x_h), rt(dy)
+    xt, dyt = rt(x), rt(dy)
     flops = 2.0 * dy.shape[0] * dy.shape[1] * dy.shape[2] * dy.shape[3] * dy.shape[4] * x.shape[4] * kernel[0] * kernel[1] * kernel[2]
     tag = f"wgrad {x.shape[4]}->{dy.shape[4]} in{x.shape[1]}x{x.shape[2]}x{x.shape[3]} k{kernel} s{stride}" if _ktimer is not None else ""
-    if USE_MARCH and lib().rehr_conv3d_wgrad_march_supported(C.byref(desc), C.byref(xt), C.byref(dyt)):
+    route = _wgrad_route(desc, xt, dyt)
+    if route == "march":
         need = lib().rehr_conv3d_wgrad_march_workspace(C.byref(xt), C.byref(dyt), int(kernel[0]))
         ws = _ws(need, x.device)
         with _timed("wgrad_march_kernel", flops, tag):
-            if norm is not None:
-                check(lib().rehr_conv3d_wgrad_march_norm(C.byref(xt), ptr(norm), C.byref(dyt), int(kernel[0]), int(wshape[0]), ptr(dw),
-                                                         0, ptr(ws), need, stream_ptr()), "conv3d_wgrad_march_norm")
-            else:
-                check(lib().rehr_conv3d_wgrad_march(C.byref(xt), C.byref(dyt), int(kernel[0]), int(wshape[0]), ptr(dw), 0, ptr(ws),
-                                                    need, stream_ptr()), "conv3d_wgrad_march")
+            check(lib().rehr_conv3d_wgrad_march(C.byref(xt), C.byref(dyt), int(kernel[0]), int(wshape[0]), ptr(dw), 0, ptr(ws),
+                                                need, stream_ptr()), "conv3d_wgrad_march")
         _count(2)
         return dw
-    if USE_MARCH and dy.shape[0] * dy.shape[1] * dy.shape[2] * dy.shape[3] >= S2_WGRAD_MARCH_MIN_VOXELS \
-            and lib().rehr_conv3d_wgrad_march_s2_supported(C.byref(desc), C.byref(xt), C.byref(dyt)):
-        # one marching pass per parity class of x; its fixed cost (TMEM drain + partial reduction per class) only pays off on
-        # the full-resolution stage-entry conv (measured: 32->64 @128^3 0.86 -> 0.57 ms, 64->128 @64^3 0.14 -> 0.48 ms)
+    if route == "march_s2":
         need = lib().rehr_conv3d_wgrad_march_s2_workspace(C.byref(desc), C.byref(xt), C.byref(dyt))
         ws = _ws(need, x.device)
         with _timed("wgrad_march_kernel", flops, tag):
-            if norm is not None:
-                check(lib().rehr_conv3d_wgrad_march_s2_norm(C.byref(desc), C.byref(xt), ptr(norm), C.byref(dyt), ptr(dw), 0, ptr(ws),
-                                                            need, stream_ptr()), "conv3d_wgrad_march_s2_norm")
-            else:
-                check(lib().rehr_conv3d_wgrad_march_s2(C.byref(desc), C.byref(xt), C.byref(dyt), ptr(dw), 0, ptr(ws), need,
-                                                       stream_ptr()), "conv3d_wgrad_march_s2")
+            check(lib().rehr_conv3d_wgrad_march_s2(C.byref(desc), C.byref(xt), C.byref(dyt), ptr(dw), 0, ptr(ws), need,
+                                                   stream_ptr()), "conv3d_wgrad_march_s2")
         _count(2 * stride[0] * stride[1] * stride[2])
         return dw
-    if norm is not None:
-        raise L.RehrError("conv3d_wgrad_raw(norm=...): this layer has no normalise-on-load path (check wgrad_route first)")
     need = lib().rehr_conv3d_wgrad_workspace(C.byref(desc), C.byref(xt), C.byref(dyt))
     if need == 0:
         raise L.RehrError(f"conv3d_wgrad: unsupported configuration x={tuple(x.shape)} dy={tuple(dy.shape)}")
@@ -854,14 +742,9 @@ def act_bwd_raw(a: torch.Tensor, da: torch.Tensor, act: int, slope: float, a_h: 
 # constructed at models/seg_model.py:174-191 with the ops chosen at train_all.py:474-493)
 # --------------------------------------------------------------------------------------------------
 class ConvNormAct(torch.autograd.Function):
-    """Two output modes.
-    * DEFER_NORM (default): returns the RAW fp16 conv output y and the (scale, shift, slope) table of this block's InstanceNorm +
-      LeakyReLU; the normalise pass does not run -- consumers apply it on their operand path or materialise it (see `operand`).
-    * otherwise: returns the activation `a` (format FWD_FP16) and, when a gradient will be needed, its bf16 twin `a2` (the
-      weight-gradient operand of the consumer; written by the same normalise pass).
-    The second / third outputs are non-differentiable side tensors; the gradient of output 0 is always d(loss)/d(activation)."""
-
-    last_prod = None   # set by forward for the wrapper (conv_norm_act) to hang on the returned activation
+    """Returns the activation `a` (format FWD_FP16) and, when a gradient will be needed, its bf16 twin `a2` (the weight-gradient
+    operand of the consumer; written by the same normalise pass).  `a2` is a non-differentiable side tensor; the gradient of
+    output 0 is d(loss)/d(activation)."""
 
     @staticmethod
     def forward(ctx, x, weight, bias, gamma, beta, kernel, stride, padding, eps, slope, small_cin, cat_room):
@@ -869,11 +752,8 @@ class ConvNormAct(torch.autograd.Function):
         cout = weight.shape[0]
         desc = conv_desc(kernel, stride, padding)
         a_h = FWD_FP16
-        y_h = Y_FP16
-        defer = DEFER_NORM
         train = any(ctx.needs_input_grad)
-        ctx.set_materialize_grads(False)   # side outputs are non-differentiable: no zero-filled gradient tensors for them
-        x_norm, x_raw_h = None, False
+        ctx.set_materialize_grads(False)   # the twin output is non-differentiable: no zero-filled gradient tensor for it
 
         def alloc(shape5):
             if cat_room:
@@ -883,13 +763,15 @@ class ConvNormAct(torch.autograd.Function):
                 return _alias(buf, cout, shape5, buf.stride())
             return torch.empty(tuple(shape5), dtype=torch.bfloat16, device=dev)
 
+        # the pre-normalisation conv output y is stored as fp16 whatever FWD_FP16 says: it is never an MMA operand, only the
+        # InstanceNorm kernels read it
         if small_cin:
             # x is the caller's NCDHW fp32 tensor (train_all.py:524)
             xs = _f32(x)
             n, cin, d, h, w = xs.shape
             od, oh, ow = (_out_size(i, k, s, p) for i, k, s, p in zip((d, h, w), kernel, stride, padding))
-            y = alloc((n, od, oh, ow, cout)) if defer else torch.empty((n, od, oh, ow, cout), dtype=torch.bfloat16, device=dev)
-            yt = rt(y, y_h)
+            y = torch.empty((n, od, oh, ow, cout), dtype=torch.bfloat16, device=dev)
+            yt = rt(y, True)
             tiles = lib().rehr_instnorm_stats_tiles(C.byref(yt))
             stats = torch.empty((n, tiles, cout, 2), dtype=torch.float32, device=dev)
             # NB the conv bias is NOT added: a per-channel constant is removed exactly by the InstanceNorm that follows
@@ -900,90 +782,43 @@ class ConvNormAct(torch.autograd.Function):
             x_saved = xs
         else:
             xc = as_cl(x)
-            n, d, h, w, cin = xc.shape
-            oshape = (n, *(_out_size(i, k, s, p) for i, k, s, p in zip((d, h, w), kernel, stride, padding)), cout)
-            out = alloc(oshape) if defer else None
-            norm_in = norm_of(x)
-            if norm_in is not None:
-                # x is a deferred activation (raw conv output + norm table): normalise on load where the kernels can
-                fwd_onload = norm_onload_fwd_ok(kernel, stride, padding, cin, cout)
-                wg_onload = train and wgrad_route(xc.shape, oshape, kernel, stride, padding) != "generic"
-                need_bf = train and not wg_onload
-                xh, xbf = operand(x, want_h=not fwd_onload, want_bf=need_bf)
-                if fwd_onload:
-                    y, stats, tiles = conv3d_raw(xc, weight, None, kernel, stride, padding, want_stats=True, x_h=True, y_h=y_h,
-                                                 out=out, norm=norm_in, op_h=a_h)
-                else:
-                    y, stats, tiles = conv3d_raw(xh, weight, None, kernel, stride, padding, want_stats=True, x_h=True, y_h=y_h, out=out)
-                if train:
-                    x_saved, x_norm, x_raw_h = (xc, norm_in, True) if wg_onload else (xbf, None, False)
-                else:
-                    x_saved = None
-            else:
-                x_saved = bf_twin(x) if train else None   # bf16 operand of this layer's weight gradient
-                y, stats, tiles = conv3d_raw(xc, weight, None, kernel, stride, padding, want_stats=True, x_h=is_h(x), y_h=y_h, out=out)
+            x_saved = bf_twin(x) if train else None   # bf16 operand of this layer's weight gradient
+            y, stats, tiles = conv3d_raw(xc, weight, None, kernel, stride, padding, want_stats=True, x_h=is_h(x), y_h=True)
         n = y.shape[0]
         vox = y.shape[1] * y.shape[2] * y.shape[3]
         mean = torch.empty((n, cout), dtype=torch.float32, device=dev)
         rstd = torch.empty((n, cout), dtype=torch.float32, device=dev)
         g32, b32 = _f32(gamma), _f32(beta)
-        ctx.cfg = (kernel, stride, padding, slope, small_cin, bias is not None, y_h, x_raw_h)
+        ctx.cfg = (kernel, stride, padding, slope, small_cin, bias is not None)
         ctx.wref = weakref.ref(weight)
         ctx.x_upcat = bool(getattr(x, "_rehr_upcat", False))   # x = [up | skip]: the transposed conv wants channel sums of dx
-        # x is the activation of another block of this kind: its backward sums come out of this conv's input-gradient epilogue
-        ctx.prod = getattr(x, "_rehr_prod", None) if (INRED and train and not small_cin and ctx.needs_input_grad[0]) else None
-        if defer:
-            ctot, coff = (2 * cout, cout) if cat_room else (cout, 0)
-            norm = torch.empty((n, 3, ctot), dtype=torch.float32, device=dev)
-            norm_own = torch.empty((n, 3, cout), dtype=torch.float32, device=dev) if cat_room else None
-            check(lib().rehr_instnorm_finalize_norm(ptr(stats), n, tiles, cout, vox, float(eps), ptr(g32), ptr(b32), float(slope),
-                                                    ptr(mean), ptr(rstd), ptr(norm), ctot, coff, ptr(norm_own), stream_ptr()),
-                  "instnorm_finalize_norm")
-            _count()
-            ctx.save_for_backward(x_saved, x_norm, weight, gamma, beta, y, mean, rstd)
-            ctx.skip_key = (y.untyped_storage().data_ptr(), y.storage_offset()) if cat_room else None
-            ctx.mark_non_differentiable(norm)
-            if norm_own is not None:
-                ctx.mark_non_differentiable(norm_own)
-            return y, norm, norm_own
-        ConvNormAct.last_prod = None
-        if INRED and train and not cat_room:
-            # same finalize, which also leaves the (scale, shift, slope) table a fusing consumer's input-gradient epilogue reads
-            ntab = torch.empty((n, 3, cout), dtype=torch.float32, device=dev)
-            check(lib().rehr_instnorm_finalize_norm(ptr(stats), n, tiles, cout, vox, float(eps), ptr(g32), ptr(b32), float(slope),
-                                                    ptr(mean), ptr(rstd), ptr(ntab), cout, 0, None, stream_ptr()), "instnorm_finalize_norm")
-            ConvNormAct.last_prod = _Prod(y, y_h, ntab)
-        else:
-            check(lib().rehr_instnorm_finalize(ptr(stats), n, tiles, cout, vox, float(eps), ptr(mean), ptr(rstd), stream_ptr()),
-                  "instnorm_finalize")
+        check(lib().rehr_instnorm_finalize(ptr(stats), n, tiles, cout, vox, float(eps), ptr(mean), ptr(rstd), stream_ptr()),
+              "instnorm_finalize")
         want_twin = a_h and train
         a = alloc(y.shape)
         a2 = alloc(y.shape) if want_twin else None
-        yt, at = rt(y, y_h), rt(a, a_h)
+        yt, at = rt(y, True), rt(a, a_h)
         a2t = rt(a2, False) if a2 is not None else None
         check(lib().rehr_instnorm_lrelu_apply(C.byref(yt), ptr(mean), ptr(rstd), ptr(g32), ptr(b32), float(slope), C.byref(at),
                                               C.byref(a2t) if a2t is not None else None, stream_ptr()), "instnorm_lrelu_apply")
         _count(2)
-        ctx.save_for_backward(x_saved, x_norm, weight, gamma, beta, y, mean, rstd)
+        ctx.save_for_backward(x_saved, weight, gamma, beta, y, mean, rstd)
         ctx.skip_key = (a.untyped_storage().data_ptr(), a.storage_offset()) if cat_room else None
         if a2 is not None:
             ctx.mark_non_differentiable(a2)
-        return a, a2, None
+        return a, a2
 
     @staticmethod
-    def backward(ctx, da, _side1=None, _side2=None):
+    def backward(ctx, da, _twin_unused=None):
         if da is None:
             return (None,) * 12
-        x, x_norm, weight, gamma, beta, y, mean, rstd = ctx.saved_tensors
+        x, weight, gamma, beta, y, mean, rstd = ctx.saved_tensors
         weight = _orig_weight(ctx, weight)
-        kernel, stride, padding, slope, small_cin, has_bias, y_h, x_raw_h = ctx.cfg
+        kernel, stride, padding, slope, small_cin, has_bias = ctx.cfg
         dev = y.device
-        da_in = da
         da = as_cl(da)
-        global _launches
         n, cout = y.shape[0], y.shape[4]
-        vox = y.shape[1] * y.shape[2] * y.shape[3]
-        yt, dat = rt(y, y_h), rt(da)
+        yt, dat = rt(y, True), rt(da)
         da2 = _skip_grads.pop(ctx.skip_key, None) if ctx.skip_key is not None else None
         da2t = rt(da2) if da2 is not None else None
         da2p = C.byref(da2t) if da2t is not None else None
@@ -992,19 +827,12 @@ class ConvNormAct(torch.autograd.Function):
         sums = torch.empty((n, cout, 2), dtype=torch.float32, device=dev)
         dgamma = torch.empty((cout,), dtype=torch.float32, device=dev)
         dbeta = torch.empty((cout,), dtype=torch.float32, device=dev)
-        ins = getattr(da_in, "_rehr_insums", None)
-        if ins is not None and da2 is None and ins[2] == y.data_ptr() and tuple(ins[0].shape) == (n, ins[1], cout, 2):
-            # the consumer's input-gradient epilogue already summed g and g*y over this block's voxels (conv3d_dgrad_raw)
-            check(lib().rehr_instnorm_lrelu_bwd_finalize_raw(ptr(ins[0]), n, ins[1], cout, ptr(mean), ptr(rstd), ptr(sums), ptr(dgamma),
-                                                             ptr(dbeta), 0, stream_ptr()), "instnorm_bwd_finalize_raw")
-            _launches -= 1
-        else:
-            tiles = lib().rehr_instnorm_stats_tiles(C.byref(yt))
-            partial = torch.empty((n, tiles, cout, 2), dtype=torch.float32, device=dev)
-            check(lib().rehr_instnorm_lrelu_bwd_reduce(C.byref(yt), C.byref(dat), da2p, ptr(mean), ptr(rstd), ptr(g32), ptr(b32),
-                                                       float(slope), ptr(partial), stream_ptr()), "instnorm_bwd_reduce")
-            check(lib().rehr_instnorm_lrelu_bwd_finalize(ptr(partial), n, tiles, cout, ptr(rstd), ptr(sums), ptr(dgamma), ptr(dbeta),
-                                                         0, stream_ptr()), "instnorm_bwd_finalize")
+        tiles = lib().rehr_instnorm_stats_tiles(C.byref(yt))
+        partial = torch.empty((n, tiles, cout, 2), dtype=torch.float32, device=dev)
+        check(lib().rehr_instnorm_lrelu_bwd_reduce(C.byref(yt), C.byref(dat), da2p, ptr(mean), ptr(rstd), ptr(g32), ptr(b32),
+                                                   float(slope), ptr(partial), stream_ptr()), "instnorm_bwd_reduce")
+        check(lib().rehr_instnorm_lrelu_bwd_finalize(ptr(partial), n, tiles, cout, ptr(rstd), ptr(sums), ptr(dgamma), ptr(dbeta),
+                                                     0, stream_ptr()), "instnorm_bwd_finalize")
         dy = torch.empty_like(y)
         dyt = rt(dy)
         check(lib().rehr_instnorm_lrelu_bwd_apply(C.byref(yt), C.byref(dat), da2p, ptr(mean), ptr(rstd), ptr(g32), ptr(b32),
@@ -1027,7 +855,7 @@ class ConvNormAct(torch.autograd.Function):
                 _count()
         else:
             dx, dw = _dgrad_and_wgrad(x, dy, weight, weight.shape, kernel, stride, padding, ctx.needs_input_grad[0],
-                                      norm=x_norm, x_h=x_raw_h, want_chsum=ctx.x_upcat, inred=ctx.prod)
+                                      want_chsum=ctx.x_upcat)
         # A per-channel constant added before InstanceNorm is removed by the mean subtraction: d(loss)/d(bias) == 0
         # exactly (PyTorch's value is rounding noise of the same sum).
         dbias = _zero_grad_slice(cout, dev) if has_bias else None
@@ -1037,25 +865,14 @@ class ConvNormAct(torch.autograd.Function):
 
 def conv_norm_act(x, weight, bias, gamma, beta, kernel, stride, padding, eps=1e-5, slope=0.01, small_cin=False,
                   cat_room=False):
-    a, s1, s2 = ConvNormAct.apply(x, weight, bias, gamma, beta, tuple(kernel), tuple(stride), tuple(padding), float(eps),
-                                  float(slope), bool(small_cin), bool(cat_room))
-    if DEFER_NORM:
-        # `a` is the raw conv output; s1 = the norm table of the whole buffer it lives in ([up | skip] for cat_room), s2 = the
-        # table of its own channels alone (cat_room only)
-        mark_h(a)
-        a._rehr_norm = s2 if cat_room else s1
-        if cat_room:
-            a._rehr_cat = (2 * weight.shape[0], weight.shape[0])
-            a._rehr_norm_cat = s1
-        return a
+    a, a2 = ConvNormAct.apply(x, weight, bias, gamma, beta, tuple(kernel), tuple(stride), tuple(padding), float(eps),
+                              float(slope), bool(small_cin), bool(cat_room))
     if FWD_FP16:
-        mark_h(a, s1)
-    if ConvNormAct.last_prod is not None:
-        a._rehr_prod, ConvNormAct.last_prod = ConvNormAct.last_prod, None
+        mark_h(a, a2)
     if cat_room:
         a._rehr_cat = (2 * weight.shape[0], weight.shape[0])
-        if s1 is not None:
-            s1._rehr_cat = a._rehr_cat
+        if a2 is not None:
+            a2._rehr_cat = a._rehr_cat
     return a
 
 
@@ -1254,12 +1071,8 @@ class ConvTranspose(torch.autograd.Function):
         x_h = is_h(x)
         train = any(ctx.needs_input_grad)
         ctx.set_materialize_grads(False)          # no zero-filled gradient for the non-differentiable twin output
-        # forward operand (fp16 payload where the producer used fp16; a deferred activation is materialised here: the tapped GEMM
-        # has no on-load path) and the bf16 operand of the weight gradient, produced by one pass when both are missing
-        xh, x_bf = operand(x, want_h=x_h, want_bf=train or not x_h)
-        x = xh if x_h else x_bf
-        if not train:
-            x_bf = None
+        x_bf = bf_twin(x) if train else None      # the bf16 operand of the weight gradient
+        x = as_cl(x)
         n, d, h, w, cin = x.shape
         cout = weight.shape[1]
         od, oh, ow = ((i - 1) * s - 2 * p + k for i, k, s, p in zip((d, h, w), kernel, stride, padding))
@@ -1267,7 +1080,6 @@ class ConvTranspose(torch.autograd.Function):
         ctx.cat = skip is not None
         ctx.skip_key = None
         full2 = None
-        skip_deferred = False
 
         def whole(t):   # the [up | skip] buffer a cat_room activation lives in
             tot, off = t._rehr_cat
@@ -1282,7 +1094,6 @@ class ConvTranspose(torch.autograd.Function):
                 raise L.RehrError("conv_transpose: input and skip use different 16-bit storage formats")
             full = whole(skip)
             y = full[..., :cout]
-            skip_deferred = norm_of(skip) is not None
         else:
             full = None
             y = torch.empty((n, od, oh, ow, cout), dtype=torch.bfloat16, device=x.device)
@@ -1290,7 +1101,7 @@ class ConvTranspose(torch.autograd.Function):
         twin_done = False
         if lib().rehr_convtranspose3d_fused_supported(C.byref(desc), cin, cout):
             wp = _packed(weight, "tconv_fused", h=x_h)  # [T][Cout][Cin]
-            tw = getattr(skip, "_rehr_bf", None) if (skip is not None and x_h and train and not skip_deferred) else None
+            tw = getattr(skip, "_rehr_bf", None) if (skip is not None and x_h and train) else None
             if tw is not None and getattr(tw, "_rehr_cat", None) == skip._rehr_cat:
                 # the bf16 twin of the up-sampled half goes straight into the twin's [up | skip] buffer from the same epilogue
                 full2 = whole(tw)
@@ -1308,7 +1119,7 @@ class ConvTranspose(torch.autograd.Function):
             check(lib().rehr_convtranspose3d_fwd(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt), act,
                                                  float(slope), stream_ptr()), "convtranspose3d_fwd")
             _count(stride[0] * stride[1] * stride[2])
-        if x_h and train and not skip_deferred and not twin_done:
+        if x_h and train and not twin_done:
             # bf16 twin of the result for the weight-gradient GEMM of the consumer: the skip half already has one (written by
             # the skip's normalise pass), the up-sampled half is converted here
             if skip is not None:
@@ -1397,10 +1208,6 @@ def conv_transpose(x, weight, bias, kernel, stride, padding=(0, 0, 0), act=ACT_N
         mark_h(out, twin)
     if skip is not None:
         out._rehr_upcat = True
-    if skip is not None and norm_of(skip) is not None:
-        # [up | skip] where the skip half still holds the raw conv output of its block: the buffer is a deferred activation whose
-        # table is the identity on the up-sampled channels (written by the skip's finalize pass)
-        out._rehr_norm = skip._rehr_norm_cat
     return out
 
 
@@ -1410,7 +1217,6 @@ def conv_transpose(x, weight, bias, kernel, stride, padding=(0, 0, 0), act=ACT_N
 class SegHead(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias):
-        x = plain_h(x)
         x_h = is_h(x)
         x = as_cl(x)
         n, d, h, w, cin = x.shape
@@ -1453,7 +1259,6 @@ def seg_head(x, weight, bias):
 class UpsampleD(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, out_d):
-        x = plain_h(x)
         x_h = is_h(x)
         x = as_cl(x)
         n, d, h, w, c = x.shape
@@ -1504,7 +1309,6 @@ class FromChannelsLast(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x):
-        x = plain_h(x)
         x_h = is_h(x)
         x = as_cl(x)
         n, d, h, w, c = x.shape

@@ -120,7 +120,6 @@ def run_transpconv(tc: nn.ConvTranspose3d, x: torch.Tensor, skip: torch.Tensor =
         return F_.conv_transpose(x, tc.weight, tc.bias, k, s, p, skip=skip)
     # no concat room (a caller-built skip): plain copy; fp16 payloads concatenate bit-wise, their bf16 twins likewise
     up = F_.conv_transpose(x, tc.weight, tc.bias, k, s, p)
-    skip = F_.plain_h(skip)
     if F_.is_h(up) != F_.is_h(skip):
         raise RehrError("run_transpconv: up-sampled tensor and skip use different 16-bit storage formats")
     cat = torch.cat((up, skip), dim=4)

@@ -404,148 +404,38 @@ def test_wgrad_march_stride2(case):
     assert rel_l2(dw, ref) < 1e-3, (case, rel_l2(dw, ref))
 
 
-# ------------------------------------------------------------------------------------------------------------------
-# normalise-on-load: the marching kernels apply lrelu(x*scale + shift) to the landed tile instead of reading a materialised
-# activation.  Both paths round the same fp32 value to the same 16-bit format, so they must agree to the last bit of the
-# operand; the only difference left is the (identical) MMA accumulation -> results are compared at 1e-6.
-# ------------------------------------------------------------------------------------------------------------------
-def _raw_and_norm(n, dhw, c, seed, identity_lo=0):
-    g = torch.Generator().manual_seed(seed)
-    y = (2.0 * torch.randn((n, *dhw, c), generator=g) + 0.3).cuda().to(torch.float16)
-    norm = torch.empty((n, 3, c))
-    norm[:, 0] = 0.5 + torch.rand((n, c), generator=g)
-    norm[:, 1] = 0.3 * torch.randn((n, c), generator=g)
-    norm[:, 2] = 0.01
-    if identity_lo:
-        norm[:, 0, :identity_lo], norm[:, 1, :identity_lo], norm[:, 2, :identity_lo] = 1.0, 0.0, 1.0
-    return y.view(torch.bfloat16), norm.cuda().contiguous()
-
-
-NORM_CASES = [
-    # n, cin, cout, (d,h,w), kernel, padding, identity_lo
-    (2, 32, 32, (6, 16, 8), (3, 3, 3), (1, 1, 1), 0),
-    (1, 64, 32, (5, 20, 12), (3, 3, 3), (1, 1, 1), 32),      # [up | skip] concat table, ragged tiles
-    (2, 64, 64, (12, 32, 16), (3, 3, 3), (1, 1, 1), 0),      # Cout tiled 2 x 32
-    (1, 128, 64, (6, 16, 16), (3, 3, 3), (1, 1, 1), 64),     # 2 channel chunks, tile 16
-    (1, 32, 32, (4, 16, 16), (1, 3, 3), (0, 1, 1), 0),       # planar
-    (1, 32, 16, (9, 7, 5), (3, 3, 3), (1, 1, 1), 0),         # everything ragged
+FP16_CASES = [
+    # n, cin, cout, (d,h,w), kernel, padding: marching-kernel shapes
+    (2, 32, 32, (6, 16, 8), (3, 3, 3), (1, 1, 1)),
+    (1, 64, 32, (5, 20, 12), (3, 3, 3), (1, 1, 1)),      # ragged tiles
+    (2, 64, 64, (12, 32, 16), (3, 3, 3), (1, 1, 1)),     # Cout tiled 2 x 32
+    (1, 128, 64, (6, 16, 16), (3, 3, 3), (1, 1, 1)),     # 2 channel chunks, tile 16
+    (1, 32, 32, (4, 16, 16), (1, 3, 3), (0, 1, 1)),      # planar
+    (1, 32, 16, (9, 7, 5), (3, 3, 3), (1, 1, 1)),        # everything ragged
 ]
 
 
-@pytest.mark.parametrize("case", NORM_CASES)
-def test_march_forward_normalise_on_load(case):
+@pytest.mark.parametrize("case", FP16_CASES)
+def test_march_forward_fp16(case):
+    """The forward activations of the InstanceNorm'ed SegModel path are fp16 (functional.FWD_FP16): the marching forward on fp16
+    operands and fp16 output against F.conv3d on the same fp16-rounded operands, and the bf16 twin such an activation hands a
+    weight gradient (converted on demand, cached on the tensor) against the bf16 rounding of its values."""
     from rehrseg_b200 import functional as Fn
-    n, cin, cout, dhw, k, p, ident = case
-    y, norm = _raw_and_norm(n, dhw, cin, 31, ident)
-    Fn.mark_h(y)
-    y._rehr_norm = norm
-    a = Fn.plain_h(y)                                          # materialised fp16 activation (rehr_norm_apply)
-    yf = y.view(torch.float16).float()
-    z = yf * norm[:, 0].view(n, 1, 1, 1, cin) + norm[:, 1].view(n, 1, 1, 1, cin)
-    want_a = torch.where(z > 0, z, z * norm[:, 2].view(n, 1, 1, 1, cin))
-    assert rel_l2(a.view(torch.float16).float(), want_a) < 1e-3
-    w = (torch.randn((cout, cin, *k), generator=torch.Generator().manual_seed(32)) / (cin * k[0] * 9) ** 0.5).cuda()
-    assert Fn.norm_onload_fwd_ok(k, (1, 1, 1), p, cin, cout)
-    out1, st1, _ = Fn.conv3d_raw(y, w, None, k, (1, 1, 1), p, want_stats=True, x_h=True, y_h=True, norm=norm, op_h=True)
-    out2, st2, _ = Fn.conv3d_raw(a, w, None, k, (1, 1, 1), p, want_stats=True, x_h=True, y_h=True)
+    from rehrseg_b200._lib import conv_desc
+    n, cin, cout, dhw, k, p = case
+    assert Fn._march_route(conv_desc(k, (1, 1, 1), p), cin, cout)
+    g = torch.Generator().manual_seed(31)
+    x = torch.randn((n, *dhw, cin), generator=g).cuda().to(torch.float16)
+    w = (torch.randn((cout, cin, *k), generator=g) / (cin * k[0] * k[1] * k[2]) ** 0.5).cuda()
+    xh = Fn.mark_h(x.view(torch.bfloat16))
+    y, stats, _ = Fn.conv3d_raw(xh, w, None, k, (1, 1, 1), p, want_stats=True, x_h=True, y_h=True)
+    tw = Fn.bf_twin(xh)
     torch.cuda.synchronize()
-    assert rel_l2(out1.view(torch.float16).float(), out2.view(torch.float16).float()) < 1e-6
-    assert rel_l2(st1, st2) < 1e-6
-    ref = F.conv3d(want_a.permute(0, 4, 1, 2, 3), w.to(torch.float16).float(), None, padding=p)
-    assert rel_l2(out1.view(torch.float16).float().permute(0, 4, 1, 2, 3), ref) < 2e-3
-
-
-WG_NORM_CASES = [
-    (2, 32, 32, (16, 32, 32), (3, 3, 3), (1, 1, 1), 0),       # role / piece choice: CH 32
-    (1, 64, 32, (24, 44, 36), (3, 3, 3), (1, 1, 1), 32),      # [up | skip] table, ragged tiles, CH 64
-    (2, 64, 64, (16, 32, 32), (3, 3, 3), (1, 1, 1), 0),
-    (2, 128, 64, (16, 32, 32), (3, 3, 3), (1, 1, 1), 64),
-    (2, 32, 32, (10, 48, 40), (1, 3, 3), (0, 1, 1), 0),       # planar
-    (2, 32, 16, (17, 23, 29), (3, 3, 3), (1, 1, 1), 0),       # everything ragged
-]
-
-
-@pytest.mark.parametrize("case", WG_NORM_CASES)
-def test_march_wgrad_normalise_on_load(case):
-    from rehrseg_b200 import functional as Fn
-    n, cin, cout, dhw, k, p, ident = case
-    assert Fn.wgrad_route((n, *dhw, cin), (n, *dhw, cout), k, (1, 1, 1), p) == "march"
-    y, norm = _raw_and_norm(n, dhw, cin, 33, ident)
-    Fn.mark_h(y)
-    y._rehr_norm = norm
-    abf = Fn.bf_twin(y)                                        # materialised bf16 activation
-    dy = torch.randn((n, *dhw, cout), generator=torch.Generator().manual_seed(34)).cuda().to(torch.bfloat16)
-    wshape = (cout, cin, *k)
-    dw1 = Fn.conv3d_wgrad_raw(y, dy, wshape, k, (1, 1, 1), p, norm=norm, x_h=True)
-    dw2 = Fn.conv3d_wgrad_raw(abf, dy, wshape, k, (1, 1, 1), p)
-    torch.cuda.synchronize()
-    assert rel_l2(dw1, dw2) < 1e-6
-    xr = abf.float().permute(0, 4, 1, 2, 3).requires_grad_(False)
-    wz = torch.zeros(wshape, device="cuda", requires_grad=True)
-    ref, = torch.autograd.grad(F.conv3d(xr, wz, None, padding=p), wz, dy.float().permute(0, 4, 1, 2, 3))
-    assert rel_l2(dw1, ref) < 2e-3
-
-
-@pytest.mark.parametrize("dhw", [(32, 64, 64), (31, 66, 61)])
-def test_march_s2_wgrad_normalise_on_load(dhw):
-    """Stride-2 stage entry: the parity-class views of the RAW producer output are normalised on load."""
-    from rehrseg_b200 import functional as Fn
-    n, cin, cout = 2, 32, 64
-    k, s, p = (3, 3, 3), (2, 2, 2), (1, 1, 1)
-    y, norm = _raw_and_norm(n, dhw, cin, 35)
-    Fn.mark_h(y)
-    y._rehr_norm = norm
-    abf = Fn.bf_twin(y)
-    odhw = tuple((v + 2 - 3) // 2 + 1 for v in dhw)
-    dy = torch.randn((n, *odhw, cout), generator=torch.Generator().manual_seed(36)).cuda().to(torch.bfloat16)
-    old = Fn.S2_WGRAD_MARCH_MIN_VOXELS
-    Fn.S2_WGRAD_MARCH_MIN_VOXELS = 0
-    try:
-        assert Fn.wgrad_route((n, *dhw, cin), (n, *odhw, cout), k, s, p) == "march_s2"
-        dw1 = Fn.conv3d_wgrad_raw(y, dy, (cout, cin, *k), k, s, p, norm=norm, x_h=True)
-        dw2 = Fn.conv3d_wgrad_raw(abf, dy, (cout, cin, *k), k, s, p)
-    finally:
-        Fn.S2_WGRAD_MARCH_MIN_VOXELS = old
-    torch.cuda.synchronize()
-    assert rel_l2(dw1, dw2) < 1e-6
-
-
-@pytest.mark.parametrize("case", [(2, 32, 32, (16, 32, 32)), (1, 64, 64, (16, 16, 24)), (2, 64, 128, (8, 16, 16)), (1, 32, 64, (9, 17, 23))])
-def test_in_bwd_sums_from_dgrad_epilogue(case, monkeypatch):
-    """Two stacked Conv -> InstanceNorm -> LeakyReLU blocks: the second block's marching input-gradient epilogue also produces the
-    FIRST block's InstanceNorm backward sums (rehr_conv3d_march_dgrad_inred + ..._bwd_finalize_raw), so its reduce pass is skipped.
-    Every gradient must match the unfused path (same kernels otherwise) to fp32 summation-order accuracy."""
-    from rehrseg_b200 import functional as Fn
-    n, c1, c2, dhw = case
-    g = torch.Generator().manual_seed(11)
-    x = torch.randn((n, *dhw, 32), generator=g).cuda().to(torch.bfloat16)
-    w1 = (torch.randn((c1, 32, 3, 3, 3), generator=g) / (27 * 32) ** 0.5).cuda()
-    w2 = (torch.randn((c2, c1, 3, 3, 3), generator=g) / (27 * c1) ** 0.5).cuda()
-    ga1, be1 = (1 + 0.2 * torch.randn((c1,), generator=g)).cuda(), (0.3 * torch.randn((c1,), generator=g)).cuda()
-    ga2, be2 = (1 + 0.2 * torch.randn((c2,), generator=g)).cuda(), (0.3 * torch.randn((c2,), generator=g)).cuda()
-    go = torch.randn((n, *dhw, c2), generator=g).cuda().to(torch.bfloat16)
-
-    def run(fused):
-        monkeypatch.setattr(Fn, "INRED", fused)
-        leaves = [t.clone().requires_grad_(True) for t in (x, w1, ga1, be1, w2, ga2, be2)]
-        xx, a1w, a1g, a1b, a2w, a2g, a2b = leaves
-        h = Fn.conv_norm_act(xx, a1w, None, a1g, a1b, (3, 3, 3), (1, 1, 1), (1, 1, 1))
-        out = Fn.conv_norm_act(h, a2w, None, a2g, a2b, (3, 3, 3), (1, 1, 1), (1, 1, 1))
-        grads = torch.autograd.grad(out, leaves, go)
-        torch.cuda.synchronize()
-        return [t.float() for t in grads]
-
-    hits = Fn.path_hits["in_bwd_sums_from_dgrad_epilogue"]
-    fused = run(True)
-    assert Fn.path_hits["in_bwd_sums_from_dgrad_epilogue"] == hits + 1
-    plain = run(False)
-    assert Fn.path_hits["in_bwd_sums_from_dgrad_epilogue"] == hits + 1
-    names = ["dx", "dw1", "dgamma1", "dbeta1", "dw2", "dgamma2", "dbeta2"]
-    for name, a, b in zip(names, fused, plain):
-        # block 2's own gradients do not depend on the fusion at all; block 1's differ by the bf16 rounding of dA the stand-alone
-        # reduce pass sees (the epilogue sums the fp32 accumulators) and by summation order
-        tol = 0.0 if name in ("dw2", "dgamma2", "dbeta2") else 4e-3
-        assert rel_l2(a, b) <= tol, (name, rel_l2(a, b))
+    ref = F.conv3d(x.float().permute(0, 4, 1, 2, 3), w.to(torch.float16).float(), None, padding=p)
+    got = y.view(torch.float16).float().permute(0, 4, 1, 2, 3)
+    assert rel_l2(got, ref) < 2e-3, (case, rel_l2(got, ref))
+    assert rel_l2(stats.sum(1)[..., 0], ref.sum((2, 3, 4))) < 2e-3     # InstanceNorm partial sums of the epilogue
+    assert torch.equal(tw, x.float().to(torch.bfloat16)) and Fn.bf_twin(xh) is tw
 
 
 @pytest.mark.parametrize("shape,out_d", [((2, 16, 24, 20, 32), 64), ((1, 5, 9, 7, 16), 18), ((1, 1, 8, 8, 8), 4), ((2, 7, 6, 6, 8), 7),

@@ -22,7 +22,7 @@ def test_library_exports_every_declared_symbol():
     assert not missing, missing
     undeclared = [n for n in lib._rehr_signatures if n not in names]
     assert not undeclared, undeclared
-    assert lib.rehr_version() == 5
+    assert lib.rehr_version() == 6
     assert lib.rehr_strerror(-2).decode().startswith("configuration not supported")
 
 
