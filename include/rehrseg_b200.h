@@ -66,7 +66,8 @@ const char* rehr_strerror(int status);
 int rehr_last_cuda_error(void);     /* cudaError_t of the last failing CUDA call on this thread */
 int rehr_version(void);             /* ABI version, currently 6 (4: rehr_tensor.dtype, dtype arguments of the weight packers; 5: batched
                                      * re-pack and fused InstanceNorm-backward sums added -- additive; 6: the normalise-on-load and fused
-                                     * InstanceNorm-backward-sum entry points removed) */
+                                     * InstanceNorm-backward-sum entry points removed; the rehr_intensity_* entry points were added
+                                     * later without a bump -- additive) */
 int rehr_device_sm_count(void);
 
 /* ------------------------------------------------------------------------------------------------
@@ -326,6 +327,46 @@ int rehr_resample_axis(const float* x, float* y, long long outer, int n_in, int 
 int rehr_bspline_prefilter_axis(float* c, long long outer, int n, long long inner, rehr_stream stream);
 int rehr_affine_sample2d(const float* src, float* dst, const float* affine, int slices, int x, int y, int px, int py, int slices_per_sample,
                          int order, float cval, const float* labels_host, int n_labels, rehr_stream stream);
+
+/* Stage-2 intensity augmentation (rehrseg_b200/intensity.py): the noise / blur / brightness / contrast / low-resolution / gamma
+ * transforms get_training_transforms appends after the spatial part (utils/seg_utils.py:677-689), batchgenerators 0.25 semantics
+ * (restated, parity unpinned).  Every entry point works on ROWS: a row is one (sample, channel) volume [z][x][y] of the f32 data
+ * tensor the transform fired on, described by one rehr_irow of a DEVICE table; rows not listed are never read.  One launch covers
+ * all rows.  Moment tables are f64 [rows][rehr_intensity_moment_doubles()]: per-chunk partials of a row, reduced in a fixed order
+ * (the chunking depends on the row's length only, so results do not depend on which other rows share the launch).
+ *   rehr_intensity_moments     partials of (sum, sum of squares, min, max) of row.len elements at base + row.off (from_aux = 0)
+ *                              or base + row.aux (from_aux = 1).
+ *   rehr_intensity_pointwise   op 0: x += noise[aux + i] (the sum in f64, stored f32); op 1: x *= p[0]; op 2: contrast
+ *                              (x - mean) * p[0] + mean from `moments` of the same rows, clipped to their [min, max] when n[0].
+ *   rehr_intensity_blur_axis   scipy.ndimage.gaussian_filter1d along `axis` (0 = z, 1 = x, 2 = y) of the [z][x][y] rows, sigma p[axis],
+ *                              radius n[axis] (<= 63), mode 'reflect' for any length; src / dst at row.off or, when *_aux, row.aux.
+ *   rehr_intensity_gamma       augment_gamma on s * x (s = p[1] = +-1, gamma p[0], retain_stats n[0]) with the `moments` of x:
+ *                              apply = 0 writes the moments of the powered values to `powered`; apply = 1 writes the result.
+ *   rehr_intensity_lowres_*    resize(x, (z, n[0], n[1]), order 0) then resize(., (z, x, y), order 3), scikit-image 'edge' semantics:
+ *                              gather writes the order-0 image edge-padded by 12 samples, [z][n[0] + 24][n[1] + 24] at pad + row.aux
+ *                              (row.len elements); prefilter runs the mirror B-spline prefilter along axis 1 or 2 of it; upsample
+ *                              evaluates the cubic spline, clipped to the [min, max] of `moments` (of the padded rows). */
+typedef struct {
+  long long off;  /* first element of the row in the data tensor */
+  long long aux;  /* first element of the row's scratch (noise field, blur temporary, padded low-resolution image) */
+  long long len;  /* elements of the row, or of its scratch (low resolution) */
+  int n[4];       /* integer parameters */
+  double p[4];    /* real parameters */
+} rehr_irow;
+int rehr_intensity_moment_doubles(void);
+int rehr_intensity_moments(const float* base, const rehr_irow* rows, int nrows, int from_aux, long long max_len, double* moments,
+                           rehr_stream stream);
+int rehr_intensity_pointwise(float* x, const rehr_irow* rows, int nrows, long long len, int op, const float* noise, const double* moments,
+                             rehr_stream stream);
+int rehr_intensity_blur_axis(const float* src, int src_aux, float* dst, int dst_aux, const rehr_irow* rows, int nrows, int z, int x, int y,
+                             int axis, rehr_stream stream);
+int rehr_intensity_gamma(float* x, const rehr_irow* rows, int nrows, long long len, const double* moments, double* powered, int apply,
+                         rehr_stream stream);
+int rehr_intensity_lowres_gather(const float* x, float* pad, const rehr_irow* rows, int nrows, int z, int xs, int ys, long long max_len,
+                                 rehr_stream stream);
+int rehr_intensity_lowres_prefilter(float* pad, const rehr_irow* rows, int nrows, int z, int axis, long long max_lines, rehr_stream stream);
+int rehr_intensity_lowres_upsample(float* x, const float* pad, const rehr_irow* rows, int nrows, int z, int xs, int ys,
+                                   const double* moments, rehr_stream stream);
 
 /* rotate_vol_2d (utils/rotate.py:5-31): rot90 by k quarter turns over dims (0,1) of vol[X][Y][inner]. */
 int rehr_rot90(const void* src, void* dst, int X, int Y, long long inner_bytes, int k, rehr_stream stream);

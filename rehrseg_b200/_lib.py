@@ -136,6 +136,14 @@ def _declare(L: C.CDLL) -> None:
         "rehr_resample_axis": (i, [vp, vp, ll, i, i, ll, f, i, vp]),
         "rehr_bspline_prefilter_axis": (i, [vp, ll, i, ll, vp]),
         "rehr_affine_sample2d": (i, [vp, vp, vp, i, i, i, i, i, i, i, f, vp, i, vp]),
+        "rehr_intensity_moment_doubles": (i, []),
+        "rehr_intensity_moments": (i, [vp, vp, i, i, ll, vp, vp]),
+        "rehr_intensity_pointwise": (i, [vp, vp, i, ll, i, vp, vp, vp]),
+        "rehr_intensity_blur_axis": (i, [vp, i, vp, i, vp, i, i, i, i, i, vp]),
+        "rehr_intensity_gamma": (i, [vp, vp, i, ll, vp, vp, i, vp]),
+        "rehr_intensity_lowres_gather": (i, [vp, vp, vp, i, i, i, i, ll, vp]),
+        "rehr_intensity_lowres_prefilter": (i, [vp, vp, i, i, i, ll, vp]),
+        "rehr_intensity_lowres_upsample": (i, [vp, vp, vp, i, i, i, i, vp, vp]),
         "rehr_rot90": (i, [vp, vp, i, i, ll, i, vp]),
         "rehr_fba_combine": (i, [vp, i, f, vp, ll, vp]),
         "rehr_mean_stack": (i, [vp, i, vp, ll, vp]),

@@ -7,6 +7,8 @@ and the uncertainty map, order-1 per-label interpolation for the two segmentatio
 deformation, rotation about x and isotropic scaling with p = 0.2 each, no random crop) the coordinate field of a sample is AFFINE,
 so the whole transform is two kernels: scipy's cubic B-spline prefilter along both image axes (`rehr_bspline_prefilter_axis`) and
 one gather per output pixel (`rehr_affine_sample2d`).  The random decisions are drawn from `np.random` in the reference's order.
+The intensity transforms that follow the spatial part (utils/seg_utils.py:677-689) are rehrseg_b200/intensity.py; `Stage2Sampler`
+runs them when given an `IntensityAugment`.
 
 Parity: tests/test_augment_gpu.py against tests/golden/spatial_aug.npz (the reference's OWN `augment_spatial` with scipy's real
 map_coordinates) and against oracle/augment.py on other shapes."""
@@ -21,6 +23,7 @@ import torch
 
 from . import functional as F_
 from ._lib import RehrError, check, lib, ptr, stream_ptr
+from .intensity import IntensityAugment, IntensityPlan
 
 
 def draw_affine_2d(rng=np.random, do_rotation=True, angle_x=(-math.pi, math.pi), do_scale=True, scale=(0.7, 1.4),
@@ -125,15 +128,18 @@ class Stage2Sampler:
     """`TrainSetMultipleSegSREfficient` (utils/train_set.py:21-159) with the subjects resident on the GPU: `sample(i)` is
     `__getitem__` -- z-score of the volume, random crop (Python `random`, the reference's order), constant padding, flips, slice
     decimation, the [1, 1, z, y, x] layout, the uncertainty rescaling -- followed by the SPATIAL part of `self.train_transform`
-    (`spatial_transform_dummy_2d`, `np.random`).  The intensity transforms `get_training_transforms` appends after it are
-    third-party batchgenerators classes and are not part of this port; `batch` stacks samples like the DataLoader's collate."""
+    (`spatial_transform_dummy_2d`, `np.random`) and, when `intensity` is given, by the intensity transforms `get_training_transforms`
+    appends after it (`rehrseg_b200.intensity.IntensityAugment`, drawn right after the sample's spatial decisions); `batch` stacks
+    samples like the DataLoader's collate and runs the intensity transforms of all its samples in one pass."""
 
     def __init__(self, patch_size: Sequence[int], separation: int, norm: bool = True, random_flip: bool = True,
-                 uncertainty: bool = True, device=None, p_rot_per_sample: float = 0.2, p_scale_per_sample: float = 0.2):
+                 uncertainty: bool = True, device=None, p_rot_per_sample: float = 0.2, p_scale_per_sample: float = 0.2,
+                 intensity: Optional["IntensityAugment"] = None):
         self.patch_size = list(patch_size)            # (x, y, z_lr) as in the reference's patch_size_ori
         self.separation = int(separation)
         self.norm, self.random_flip, self.uncertainty = bool(norm), bool(random_flip), bool(uncertainty)
         self.p_rot, self.p_scale = float(p_rot_per_sample), float(p_scale_per_sample)
+        self.intensity = intensity
         self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         self.imgs: List[torch.Tensor] = []
         self.labels: List[torch.Tensor] = []
@@ -162,6 +168,13 @@ class Stage2Sampler:
         return torch.nn.functional.pad(t, flat) if any(flat) else t
 
     def sample(self, i: int, rng_py=None, rng_np=np.random, seg_labels: Optional[Sequence[float]] = None):
+        out, plan = self._sample(i, rng_py, rng_np, seg_labels)
+        if plan is not None:
+            self.intensity.apply(out[0][None], plan)
+        return out
+
+    def _sample(self, i: int, rng_py, rng_np, seg_labels):
+        """One sample before its intensity transforms: (outputs of `sample`, the drawn IntensityPlan or None)."""
         import random as _random
         rng = rng_py or _random
         img, label = self.imgs[i], self.labels[i]
@@ -194,9 +207,15 @@ class Stage2Sampler:
         out = spatial_transform_dummy_2d({k: v.contiguous() for k, v in dd.items()}, patch_zyx, keys=tuple(keys),
                                          enable_uncertainty=self.uncertainty, rng=rng_np, seg_labels=seg_labels,
                                          p_rot_per_sample=self.p_rot, p_scale_per_sample=self.p_scale)
+        plan = None
+        if self.intensity is not None:
+            plan = self.intensity.draw(1, 1, out["data"].shape[2:], rng, rng_np)
         unc_out = out["uncertainty"].squeeze(0) if self.uncertainty else 0
-        return out["data"].squeeze(0), out["seg"].squeeze(0), out["seg_sr"].squeeze(0), unc_out
+        return (out["data"].squeeze(0), out["seg"].squeeze(0), out["seg_sr"].squeeze(0), unc_out), plan
 
     def batch(self, indices: Sequence[int], rng_py=None, rng_np=np.random, seg_labels: Optional[Sequence[float]] = None):
-        rows = [self.sample(i, rng_py, rng_np, seg_labels) for i in indices]
-        return tuple(torch.stack([r[k] for r in rows]) for k in range(4 if self.uncertainty else 3))
+        drawn = [self._sample(i, rng_py, rng_np, seg_labels) for i in indices]
+        out = tuple(torch.stack([r[k] for r, _ in drawn]) for k in range(4 if self.uncertainty else 3))
+        if self.intensity is not None:
+            self.intensity.apply(out[0], IntensityPlan.concat([p for _, p in drawn]))
+        return out
