@@ -338,6 +338,11 @@ int rehr_affine_sample2d(const float* src, float* dst, const float* affine, int 
  *                              or base + row.aux (from_aux = 1).
  *   rehr_intensity_pointwise   op 0: x += noise[aux + i] (the sum in f64, stored f32); op 1: x *= p[0]; op 2: contrast
  *                              (x - mean) * p[0] + mean from `moments` of the same rows, clipped to their [min, max] when n[0].
+ *   rehr_intensity_noise_philox  x += (float)(p[0] * z_i) (the sum in f64, stored f32) with z generated in the kernel: row r's key is
+ *                              keys[2r], keys[2r + 1] (a DEVICE array); element i takes word i % 4 of Philox4x64-10 block i / 4 at
+ *                              counter (i / 4 + 1, 0, 0, 0) -- np.random.Philox(key=key).random_raw -- and z is Box-Muller in f64 over
+ *                              the word pairs (2j, 2j + 1): u1 = ((w >> 11) + 1) 2^-53, u2 = (w' >> 11) 2^-53, r = sqrt(-2 ln u1),
+ *                              z_2j = r cos(2 pi u2), z_2j+1 = r sin(2 pi u2).
  *   rehr_intensity_blur_axis   scipy.ndimage.gaussian_filter1d along `axis` (0 = z, 1 = x, 2 = y) of the [z][x][y] rows, sigma p[axis],
  *                              radius n[axis] (<= 63), mode 'reflect' for any length; src / dst at row.off or, when *_aux, row.aux.
  *   rehr_intensity_gamma       augment_gamma on s * x (s = p[1] = +-1, gamma p[0], retain_stats n[0]) with the `moments` of x:
@@ -358,6 +363,8 @@ int rehr_intensity_moments(const float* base, const rehr_irow* rows, int nrows, 
                            rehr_stream stream);
 int rehr_intensity_pointwise(float* x, const rehr_irow* rows, int nrows, long long len, int op, const float* noise, const double* moments,
                              rehr_stream stream);
+int rehr_intensity_noise_philox(float* x, const rehr_irow* rows, const unsigned long long* keys, int nrows, long long len,
+                                rehr_stream stream);
 int rehr_intensity_blur_axis(const float* src, int src_aux, float* dst, int dst_aux, const rehr_irow* rows, int nrows, int z, int x, int y,
                              int axis, rehr_stream stream);
 int rehr_intensity_gamma(float* x, const rehr_irow* rows, int nrows, long long len, const double* moments, double* powered, int apply,

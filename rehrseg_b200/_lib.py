@@ -139,6 +139,7 @@ def _declare(L: C.CDLL) -> None:
         "rehr_intensity_moment_doubles": (i, []),
         "rehr_intensity_moments": (i, [vp, vp, i, i, ll, vp, vp]),
         "rehr_intensity_pointwise": (i, [vp, vp, i, ll, i, vp, vp, vp]),
+        "rehr_intensity_noise_philox": (i, [vp, vp, vp, i, ll, vp]),
         "rehr_intensity_blur_axis": (i, [vp, i, vp, i, vp, i, i, i, i, i, vp]),
         "rehr_intensity_gamma": (i, [vp, vp, i, ll, vp, vp, i, vp]),
         "rehr_intensity_lowres_gather": (i, [vp, vp, vp, i, i, i, i, ll, vp]),

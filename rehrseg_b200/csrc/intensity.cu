@@ -166,6 +166,60 @@ __global__ void __launch_bounds__(kIThreads) intensity_pointwise_kernel(float* _
   }
 }
 
+// ---- Gaussian noise from a counter-based generator -----------------------------------------------------------------------------------
+// Philox4x64-10 (Random123 constants).  Block g of a row with key (k0, k1) is philox(counter = (g + 1, 0, 0, 0), key): the word stream
+// of np.random.Philox(key=key).random_raw, whose first block is counter 1.
+__device__ __forceinline__ void philox4x64_10(unsigned long long c[4], unsigned long long k0, unsigned long long k1) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) {
+      k0 += 0x9E3779B97F4A7C15ull;
+      k1 += 0xBB67AE8584CAA73Bull;
+    }
+    const unsigned long long h0 = __umul64hi(0xD2E7470EE14C6C93ull, c[0]), l0 = 0xD2E7470EE14C6C93ull * c[0];
+    const unsigned long long h1 = __umul64hi(0xCA5A826395121157ull, c[2]), l1 = 0xCA5A826395121157ull * c[2];
+    c[0] = h1 ^ c[1] ^ k0;
+    c[1] = l1;
+    c[2] = h0 ^ c[3] ^ k1;
+    c[3] = l0;
+  }
+}
+
+// Box-Muller of the word pair (a, b) in f64: u1 = ((a >> 11) + 1) 2^-53 in (0, 1], u2 = (b >> 11) 2^-53, r = sqrt(-2 ln u1);
+// the pair's normals are r cos(2 pi u2), r sin(2 pi u2).  sincospi(2 u2) takes the angle without rounding 2 pi u2 (numpy's
+// cos(2.0 * np.pi * u2) differs by at most 5e-16 absolute) and has no large-argument reduction, whose scratch array would live in
+// local memory.
+__device__ __forceinline__ void box_muller(unsigned long long a, unsigned long long b, double& zc, double& zs) {
+  const double u1 = __dmul_rn((double)((a >> 11) + 1), 0x1p-53), u2 = __dmul_rn((double)(b >> 11), 0x1p-53);
+  const double r = sqrt(__dmul_rn(-2.0, log(u1)));
+  double s, c;
+  sincospi(2.0 * u2, &s, &c);
+  zc = __dmul_rn(r, c);
+  zs = __dmul_rn(r, s);
+}
+
+// x += (float)(p[0] * z) per element, the sum in f64 and stored f32 (the arithmetic of the host-field path).  Each thread makes whole
+// Philox blocks, i.e. 4 elements; a chunk's length is a multiple of 1024, so no block straddles two chunks.
+__global__ void __launch_bounds__(kIThreads) intensity_noise_philox_kernel(float* __restrict__ x, const rehr_irow* __restrict__ rows,
+                                                                           const unsigned long long* __restrict__ keys, long long len) {
+  const int r = blockIdx.y;
+  const double vh = rows[r].p[0];
+  const unsigned long long k0 = keys[2 * r], k1 = keys[2 * r + 1];
+  float* p = x + rows[r].off;
+  const long long cl = ichunk_len(len), e0 = (long long)blockIdx.x * cl, e1 = min(len, e0 + cl);
+  for (long long g = e0 / 4 + threadIdx.x; 4 * g < e1; g += kIThreads) {
+    unsigned long long w[4] = {(unsigned long long)g + 1, 0ull, 0ull, 0ull};
+    philox4x64_10(w, k0, k1);
+    double z[4];
+    box_muller(w[0], w[1], z[0], z[1]);
+    box_muller(w[2], w[3], z[2], z[3]);
+    const long long e = 4 * g;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if (e + i < e1) p[e + i] = (float)((double)p[e + i] + (double)(float)__dmul_rn(vh, z[i]));
+  }
+}
+
 // ---- Gaussian blur, one axis -------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int reflect_idx(int i, int n) {  // scipy 'reflect' (d c b a | a b c d | d c b a), any length
   const int period = 2 * n;
@@ -357,6 +411,14 @@ int rehr_intensity_pointwise(float* x, const rehr_irow* rows, int nrows, long lo
   if (!x || !rows_ok(rows, nrows) || len <= 0) return REHR_BAD_SHAPE;
   if (op < 0 || op > 2 || (op == 0 && !noise) || (op == 2 && !moments)) return REHR_BAD_SHAPE;
   intensity_pointwise_kernel<<<dim3(ichunks(len), nrows), kIThreads, 0, (cudaStream_t)stream>>>(x, rows, len, op, noise, moments);
+  REHR_CHECK_LAUNCH();
+  return REHR_OK;
+}
+
+int rehr_intensity_noise_philox(float* x, const rehr_irow* rows, const unsigned long long* keys, int nrows, long long len,
+                                rehr_stream stream) {
+  if (!x || !keys || !rows_ok(rows, nrows) || len <= 0) return REHR_BAD_SHAPE;
+  intensity_noise_philox_kernel<<<dim3(ichunks(len), nrows), kIThreads, 0, (cudaStream_t)stream>>>(x, rows, keys, len);
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }

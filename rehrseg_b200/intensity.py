@@ -8,9 +8,14 @@ and the default parameters are nnU-Net v2's `get_training_transforms` values for
 keyword argument, so checking them against the reference's lines means changing defaults, not kernels.
 
 None of the random decisions depends on the data, so `draw` makes all of them on the host in the reference's order (`rng_np` for
-np.random, `rng_py` for Python's random), including the noise field, which only `rng_np.normal` can produce without disturbing every
-later draw; it goes to pinned memory and reaches the GPU with an asynchronous copy.  `apply` then runs every transform that fired
-anywhere in the batch with a fixed number of launches over the (sample, channel) rows it fired on (csrc/intensity.cu)."""
+np.random, `rng_py` for Python's random).  By default (`noise_rng="numpy"`) that includes the noise field, which only
+`rng_np.normal` can produce without disturbing every later draw; it goes to pinned memory and reaches the GPU with an asynchronous
+copy.  With `noise_rng="philox"` the noise row instead draws a 128-bit key, `rng_np.randint(0, 2**64, size=2, dtype=np.uint64)`, at
+the place of that `normal` call, and the kernel generates the field from it (Philox4x64-10 and Box-Muller, restated in
+oracle/intensity_philox.py): no host draw and no upload of the field.  Both streams stay deterministic, but np.random diverges
+from the reference's after the first noised row, so every later draw (and every later batch) differs from batchgenerators'.
+`apply` then runs every transform that fired anywhere in the batch with a fixed number of launches over the (sample, channel) rows
+it fired on (csrc/intensity.cu)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -38,6 +43,7 @@ NAMES = tuple(k for k, _ in TRANSFORMS)
 
 _PAD = 12               # scipy's pre-padding of an order-3 spline in mode 'nearest' (csrc/intensity.cu kLowresPad)
 _MAX_BLUR_RADIUS = 63   # csrc/intensity.cu kMaxBlurRadius
+NOISE_RNGS = ("numpy", "philox")
 # mirror of rehr_irow (include/rehrseg_b200.h)
 IROW = np.dtype([("off", "<i8"), ("aux", "<i8"), ("len", "<i8"), ("n", "<i4", (4,)), ("p", "<f8", (4,))], align=True)
 assert IROW.itemsize == 72
@@ -57,12 +63,15 @@ def _split_uniform(rng_np, r):
 
 class IntensityPlan:
     """The host-drawn decisions for a batch [b, c, *shape]: per transform, the rows (sample, channel, parameters...) it fired on,
-    and the noise fields (fp32 host tensors, pinned when CUDA is available) in the order of the noise rows."""
+    and, in the order of the noise rows, the noise fields (`noise_rng="numpy"`: fp32 host tensors, pinned when CUDA is available) or
+    the Philox keys (`noise_rng="philox"`: `noise_keys`, uint64 [rows, 2])."""
 
-    def __init__(self, b: int, c: int, shape: Sequence[int]):
+    def __init__(self, b: int, c: int, shape: Sequence[int], noise_rng: str = "numpy"):
         self.b, self.c, self.shape = int(b), int(c), tuple(int(s) for s in shape)
+        self.noise_rng = noise_rng
         self.rows: Dict[str, List[tuple]] = {k: [] for k in NAMES}
         self.noise: List[torch.Tensor] = []
+        self.noise_keys = np.zeros((0, 2), np.uint64)
 
     def fired(self) -> List[str]:
         return [k for k in NAMES if self.rows[k]]
@@ -72,13 +81,16 @@ class IntensityPlan:
         """The plan of the samples of `plans` stacked along the batch."""
         if not plans or any(p.c != plans[0].c or p.shape != plans[0].shape for p in plans):
             raise RehrError("IntensityPlan.concat: plans of the same channel count and spatial shape")
-        out = IntensityPlan(sum(p.b for p in plans), plans[0].c, plans[0].shape)
+        if any(p.noise_rng != plans[0].noise_rng for p in plans):
+            raise RehrError("IntensityPlan.concat: plans of the same noise_rng")
+        out = IntensityPlan(sum(p.b for p in plans), plans[0].c, plans[0].shape, plans[0].noise_rng)
         b0 = 0
         for p in plans:
             for k in NAMES:
                 out.rows[k] += [(r[0] + b0,) + tuple(r[1:]) for r in p.rows[k]]
             out.noise += p.noise
             b0 += p.b
+        out.noise_keys = np.concatenate([p.noise_keys for p in plans])
         return out
 
 
@@ -88,9 +100,17 @@ class IntensityAugment:
 
     `draw(b, c, spatial_shape, rng_py, rng_np)` makes every random decision on the host, consuming both streams exactly as the
     batchgenerators transforms do; `apply(data, plan)` runs the plan in place on a CUDA fp32 [b, c, z, x, y] tensor; calling the
-    object does both."""
+    object does both.
 
-    def __init__(self, **overrides):
+    `noise_rng` chooses where the Gaussian noise field comes from.  "numpy" (the default): `rng_np.normal` on the host, so np.random
+    follows batchgenerators draw for draw.  "philox": the kernel generates it from a per-row key drawn from `rng_np` in place of
+    that `normal` call -- microseconds instead of a host draw of the whole field per noised row, deterministic under the same seeds,
+    but np.random leaves the reference's sequence at the first noised row (see the module docstring)."""
+
+    def __init__(self, *, noise_rng: str = "numpy", **overrides):
+        if not isinstance(noise_rng, str) or noise_rng not in NOISE_RNGS:
+            raise RehrError(f"IntensityAugment: noise_rng must be one of {NOISE_RNGS}, not {noise_rng!r}")
+        self.noise_rng = noise_rng
         unknown = set(overrides) - set(NAMES)
         if unknown:
             raise TypeError(f"IntensityAugment: unknown transforms {sorted(unknown)}")
@@ -112,10 +132,11 @@ class IntensityAugment:
         shape = tuple(int(s) for s in spatial_shape)
         if len(shape) != 3:
             raise RehrError("IntensityAugment: spatial shape (z, x, y)")
-        plan = IntensityPlan(b, c, shape)
+        plan = IntensityPlan(b, c, shape, self.noise_rng)
         P, R = self.params, plan.rows
         V = int(np.prod(shape))
         pin = torch.cuda.is_available()
+        keys = []
 
         q = P["noise"]
         for bi in range(b):
@@ -124,10 +145,15 @@ class IntensityAugment:
                 for ci in range(c):
                     if rng_np.uniform() < q["p_per_channel"]:
                         vh = v if v is not None else _range_val(rng_py, q["noise_variance"])
-                        field = torch.empty(V, dtype=torch.float32, pin_memory=pin)
-                        field.numpy()[:] = rng_np.normal(0.0, vh, size=shape).reshape(-1)
-                        R["noise"].append((bi, ci))
-                        plan.noise.append(field)
+                        if self.noise_rng == "philox":
+                            keys.append(rng_np.randint(0, 2 ** 64, size=2, dtype=np.uint64))
+                        else:
+                            field = torch.empty(V, dtype=torch.float32, pin_memory=pin)
+                            field.numpy()[:] = rng_np.normal(0.0, vh, size=shape).reshape(-1)
+                            plan.noise.append(field)
+                        R["noise"].append((bi, ci, float(vh)))
+        if keys:
+            plan.noise_keys = np.stack(keys)
 
         q = P["blur"]
 
@@ -210,7 +236,9 @@ class IntensityAugment:
             t["off"] = [(r[0] * plan.c + r[1]) * V for r in rows]
             t["len"] = V
             t["aux"] = np.arange(len(rows), dtype=np.int64) * V
-            if k == "blur":
+            if k == "noise":
+                t["p"][:, 0] = [r[2] for r in rows]
+            elif k == "blur":
                 t["p"][:, :3] = [r[2] for r in rows]
                 t["n"][:, :3] = [[int(4.0 * s + 0.5) for s in r[2]] for r in rows]      # scipy: radius = int(truncate * sigma + 0.5)
             elif k == "brightness":
@@ -229,12 +257,18 @@ class IntensityAugment:
                 t["p"][:, 1] = [r[3] for r in rows]
                 t["n"][:, 0] = [int(r[4]) for r in rows]
             tables[k] = t
-        blob = np.concatenate([tables[k].view(np.uint8) for k in fired])
+        philox = "noise" in fired and plan.noise_rng == "philox"
+        if philox and plan.noise_keys.shape != (len(plan.rows["noise"]), 2):
+            raise RehrError(f"IntensityAugment.apply: {len(plan.rows['noise'])} noise rows but keys {plan.noise_keys.shape}")
+        # the Philox keys of the noise rows follow the tables (offset a multiple of 8: rehr_irow is 72 bytes)
+        keys = [np.ascontiguousarray(plan.noise_keys, dtype=np.uint64).view(np.uint8).reshape(-1)] if philox else []
+        blob = np.concatenate([tables[k].view(np.uint8) for k in fired] + keys)
         dev_blob = torch.from_numpy(blob).pin_memory().to(dev, non_blocking=True)
         addr, o = {}, 0
         for k in fired:
             addr[k] = C.c_void_p(dev_blob.data_ptr() + o)
             o += tables[k].nbytes
+        keys_addr = C.c_void_p(dev_blob.data_ptr() + o)
 
         L, s = lib(), stream_ptr()
         md = L.rehr_intensity_moment_doubles()
@@ -249,10 +283,13 @@ class IntensityAugment:
         for k in fired:
             n, tab = len(plan.rows[k]), addr[k]
             if k == "noise":
-                nz = torch.empty(n * V, **f32)
-                for r, field in enumerate(plan.noise):
-                    nz[r * V:(r + 1) * V].copy_(field, non_blocking=True)
-                check(L.rehr_intensity_pointwise(x, tab, n, V, 0, ptr(nz), None, s), "intensity_noise")
+                if philox:
+                    check(L.rehr_intensity_noise_philox(x, tab, keys_addr, n, V, s), "intensity_noise_philox")
+                else:
+                    nz = torch.empty(n * V, **f32)
+                    for r, field in enumerate(plan.noise):
+                        nz[r * V:(r + 1) * V].copy_(field, non_blocking=True)
+                    check(L.rehr_intensity_pointwise(x, tab, n, V, 0, ptr(nz), None, s), "intensity_noise")
                 F_._count(1)
             elif k == "blur":
                 t1, t2 = torch.empty(n * V, **f32), torch.empty(n * V, **f32)

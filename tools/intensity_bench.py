@@ -3,8 +3,11 @@ Writes one JSON file (default profiles/intensity_bench.json) with the GPU's name
   - CUDA-event time of `apply` with each transform forced on alone, for [2,1,16,256,256] and [8,1,16,256,256] patches, with the
     bytes its passes move and their share of 7.7 TB/s (HBM3e, B200 data sheet).  At these sizes the kernels are short and the call
     is bound by launches and host work, not by HBM: the share of peak says how far from the bandwidth bound it is, nothing more;
-  - host time of `draw` with only the noise forced on (the noise field comes from np.random.normal on the host);
-  - Stage2Sampler.batch samples/s, with IntensityAugment() (the reference's probabilities) and without intensity;
+  - the same for the noise with `noise_rng="philox"` (the field generated in the kernel: one read and one write of x);
+  - host time of `draw` with only the noise forced on: np.random.normal of the whole field on the host (the default), and a
+    128-bit key per row with `noise_rng="philox"`;
+  - Stage2Sampler.batch samples/s, with IntensityAugment() (the reference's probabilities), with
+    IntensityAugment(noise_rng="philox"), with the noise switched off (the other six transforms' share) and without intensity;
   - the oracle chain (numpy / scipy, one process) on the same batch shapes.
 Usage: python tools/intensity_bench.py [out.json]"""
 import json
@@ -37,7 +40,7 @@ def moved_bytes(name, plan):
     total = 0
     for r in plan.rows[name]:
         if name == "noise":
-            total += 3 * v                       # read x and the noise field, write x
+            total += 2 * v if plan.noise_rng == "philox" else 3 * v   # read x (and the noise field), write x
         elif name == "blur":
             total += 6 * v                       # three axis passes, each reads and writes a volume
         elif name == "brightness":
@@ -52,8 +55,8 @@ def moved_bytes(name, plan):
     return 4 * total
 
 
-def time_apply(name, b, iters=20):
-    aug = IntensityAugment(**{**OFF, name: FORCED[name]})
+def time_apply(name, b, iters=20, noise_rng="numpy"):
+    aug = IntensityAugment(noise_rng=noise_rng, **{**OFF, name: FORCED[name]})
     src = torch.randn(b, 1, 16, 256, 256, device="cuda")
     x = src.clone()
     plan = aug.draw(b, 1, (16, 256, 256), random.Random(0), np.random.RandomState(0))
@@ -75,16 +78,17 @@ def time_apply(name, b, iters=20):
             "bytes": nbytes, "GB_per_s": round(nbytes / (med * 1e-3) / 1e9, 1), "share_of_7.7TBps": round(nbytes / (med * 1e-3) / HBM, 4)}
 
 
-def time_noise_draw(b, iters=5):
-    aug = IntensityAugment(**{**OFF, "noise": FORCED["noise"]})
+def time_noise_draw(b, iters=5, noise_rng="numpy"):
+    """Host ms per draw."""
+    aug = IntensityAugment(noise_rng=noise_rng, **{**OFF, "noise": FORCED["noise"]})
     rn, rp = np.random.RandomState(0), random.Random(0)
     t0 = time.perf_counter()
     for _ in range(iters):
         aug.draw(b, 1, (16, 256, 256), rp, rn)
-    return round((time.perf_counter() - t0) / iters * 1e3, 2)
+    return (time.perf_counter() - t0) / iters * 1e3
 
 
-def time_sampler(intensity, b, iters=10):
+def time_sampler(intensity, b, iters=40):
     rng = np.random.RandomState(1)
     ds = augment.Stage2Sampler((256, 256, 16), 4, intensity=intensity)
     ds.add_subject((rng.rand(288, 288, 80) * 300).astype(np.float32), (rng.rand(288, 288, 80) > 0.6).astype(np.uint8),
@@ -118,14 +122,20 @@ def main():
     res = {"gpu": gpu.strip().splitlines()[0] if gpu.strip() else None, "torch_device": torch.cuda.get_device_name(0),
            "note": "apply() time per call from CUDA events around the whole call (host table build + launches + kernels); at these "
                    "sizes launch- and host-bound, so share_of_7.7TBps is far below 1 by construction",
-           "apply_forced_alone": {}, "noise_draw_host_ms": {}, "sampler_batch": {}, "oracle_chain_host": {}}
+           "apply_forced_alone": {}, "noise_draw_host_ms": {}, "noise_draw_host_us_philox": {}, "sampler_batch": {},
+           "oracle_chain_host": {}}
     for name in NAMES:
         res["apply_forced_alone"][name] = [time_apply(name, b) for b in (2, 8)]
         print(name, res["apply_forced_alone"][name], flush=True)
+    res["apply_forced_alone"]["noise_philox"] = [time_apply("noise", b, noise_rng="philox") for b in (2, 8)]
+    print("noise_philox", res["apply_forced_alone"]["noise_philox"], flush=True)
     for b in (2, 8):
-        res["noise_draw_host_ms"][f"b{b}"] = time_noise_draw(b)
+        res["noise_draw_host_ms"][f"b{b}"] = round(time_noise_draw(b), 2)
+        res["noise_draw_host_us_philox"][f"b{b}"] = round(time_noise_draw(b, iters=2000, noise_rng="philox") * 1e3, 1)
     for b in (2, 8):
         res["sampler_batch"][f"b{b}_intensity_defaults"] = time_sampler(IntensityAugment(), b)
+        res["sampler_batch"][f"b{b}_intensity_defaults_philox"] = time_sampler(IntensityAugment(noise_rng="philox"), b)
+        res["sampler_batch"][f"b{b}_intensity_no_noise"] = time_sampler(IntensityAugment(noise={"p_per_sample": 0.0}), b)
         res["sampler_batch"][f"b{b}_no_intensity"] = time_sampler(None, b)
         res["oracle_chain_host"][f"b{b}_defaults"] = time_oracle(b, {}, seeds=5)
         res["oracle_chain_host"][f"b{b}_forced"] = time_oracle(b, FORCED, seeds=1)
