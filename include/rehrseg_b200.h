@@ -66,8 +66,8 @@ const char* rehr_strerror(int status);
 int rehr_last_cuda_error(void);     /* cudaError_t of the last failing CUDA call on this thread */
 int rehr_version(void);             /* ABI version, currently 6 (4: rehr_tensor.dtype, dtype arguments of the weight packers; 5: batched
                                      * re-pack and fused InstanceNorm-backward sums added -- additive; 6: the normalise-on-load and fused
-                                     * InstanceNorm-backward-sum entry points removed; the rehr_intensity_* entry points were added
-                                     * later without a bump -- additive) */
+                                     * InstanceNorm-backward-sum entry points removed; the rehr_intensity_* and rehr_sr_loss_* entry
+                                     * points were added later without a bump -- additive) */
 int rehr_device_sm_count(void);
 
 /* ------------------------------------------------------------------------------------------------
@@ -401,6 +401,16 @@ int rehr_mean_stack(const float* const* vols_dev_ptrs, int K, float* out, long l
  *   rehr_plane_maxpool      CriterionPairWiseforWholeFeatAfterPool (models/seg_model.py:95-113): x [N][C][S][H][W], windows ph x pw,
  *                           stride = window, ceil mode -> out, idx [N][S][C][OH][OW] (idx = first arg-max inside the H*W plane)
  *   rehr_plane_maxpool_bwd  g, idx -> scatter into the caller-zeroed dx [N][C][S][H][W]
+ * and of the SR-stage step (the loss statements of train_sr, train_all.py:124-133):
+ *   rehr_sr_loss_sums       L1Loss(hat[:, 0:1], t[:, 0:1]), with the UASR head mean(|e| / u + log u) and L1Loss(u, |e|.detach())
+ *                           (:125-130), and BCEDiceLoss(hat[:, 1:], t[:, 1:]) (:133, utils/seg_utils.py:821-886).  hat [B][C][S][HW]
+ *                           contiguous (channel 0 the image, 1..C-1 segmentation logits, 2 <= C <= 4); target: contiguous H*W
+ *                           planes at batch / channel / depth strides t_batch, t_channel, t_depth (elements), so the depth window
+ *                           of patches_hr is read in place; u [B][1][S][HW] or NULL (plain head).  partial
+ *                           [rehr_loss_blocks(B*S*HW)][3 + 4(C-1)] = {sum |e|, sum |e|/u + log u, sum |u - |e||, then per
+ *                           segmentation channel sum bce(x, y), sum p*y, sum p^2, sum y^2}, e = hat_0 - t_0, p = sigmoid(x)
+ *   rehr_sr_loss_bwd        g [3 + 4(C-1)] (device; gradients of the sums in the same order) -> d_hat [B][C][S][HW] and
+ *                           d_u [B][1][S][HW] (non-NULL exactly when u is); sign(0) = 0 as torch's abs backward
  * ---------------------------------------------------------------------------------------------- */
 int rehr_loss_blocks(long long voxels);
 int rehr_seg_loss_sums(const float* logits, const float* target, const float* weight, int B, int C, long long V, float* partial,
@@ -413,6 +423,10 @@ int rehr_cosine_sums_bwd(const float* a, const float* b, int B, int C, long long
 int rehr_plane_maxpool(const float* x, int N, int C, int S, int H, int W, int ph, int pw, float* out, int* idx, rehr_stream stream);
 int rehr_plane_maxpool_bwd(const float* g, const int* idx, int N, int C, int S, int H, int W, int ph, int pw, float* dx_zeroed,
                            rehr_stream stream);
+int rehr_sr_loss_sums(const float* hat, const float* target, const float* u, int B, int C, int S, int HW, long long t_batch,
+                      long long t_channel, long long t_depth, float* partial, rehr_stream stream);
+int rehr_sr_loss_bwd(const float* hat, const float* target, const float* u, int B, int C, int S, int HW, long long t_batch,
+                     long long t_channel, long long t_depth, const float* g, float* d_hat, float* d_u, rehr_stream stream);
 
 #ifdef __cplusplus
 }

@@ -155,6 +155,8 @@ def _declare(L: C.CDLL) -> None:
         "rehr_cosine_sums_bwd": (i, [vp, vp, i, i, ll, vp, vp, vp, vp]),
         "rehr_plane_maxpool": (i, [vp, i, i, i, i, i, i, i, vp, vp, vp]),
         "rehr_plane_maxpool_bwd": (i, [vp, vp, i, i, i, i, i, i, i, vp, vp]),
+        "rehr_sr_loss_sums": (i, [vp, vp, vp, i, i, i, i, ll, ll, ll, vp, vp]),
+        "rehr_sr_loss_bwd": (i, [vp, vp, vp, i, i, i, i, ll, ll, ll, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

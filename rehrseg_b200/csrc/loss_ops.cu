@@ -1,4 +1,4 @@
-// Fused reduction kernels for the stage-2 losses (SURVEY.md 8(f) row 4: "the losses as fused CE+Dice reductions"), all HBM-bound
+// Fused reduction kernels for the stage-2 and SR-stage losses (SURVEY.md 8(f) row 4: "the losses as fused CE+Dice reductions"), all HBM-bound
 // single passes over fp32 NCDHW tensors exactly as the caller holds them (no layout change):
 //
 //   * segmentation loss sums   <- DC_and_weighted_CE_loss, utils/seg_utils.py:305-353 (RobustCrossEntropyLoss :289-303 and the
@@ -7,7 +7,9 @@
 //   * channel-cosine sums      <- cosine_distance_loss, models/seg_model.py:60-78: per (sample, channel) sums over the voxels of
 //                                 the channel-normalised maps (a.b, a.a, b.b);
 //   * plane max-pool           <- CriterionPairWiseforWholeFeatAfterPool, models/seg_model.py:95-113: per (sample, channel, slice)
-//                                 max over non-overlapping in-plane windows (ceil mode) with the arg-max for the backward scatter.
+//                                 max over non-overlapping in-plane windows (ceil mode) with the arg-max for the backward scatter;
+//   * SR-stage loss sums       <- the loss statements of train_sr, train_all.py:124-133 (L1, the UASR terms, BCEDiceLoss): the
+//                                 voxel sums of all of them from ONE read of the network output, the target window and u.
 //
 // Each forward kernel only produces the SUMS; the few scalars of the actual loss (Dice ratio, 1 - cos, Gram matrices) are then
 // ordinary autograd ops on tiny tensors in rehrseg_b200/loss_ops.py, and each backward kernel turns the gradients of those sums
@@ -21,6 +23,7 @@
 namespace rehr {
 
 static constexpr int kLossMaxClasses = 8;
+static constexpr int kSrMaxChannels = 4;   // SR-stage output channels (the reference has 2); more spill the unrolled accumulators
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
@@ -285,7 +288,203 @@ __global__ void plane_maxpool_bwd_kernel(const float* __restrict__ g, const int*
   dx[((n * C + c) * S + s) * HW + idx[i]] = g[i];
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// SR-stage loss sums <- train_all.py:124-133: L1Loss on channel 0, the UASR terms :126-129 and BCEDiceLoss (utils/seg_utils.py:
+// 821-886) on channels 1..C-1, from ONE read of the network output, the target and the uncertainty.
+// hat [B][C][S][HW] f32 contiguous; target [B][C][S][HW] with contiguous H*W planes and the given batch / channel / depth strides
+// (the depth window of patches_hr is read in place); u [B][1][S][HW] or null.  e = hat_0 - t_0, p = sigmoid(hat_c), y = t_c.
+// partial [blocks][3 + 4 (C-1)]: sum |e|, sum |e|/u + log u, sum |u - |e||, then per segmentation channel sum bce, sum p*y,
+// sum p^2, sum y^2.  One item = four voxels of one plane: 16-byte accesses when every plane start is aligned (VEC), masked
+// scalars otherwise (ragged H*W, odd strides).
+// ------------------------------------------------------------------------------------------------------------------
+struct SrLossView {
+  const float* hat;
+  const float* target;
+  const float* u;
+  long long tb, tc, ts;  // target strides (elements)
+  int S, HW;
+  long long items;       // B * S * ceil(HW / 4)
+};
+
+template <bool VEC>
+__device__ __forceinline__ void sr_ld4(const float* p, int n, bool last_use, float (&v)[4]) {
+  if (VEC) {
+    const float4 t = last_use ? __ldcs(reinterpret_cast<const float4*>(p)) : __ldg(reinterpret_cast<const float4*>(p));
+    v[0] = t.x, v[1] = t.y, v[2] = t.z, v[3] = t.w;
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) v[k] = k < n ? (last_use ? __ldcs(p + k) : __ldg(p + k)) : 0.f;
+  }
+}
+
+template <bool VEC>
+__device__ __forceinline__ void sr_st4(float* p, int n, const float (&v)[4]) {
+  if (VEC) {
+    *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+      if (k < n) p[k] = v[k];
+  }
+}
+
+// sigmoid(x) and 1 - sigmoid(x), each without cancellation; ex = exp(-|x|) is returned for the BCE's log1p
+__device__ __forceinline__ void sr_sigmoid(float x, float& p, float& q, float& ex) {
+  ex = expf(-fabsf(x));
+  const float r = 1.f / (1.f + ex);
+  p = x >= 0.f ? r : ex * r;
+  q = x >= 0.f ? ex * r : r;
+}
+
+__device__ __forceinline__ float sr_sign(float v) { return v > 0.f ? 1.f : (v < 0.f ? -1.f : 0.f); }  // sign(0) = 0, as torch
+
+// item i -> (plane = b*S + s, first voxel of the item inside the plane, valid voxels)
+__device__ __forceinline__ void sr_item(const SrLossView& a, long long i, long long& plane, long long& b, int& s, int& off, int& n) {
+  const int vpp = (a.HW + 3) >> 2;
+  plane = i / vpp;
+  off = (int)(i - plane * vpp) * 4;
+  n = min(4, a.HW - off);
+  b = plane / a.S;
+  s = (int)(plane - b * a.S);
+}
+
+template <int C, bool VEC>
+__global__ void __launch_bounds__(256) sr_loss_sums_kernel(const SrLossView a, float* __restrict__ partial) {
+  constexpr int K = 3 + 4 * (C - 1);
+  __shared__ float slot[8][K];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long cstride = (long long)a.S * a.HW;
+  float acc[K];
+#pragma unroll
+  for (int i = 0; i < K; ++i) acc[i] = 0.f;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < a.items; i += (long long)gridDim.x * blockDim.x) {
+    long long plane, b;
+    int s, off, n;
+    sr_item(a, i, plane, b, s, off, n);
+    const float* h = a.hat + (b * C * a.S + s) * (long long)a.HW + off;
+    const float* t = a.target + b * a.tb + s * a.ts + off;
+    float hv[4], tv[4];
+    sr_ld4<VEC>(h, n, false, hv);
+    sr_ld4<VEC>(t, n, false, tv);
+    if (a.u) {
+      float uv[4];
+      sr_ld4<VEC>(a.u + plane * a.HW + off, n, false, uv);
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if (VEC || k < n) {
+          const float ae = fabsf(hv[k] - tv[k]);
+          acc[0] += ae;
+          acc[1] += ae / uv[k] + logf(uv[k]);
+          acc[2] += fabsf(uv[k] - ae);
+        }
+    } else {
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if (VEC || k < n) acc[0] += fabsf(hv[k] - tv[k]);
+    }
+#pragma unroll
+    for (int c = 1; c < C; ++c) {
+      sr_ld4<VEC>(h + c * cstride, n, false, hv);
+      sr_ld4<VEC>(t + c * a.tc, n, false, tv);
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if (VEC || k < n) {
+          const float x = hv[k], y = tv[k];
+          float p, q, ex;
+          sr_sigmoid(x, p, q, ex);
+          acc[4 * c - 1] += (1.f - y) * x + fmaxf(-x, 0.f) + log1pf(ex);
+          acc[4 * c] += p * y;
+          acc[4 * c + 1] += p * p;
+          acc[4 * c + 2] += y * y;
+        }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < K; ++i) {
+    const float t = warp_sum(acc[i]);
+    if (lane == 0) slot[warp][i] = t;
+  }
+  __syncthreads();
+  if (threadIdx.x < K) {
+    float t = 0.f;
+#pragma unroll
+    for (int w = 0; w < 8; ++w) t += slot[w][threadIdx.x];
+    partial[(long long)blockIdx.x * K + threadIdx.x] = t;
+  }
+}
+
+// g [3 + 4 (C-1)]: the gradients of the sums, in the order of the partials (the sum y^2 entries are ignored).
+//   d hat_0 = sign(e) (g_abs + g_uasr / u)                    (the sum |u - |e|| has no hat gradient: the error map is detached)
+//   d u     = g_uasr / u (1 - |e| / u) + g_l1u sign(u - |e|)
+//   d hat_c = g_bce (p - y) + (g_py y + 2 g_pp p) p (1 - p)
+template <int C, bool VEC>
+__global__ void __launch_bounds__(256) sr_loss_bwd_kernel(const SrLossView a, const float* __restrict__ g, float* __restrict__ d_hat,
+                                                          float* __restrict__ d_u) {
+  const float g_abs = g[0], g_uasr = g[1], g_l1u = g[2];
+  float gb[C], gy[C], gp[C];
+#pragma unroll
+  for (int c = 1; c < C; ++c) {
+    gb[c] = g[4 * c - 1];
+    gy[c] = g[4 * c];
+    gp[c] = 2.f * g[4 * c + 1];
+  }
+  const long long cstride = (long long)a.S * a.HW;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < a.items; i += (long long)gridDim.x * blockDim.x) {
+    long long plane, b;
+    int s, off, n;
+    sr_item(a, i, plane, b, s, off, n);
+    const long long ho = (b * C * a.S + s) * (long long)a.HW + off;
+    const float* t = a.target + b * a.tb + s * a.ts + off;
+    float hv[4], tv[4], dv[4];
+    sr_ld4<VEC>(a.hat + ho, n, true, hv);
+    sr_ld4<VEC>(t, n, true, tv);
+    if (a.u) {
+      float uv[4], du[4];
+      sr_ld4<VEC>(a.u + plane * a.HW + off, n, true, uv);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const float e = hv[k] - tv[k], ae = fabsf(e), gu = g_uasr / uv[k];
+        dv[k] = sr_sign(e) * (g_abs + gu);
+        du[k] = gu * (1.f - ae / uv[k]) + g_l1u * sr_sign(uv[k] - ae);
+      }
+      sr_st4<VEC>(d_u + plane * a.HW + off, n, du);
+    } else {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) dv[k] = sr_sign(hv[k] - tv[k]) * g_abs;
+    }
+    sr_st4<VEC>(d_hat + ho, n, dv);
+#pragma unroll
+    for (int c = 1; c < C; ++c) {
+      sr_ld4<VEC>(a.hat + ho + c * cstride, n, true, hv);
+      sr_ld4<VEC>(t + c * a.tc, n, true, tv);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const float y = tv[k];
+        float p, q, ex;
+        sr_sigmoid(hv[k], p, q, ex);
+        dv[k] = gb[c] * ((1.f - y) * p - y * q) + (gy[c] * y + gp[c] * p) * (p * q);   // p - y, exact at saturated logits
+      }
+      sr_st4<VEC>(d_hat + ho + c * cstride, n, dv);
+    }
+  }
+}
+
 static int loss_blocks(long long V) { return (int)std::max<long long>(1, std::min<long long>((V + 255) / 256, (long long)sm_count() * 4)); }
+
+static bool sr_view(const float* hat, const float* target, const float* u, int B, int C, int S, int HW, long long tb, long long tc,
+                    long long ts, SrLossView& a) {
+  if (!hat || !target || B <= 0 || C < 2 || S <= 0 || HW <= 0) return false;
+  a = SrLossView{hat, target, u, tb, tc, ts, S, HW, (long long)B * S * ((HW + 3) / 4)};
+  return true;
+}
+
+static bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
+
+// every plane start of every tensor is 16-byte aligned
+static bool sr_vec(const SrLossView& a, const float* d_hat, const float* d_u) {
+  return a.HW % 4 == 0 && a.tb % 4 == 0 && a.tc % 4 == 0 && a.ts % 4 == 0 && aligned16(a.hat) && aligned16(a.target) &&
+         aligned16(a.u) && aligned16(d_hat) && aligned16(d_u);
+}
 
 }  // namespace rehr
 
@@ -324,6 +523,47 @@ int rehr_seg_loss_bwd(const float* logits, const float* target, const float* wei
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }
+
+#define REHR_SR_DISPATCH(LAUNCH)                                                                                        \
+  switch (C) {                                                                                                           \
+    case 2: LAUNCH(2); break;                                                                                            \
+    case 3: LAUNCH(3); break;                                                                                            \
+    case 4: LAUNCH(4); break;                                                                                            \
+  }
+
+int rehr_sr_loss_sums(const float* hat, const float* target, const float* u, int B, int C, int S, int HW, long long t_batch,
+                      long long t_channel, long long t_depth, float* partial, rehr_stream stream) {
+  SrLossView a;
+  if (!partial || !sr_view(hat, target, u, B, C, S, HW, t_batch, t_channel, t_depth, a)) return REHR_BAD_SHAPE;
+  if (C > kSrMaxChannels) return REHR_UNSUPPORTED;
+  const unsigned grid = (unsigned)loss_blocks((long long)B * S * HW);
+  const bool vec = sr_vec(a, nullptr, nullptr);
+#define REHR_SR_SUMS(N)                                                                  \
+  if (vec) sr_loss_sums_kernel<N, true><<<grid, 256, 0, (cudaStream_t)stream>>>(a, partial); \
+  else sr_loss_sums_kernel<N, false><<<grid, 256, 0, (cudaStream_t)stream>>>(a, partial)
+  REHR_SR_DISPATCH(REHR_SR_SUMS)
+#undef REHR_SR_SUMS
+  REHR_CHECK_LAUNCH();
+  return REHR_OK;
+}
+
+int rehr_sr_loss_bwd(const float* hat, const float* target, const float* u, int B, int C, int S, int HW, long long t_batch,
+                     long long t_channel, long long t_depth, const float* g, float* d_hat, float* d_u, rehr_stream stream) {
+  SrLossView a;
+  if (!g || !d_hat || (u != nullptr) != (d_u != nullptr) || !sr_view(hat, target, u, B, C, S, HW, t_batch, t_channel, t_depth, a))
+    return REHR_BAD_SHAPE;
+  if (C > kSrMaxChannels) return REHR_UNSUPPORTED;
+  const unsigned grid = (unsigned)loss_blocks((long long)B * S * HW);
+  const bool vec = sr_vec(a, d_hat, d_u);
+#define REHR_SR_BWD(N)                                                                                \
+  if (vec) sr_loss_bwd_kernel<N, true><<<grid, 256, 0, (cudaStream_t)stream>>>(a, g, d_hat, d_u);   \
+  else sr_loss_bwd_kernel<N, false><<<grid, 256, 0, (cudaStream_t)stream>>>(a, g, d_hat, d_u)
+  REHR_SR_DISPATCH(REHR_SR_BWD)
+#undef REHR_SR_BWD
+  REHR_CHECK_LAUNCH();
+  return REHR_OK;
+}
+#undef REHR_SR_DISPATCH
 
 int rehr_cosine_sums(const float* a, const float* b, int B, int C, long long V, float* partial, rehr_stream stream) {
   if (!a || !b || !partial || B <= 0 || C <= 0 || V <= 0) return REHR_BAD_SHAPE;

@@ -3,6 +3,8 @@
 Opt-in counterparts of the plain-PyTorch mirrors in `train_step.py` (same constructors, same values):
   * `FusedDCAndWeightedCELoss` <- `DC_and_weighted_CE_loss` as `_build_loss` configures it (utils/seg_utils.py:305-372)
   * `FusedDistiller`           <- `Distiller` (models/seg_model.py:115-151)
+  * `FusedSRLoss`              <- the SR-stage loss statements of `sr_train_step` with `nn.L1Loss()` and `BCEDiceLoss(alpha, beta)`
+                                  (train_all.py:124-133, incl. the UASR terms)
 Each kernel makes one pass over the fp32 NCDHW tensor and returns per-(sample, class/channel) SUMS; the handful of scalar
 operations that turn sums into the loss stay ordinary autograd ops on tiny tensors, and the backward kernels consume the
 gradients of the sums.  CUDA only: like every engine op they raise `RehrError` on a CPU tensor or a missing library.
@@ -120,6 +122,63 @@ class PlaneMaxPool(torch.autograd.Function):
         return dx.to(dt), None, None
 
 
+def _plane_strides(t: torch.Tensor, what: str) -> tuple:
+    """(batch, channel, depth) element strides of a [B,C,S,H,W] CUDA tensor whose H*W planes are contiguous."""
+    if not t.is_cuda:
+        raise L.RehrError(f"{what}: expected a CUDA tensor (rehrseg_b200 has no CPU path)")
+    h, w = t.shape[3], t.shape[4]
+    if (w > 1 and t.stride(4) != 1) or (h > 1 and t.stride(3) != w):
+        raise L.RehrError(f"{what}: the H*W planes must be contiguous (strides {tuple(t.stride())})")
+    return t.stride(0), t.stride(1), t.stride(2)
+
+
+class SRLossSums(torch.autograd.Function):
+    """(hat [B,C,S,H,W], target [B,C,S,H,W] with contiguous H*W planes, u [B,1,S,H,W] or None) -> sums [3 + 4 (C-1)]:
+    sum |e|, sum |e|/u + log u, sum |u - |e||, then per segmentation channel c = 1..C-1: sum bce(hat_c, t_c), sum p*t_c,
+    sum p^2, sum t_c^2, where e = hat_0 - t_0 and p = sigmoid(hat_c) (the u terms are 0 without u).  The target is read in
+    place (a depth window of patches_hr needs no copy); gradients flow to `hat` and `u` only."""
+
+    @staticmethod
+    def forward(ctx, hat, target, u):
+        from . import functional as F_
+        h32 = _f32c(hat.detach(), "sr_loss_sums")
+        u32 = _f32c(u.detach(), "sr_loss_sums") if u is not None else None
+        if h32.dim() != 5 or target.shape != h32.shape or h32.shape[1] < 2:
+            raise L.RehrError(f"sr_loss_sums: hat and target must be equal [B,C>=2,S,H,W] shapes, got {tuple(h32.shape)} and "
+                              f"{tuple(target.shape)}")
+        tg = target.detach() if target.dtype == torch.float32 else target.detach().float()
+        strides = _plane_strides(tg, "sr_loss_sums target")
+        b, c, s, hh, ww = h32.shape
+        if u32 is not None and u32.shape != (b, 1, s, hh, ww):
+            raise L.RehrError(f"sr_loss_sums: uncertainty must be [B,1,S,H,W] = {(b, 1, s, hh, ww)}, got {tuple(u32.shape)}")
+        if tg.device != h32.device or (u32 is not None and u32.device != h32.device):
+            raise L.RehrError("sr_loss_sums: hat, target and uncertainty must be on one device")
+        with L.device_of(h32):
+            blocks = lib().rehr_loss_blocks(b * s * hh * ww)
+            partial = torch.empty((blocks, 3 + 4 * (c - 1)), dtype=torch.float32, device=h32.device)
+            check(lib().rehr_sr_loss_sums(ptr(h32), ptr(tg), ptr(u32), b, c, s, hh * ww, *strides, ptr(partial), stream_ptr()),
+                  "sr_loss_sums")
+            F_._count()
+            sums = partial.sum(0)
+        ctx.save_for_backward(h32, tg, u32)
+        ctx.meta = (strides, hat.dtype, None if u is None else u.dtype)
+        return sums
+
+    @staticmethod
+    def backward(ctx, g):
+        from . import functional as F_
+        h32, tg, u32 = ctx.saved_tensors
+        strides, hdt, udt = ctx.meta
+        b, c, s, hh, ww = h32.shape
+        d_hat = torch.empty_like(h32)
+        d_u = torch.empty_like(u32) if u32 is not None else None
+        with L.device_of(h32):
+            check(lib().rehr_sr_loss_bwd(ptr(h32), ptr(tg), ptr(u32), b, c, s, hh * ww, *strides, ptr(g.float().contiguous()),
+                                         ptr(d_hat), ptr(d_u), stream_ptr()), "sr_loss_bwd")
+            F_._count()
+        return d_hat.to(hdt), None, (d_u.to(udt) if d_u is not None else None)
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # loss modules
 # ---------------------------------------------------------------------------------------------------------------
@@ -183,6 +242,31 @@ class FusedDistiller(nn.Module):
         if self.lambda_cosine > 0:
             loss = loss + self.lambda_cosine * fused_cosine_distance_loss(projected, feature_teacher)
         return loss
+
+
+class FusedSRLoss(nn.Module):
+    """The SR-stage loss of `train_step.sr_train_step` (train_all.py:124-133) on one fused reduction per direction:
+    `L1Loss` on channel 0, with the UASR head `mean(|e| / u + log u) + L1Loss(u, |e|.detach())`, plus
+    `BCEDiceLoss(alpha, beta)` on channels 1..C-1.  `forward(hat, target, uncertainty)` takes the network output, the target
+    window (a strided view is read in place) and, exactly when `enable_uncertainty`, the uncertainty map."""
+
+    def __init__(self, alpha: float = 1.0, beta: float = 1.0, enable_uncertainty: bool = False):
+        super().__init__()
+        self.alpha, self.beta, self.enable_uncertainty = alpha, beta, enable_uncertainty
+
+    def forward(self, hat: torch.Tensor, target: torch.Tensor, uncertainty: Optional[torch.Tensor] = None) -> torch.Tensor:
+        if (uncertainty is not None) != self.enable_uncertainty:
+            raise L.RehrError(f"FusedSRLoss(enable_uncertainty={self.enable_uncertainty}) called "
+                              f"{'without' if uncertainty is None else 'with'} an uncertainty map")
+        sums = SRLossSums.apply(hat, target, uncertainty)
+        n = hat[:, 0].numel()
+        k = hat.shape[1] - 1
+        loss = sums[0] / n
+        if uncertainty is not None:
+            loss = loss + (sums[1] + sums[2]) / n
+        per = sums[3:].view(k, 4)
+        dice = 2 * per[:, 1] / (per[:, 2] + per[:, 3]).clamp(min=1e-6)
+        return loss + (self.alpha * per[:, 0].sum() / (n * k) + self.beta * (1.0 - dice.mean()))
 
 
 def build_fused_loss(enable_deep_supervision: bool = False, weight_dice: float = 1) -> nn.Module:

@@ -12,6 +12,7 @@
                               distillation on `features_seg[1]` / `features_sr[1]`, zero_grad / backward / step.
   * `BCEDiceLoss`, `sr_train_step` <- the SR-stage loss `BCEDiceLoss(alpha, beta)` (utils/seg_utils.py:786-886) and the loop body
                               of `train_sr`, train_all.py:118-139, incl. the UASR terms :125-130 (L1 + |err|/u + log u + L1(u, |err|)).
+  * `GraphedSRStep`        <- the same SR-stage iteration replayed from one CUDA graph (as `GraphedJointStep` for stage 2).
   * `allreduce_gradients`  <- what DistributedDataParallel would do for the reference: one flat bucket, mean over ranks
                               (NCCL over NVLink; InstanceNorm is per sample, so no other cross-rank traffic exists).
 
@@ -306,31 +307,41 @@ class BCEDiceLoss(nn.Module):
         return self.alpha * self.bce(input, target) + self.beta * (1.0 - dice.mean())
 
 
-def sr_train_step(model: nn.Module, batch: Sequence[torch.Tensor], loss_obj: nn.Module, loss_seg: nn.Module,
-                  opt: Optional[torch.optim.Optimizer] = None, scheduler=None, slice_separation: int = 4, num_slices: int = 4,
-                  enable_uncertainty: bool = False, group=None, device=None) -> dict:
-    """One iteration of `train_sr` (train_all.py:118-139).  `batch` = (patches_lr [B,2,num_slices,H,W], patches_hr [B,2,S,H,W]) as the
-    DataLoader yields them; with `num_slices > 1` the target is the `slice_separation` HR slices between the two central LR slices
-    (:122-123).  `enable_uncertainty` adds the UASR terms :125-130 on the model's (prediction, uncertainty) pair.  The reference
-    calls `model(patches_lr)`, whose forward subtracts the channel-0 mean IN PLACE from the batch (FLAVR_arch.py:180-181) --
-    preserved: `patches_lr` on the device is mutated.  Gradients are averaged over `group` before the optimiser step."""
-    patches_lr, patches_hr = batch
-    device = device if device is not None else next(model.parameters()).device
-    patches_hr = patches_hr.to(device, non_blocking=True)
-    patches_lr = patches_lr.to(device, non_blocking=True)
+def _sr_loss(out, patches_hr: torch.Tensor, loss_obj: Optional[nn.Module], loss_seg: Optional[nn.Module], slice_separation: int,
+             num_slices: int, enable_uncertainty: bool, fused_loss: Optional[nn.Module]) -> torch.Tensor:
+    """The loss of train_all.py:122-133 from the model output `out` ((prediction, uncertainty) with the UASR head) and the full
+    HR batch: the target window, then the plain statements or, when given, `fused_loss` (loss_ops.FusedSRLoss)."""
     if num_slices > 1:
         patches_hr = patches_hr[:, :, int(slice_separation) * (num_slices // 2 - 1):int(slice_separation) * (num_slices // 2), ...]
+    patches_hr_hat, uncertainty = out if enable_uncertainty else (out, None)
+    if fused_loss is not None:
+        return fused_loss(patches_hr_hat, patches_hr, uncertainty)
     if enable_uncertainty:
-        patches_hr_hat, uncertainty = model(patches_lr)
         loss = loss_obj(patches_hr_hat[:, 0:1, ...], patches_hr[:, 0:1, ...])
         loss = loss + torch.mean(torch.div(torch.abs(patches_hr_hat[:, 0:1, ...] - patches_hr[:, 0:1, ...]), uncertainty)
                                  + torch.log(uncertainty))
         error_map = torch.abs(patches_hr_hat[:, 0:1, ...].detach() - patches_hr[:, 0:1, ...])
         loss = loss + loss_obj(uncertainty, error_map)
     else:
-        patches_hr_hat = model(patches_lr)
         loss = loss_obj(patches_hr_hat[:, 0:1, ...], patches_hr[:, 0:1, ...])
-    loss = loss + loss_seg(patches_hr_hat[:, 1:, ...], patches_hr[:, 1:, ...]) * 1.0
+    return loss + loss_seg(patches_hr_hat[:, 1:, ...], patches_hr[:, 1:, ...]) * 1.0
+
+
+def sr_train_step(model: nn.Module, batch: Sequence[torch.Tensor], loss_obj: nn.Module, loss_seg: nn.Module,
+                  opt: Optional[torch.optim.Optimizer] = None, scheduler=None, slice_separation: int = 4, num_slices: int = 4,
+                  enable_uncertainty: bool = False, group=None, device=None, fused_loss: Optional[nn.Module] = None) -> dict:
+    """One iteration of `train_sr` (train_all.py:118-139).  `batch` = (patches_lr [B,2,num_slices,H,W], patches_hr [B,2,S,H,W]) as the
+    DataLoader yields them; with `num_slices > 1` the target is the `slice_separation` HR slices between the two central LR slices
+    (:122-123).  `enable_uncertainty` adds the UASR terms :125-130 on the model's (prediction, uncertainty) pair.  The reference
+    calls `model(patches_lr)`, whose forward subtracts the channel-0 mean IN PLACE from the batch (FLAVR_arch.py:180-181) --
+    preserved: `patches_lr` on the device is mutated.  Gradients are averaged over `group` before the optimiser step.
+    `fused_loss` (opt-in, a `loss_ops.FusedSRLoss` built with the same alpha, beta and enable_uncertainty) replaces the loss
+    statements with one fused CUDA reduction per direction; `loss_obj` / `loss_seg` are then unused."""
+    patches_lr, patches_hr = batch
+    device = device if device is not None else next(model.parameters()).device
+    patches_hr = patches_hr.to(device, non_blocking=True)
+    patches_lr = patches_lr.to(device, non_blocking=True)
+    loss = _sr_loss(model(patches_lr), patches_hr, loss_obj, loss_seg, slice_separation, num_slices, enable_uncertainty, fused_loss)
     params = list(model.parameters())
     if opt is not None:
         opt.zero_grad()
@@ -344,3 +355,37 @@ def sr_train_step(model: nn.Module, batch: Sequence[torch.Tensor], loss_obj: nn.
     if scheduler is not None:
         scheduler.step()
     return {"loss": loss.detach()}
+
+
+class GraphedSRStep:
+    """The SR-stage iteration (train_all.py:118-138: forward, target window, L1 / UASR / BCE-Dice loss, backward) captured into ONE
+    CUDA graph and replayed; the optimiser and scheduler steps stay outside.  Same loss as `sr_train_step` with the same
+    arguments: the plain `loss_obj` / `loss_seg` statements, or `fused_loss` (loss_ops.FusedSRLoss) when given.
+
+        step = GraphedSRStep(model, batch0, fused_loss=loss_ops.FusedSRLoss(1, 1, enable_uncertainty=True), enable_uncertainty=True)
+        for batch in loader:                      # (patches_lr, patches_hr), host (pinned) or device tensors of the captured shapes
+            out = step(batch)                     # copies the batch into the static inputs, replays; out["loss"] is static
+            opt.step(); scheduler.step()          # .grad tensors are static, re-attached after every replay
+
+    One difference from `sr_train_step`: the model's forward subtracts the channel-0 mean in place from the STATIC copy of
+    `patches_lr` on every replay; the caller's `patches_lr` is left unchanged.  `dp_group` is passed to `graphs.GraphedTrainStep`
+    (the gradient mean over ranks is then part of the captured step)."""
+
+    def __init__(self, model: nn.Module, example_batch: Sequence[torch.Tensor], loss_obj: Optional[nn.Module] = None,
+                 loss_seg: Optional[nn.Module] = None, slice_separation: int = 4, num_slices: int = 4, enable_uncertainty: bool = False,
+                 fused_loss: Optional[nn.Module] = None, dp_group=None):
+        from .graphs import GraphedTrainStep
+        if fused_loss is None and (loss_obj is None or loss_seg is None):
+            raise ValueError("GraphedSRStep needs either fused_loss or both loss_obj and loss_seg")
+
+        def loss_fn(out, patches_hr):
+            return _sr_loss(out, patches_hr, loss_obj, loss_seg, slice_separation, num_slices, enable_uncertainty, fused_loss)
+
+        self.step = GraphedTrainStep(model, loss_fn, tuple(example_batch), dp_group=dp_group)
+
+    def __call__(self, batch: Sequence[torch.Tensor]) -> dict:
+        self.step.load(*batch)
+        return {"loss": self.step.replay()}
+
+    def close(self) -> None:
+        self.step.close()
