@@ -214,6 +214,11 @@ TCONV_CASES = [
     (2, 320, 320, (4, 4, 4), (2, 2, 2), (2, 2, 2), (0, 0, 0)),
     (1, 64, 32, (4, 8, 8), (1, 2, 2), (1, 2, 2), (0, 0, 0)),
     (1, 128, 64, (4, 8, 8), (3, 4, 4), (1, 2, 2), (1, 1, 1)),   # FLAVR upConv3D (FLAVR_arch.py:49-51)
+    # the three FLAVR up-convs of the C2 step ([8, 2, 4, 256, 256]): decoder.1, .2, .4; the last one's weight gradient is too
+    # big for the side stream
+    (8, 512, 128, (4, 32, 32), (3, 4, 4), (1, 2, 2), (1, 1, 1)),
+    (8, 256, 64, (4, 64, 64), (3, 4, 4), (1, 2, 2), (1, 1, 1)),
+    (8, 128, 64, (4, 128, 128), (3, 4, 4), (1, 2, 2), (1, 1, 1)),
 ]
 
 
