@@ -167,6 +167,17 @@ int rehr_pack_batch_begin(void);
 int rehr_pack_batch_launch(rehr_stream stream);
 int rehr_pack_batch_abort(void);
 
+/* fp16 saturation check (opt-in; csrc/ptx.cuh range_check).  rehr_range_sink(slots, slot) makes every later fp16 activation
+ * store launched ON THIS THREAD by the conv forward (tapped, marching, small-Cin / tensor-core stem, the transposed-conv scatter
+ * and the bias-only class fill), rehr_instnorm_lrelu_apply, rehr_upsample_linear_d and rehr_convert16 count into slots[slot]:
+ * 16 bytes per slot, { uint64 count; uint32 max_abs_bits; uint32 pad }.  A value v saturates when !(|v| < 65520) (it rounds to
+ * +-inf or is NaN; the store still writes +-65504 or NaN, bit-identical to an unchecked run); max_abs_bits is the largest
+ * |v| of the saturated values as fp32 bits (atomicMax: NaN sorts above inf).  bf16 and fp32 stores are not checked.
+ * slots == NULL turns the sink off: the kernels then take a null slot and check nothing.  The pointer is baked into the
+ * launches, so a captured CUDA graph keeps writing to it on replay.  rehr_range_clear zeroes n slots with one memset. */
+int rehr_range_sink(void* slots, int slot);
+int rehr_range_clear(void* slots, int n, rehr_stream stream);
+
 /* Input gradient of a k3 / pad 1 conv with strides in {1, 2} (the nnU-Net stage-entry convs) through the marching kernel:
  * every output parity class of dx is a stride-1 correlation over dy with 1 or 2 taps per strided dimension, written in place
  * at (2i + r).  w = conv weight f32 [Cout][Cin][27]; cin / cout are the CONV's channel counts. */

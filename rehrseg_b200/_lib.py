@@ -95,6 +95,8 @@ def _declare(L: C.CDLL) -> None:
         "rehr_pack_batch_begin": (i, []),
         "rehr_pack_batch_launch": (i, [vp]),
         "rehr_pack_batch_abort": (i, []),
+        "rehr_range_sink": (i, [vp, i]),
+        "rehr_range_clear": (i, [vp, i, vp]),
         "rehr_conv3d_march_s2dgrad": (i, [D, T, vp, T, vp]),
         "rehr_conv3d_wgrad_march_supported": (i, [D, T, T]),
         "rehr_conv3d_wgrad_march_workspace": (sz, [T, T, i]),

@@ -26,7 +26,7 @@ bool conv_shapes_ok(const rehr_conv_desc* d, const rehr_tensor* x, const rehr_te
 // out(class) = act(bias): used for output parity classes no tap reaches.
 __global__ void fill_class_kernel(void* out, int out_f32, int out_f16, long long ld, int cout, const float* bias, int act, float slope,
                                   int O0, int O1, int O2, int N, int s0, int s1, int s2, int o0, int o1, int o2, int A0, int A1,
-                                  int A2) {
+                                  int A2, RangeSlot* range) {
   const long long total = (long long)N * O2 * O1 * O0 * cout;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int c = (int)(i % cout);
@@ -45,10 +45,18 @@ __global__ void fill_class_kernel(void* out, int out_f32, int out_f16, long long
       reinterpret_cast<float*>(out)[vox * ld + c] = v;
     else
       reinterpret_cast<unsigned short*>(out)[vox * ld + c] = pack16(v, out_f16);
+    if (range) range_check<1>(range, &v);
   }
 }
 
+thread_local RangeSlot* g_range_slots = nullptr;
+thread_local int g_range_slot = 0;
+
 }  // namespace
+
+namespace rehr {
+RangeSlot* range_target(int out_f16) { return out_f16 && g_range_slots ? g_range_slots + g_range_slot : nullptr; }
+}  // namespace rehr
 
 extern "C" {
 
@@ -66,6 +74,22 @@ const char* rehr_strerror(int status) {
 int rehr_last_cuda_error(void) { return g_last_cuda_error; }
 int rehr_version(void) { return 6; }
 int rehr_device_sm_count(void) { return sm_count(); }
+
+int rehr_range_sink(void* slots, int slot) {
+  if (slots && slot < 0) return REHR_BAD_SHAPE;
+  g_range_slots = reinterpret_cast<RangeSlot*>(slots);
+  g_range_slot = slots ? slot : 0;
+  return REHR_OK;
+}
+int rehr_range_clear(void* slots, int n, rehr_stream stream) {
+  if (!slots || n <= 0) return REHR_BAD_SHAPE;
+  cudaError_t e = cudaMemsetAsync(slots, 0, sizeof(RangeSlot) * (size_t)n, (cudaStream_t)stream);
+  if (e != cudaSuccess) {
+    g_last_cuda_error = (int)e;
+    return REHR_CUDA_ERROR;
+  }
+  return REHR_OK;
+}
 
 int rehr_pack_weight(const float* src, void* dst16, int R, int C, int T, long long sr, long long sc, long long st, int dtype,
                      rehr_stream stream) {
@@ -183,7 +207,8 @@ static int conv_dgrad_impl(const rehr_conv_desc* desc, const rehr_tensor* dy, co
           const long long total = (long long)O[0] * O[1] * O[2] * O[3] * dx->c;
           const int blocks = (int)std::min<long long>((total + 255) / 256, 148 * 8);
           fill_class_kernel<<<blocks, 256, 0, cstream>>>(dx->ptr, dx_is_f32, dx->dtype == REHR_F16, dx->ld, dx->c, bias, act, slope, O[0], O[1],
-                                                                     O[2], O[3], s[0], s[1], s[2], cw, ch, cd, dx->w, dx->h, dx->d);
+                                                                     O[2], O[3], s[0], s[1], s[2], cw, ch, cd, dx->w, dx->h, dx->d,
+                                                                     range_target(!dx_is_f32 && dx->dtype == REHR_F16));
           REHR_CHECK_LAUNCH();
           continue;
         }

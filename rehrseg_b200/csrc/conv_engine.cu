@@ -311,6 +311,7 @@ struct alignas(64) FwdParams {
   void* out2;
   long long out2_ld;
   int out2_f16;
+  RangeSlot* range;  // fp16 saturation record of the stored values (rehr_range_sink), null = not checked
   long long out_ld;
   int O[4];        // class-local output extents (w h d n)
   int os[3], oo[3];  // actual coord = o*os + oo (w h d)
@@ -340,6 +341,7 @@ __device__ __forceinline__ float apply_act(float v, int act, float slope) {
 }
 
 // bias + InstanceNorm partial sums + activation + store of one 16-column chunk of one accumulator row (non-scatter epilogue)
+template <bool RC>
 __device__ __forceinline__ void finish_chunk(const FwdParams& p, float (&f)[16], bool valid, long long vox, int nbase, int c0,
                                              int lane, float* mypart);
 
@@ -363,6 +365,8 @@ __device__ __forceinline__ void issue_kblock(uint32_t d_tmem, uint32_t a_lo, uin
   }
 }
 
+// RC: the fp16 saturation check of the stored values (p.range != null) is compiled in (see conv_tapped_gemm_kernel)
+template <bool RC>
 __device__ __forceinline__ void finish_chunk(const FwdParams& p, float (&f)[16], bool valid, long long vox, int nbase, int c0,
                                              int lane, float* mypart) {
   if (p.bias != nullptr) {
@@ -411,6 +415,7 @@ __device__ __forceinline__ void finish_chunk(const FwdParams& p, float (&f)[16],
       }
     } else {
       unsigned short* o = reinterpret_cast<unsigned short*>(p.out) + vox * p.out_ld + cbase;
+      if constexpr (RC) range_check<16>(p.range, f, p.cout - cbase);
       if (cbase + 16 <= p.cout && (p.out_ld & 7) == 0) {
         uint4 lo, hi;
         lo.x = pack16x2(f[0], f[1], p.out_f16);
@@ -431,6 +436,8 @@ __device__ __forceinline__ void finish_chunk(const FwdParams& p, float (&f)[16],
   }
 }
 
+// RC: the fp16 saturation check of the stored values is compiled in; the default instantiation has no trace of it.
+template <bool RC>
 __global__ void __launch_bounds__(kFwdThreads, 1) conv_tapped_gemm_kernel(const __grid_constant__ FwdParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // 1024-B alignment of the dynamic window is required by the 128B swizzle atoms.
@@ -620,6 +627,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tapped_gemm_kernel(const 
             }
 #pragma unroll
             for (int i = 0; i < 16; ++i) f[i] = apply_act(f[i], p.act, p.slope);
+            if constexpr (RC) range_check<16>(p.range, f);
             unsigned short* o = reinterpret_cast<unsigned short*>(p.out) + ov * p.out_ld + co0;
             uint4 lo, hi;
             lo.x = pack16x2(f[0], f[1], p.out_f16);
@@ -658,7 +666,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tapped_gemm_kernel(const 
         }
 #pragma unroll
         for (int i = 0; i < 16; ++i) f[i] = __uint_as_float(v[i]);
-        finish_chunk(p, f, valid, vox, nbase, c0, lane, mypart);
+        finish_chunk<RC>(p, f, valid, vox, nbase, c0, lane, mypart);
       }
       // accumulator drained: hand the TMEM stage back to the MMA warp
       tc_fence_before();
@@ -693,6 +701,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tapped_gemm_kernel(const 
 
 // Second stage of split-K: one CTA of 128 threads per (output tile, 16-column chunk); thread = accumulator row; sums the `ksplit`
 // raw partials and runs the same per-chunk epilogue (bias, InstanceNorm partial sums, activation, store) as the fused path.
+template <bool RC>
 __global__ void __launch_bounds__(128) conv_splitk_finish_kernel(const __grid_constant__ FwdParams p) {
   __shared__ float part[4 * 2 * 256];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -736,7 +745,7 @@ __global__ void __launch_bounds__(128) conv_splitk_finish_kernel(const __grid_co
       f[4 * i] += v.x; f[4 * i + 1] += v.y; f[4 * i + 2] += v.z; f[4 * i + 3] += v.w;
     }
   }
-  finish_chunk(p, f, valid, vox, nbase, c0, lane, mypart);
+  finish_chunk<RC>(p, f, valid, vox, nbase, c0, lane, mypart);
   if (p.stats != nullptr) {
     __syncthreads();
     if (threadIdx.x < 16 && nbase + c0 + threadIdx.x < p.cout) {
@@ -808,6 +817,7 @@ int launch_tapped_gemm(const TapPlan& plan, const rehr_tensor& in, const void* w
     p.out2_ld = out2->ld;
     p.out2_f16 = out2->dtype == REHR_F16;
   }
+  p.range = range_target(!out_f32 && (p.out_f16 || (out2 != nullptr && p.out2_f16)));
   p.out_ld = out.ld;
   p.cout = cout;
   p.bias = bias;
@@ -868,7 +878,11 @@ int launch_tapped_gemm(const TapPlan& plan, const rehr_tensor& in, const void* w
   p.stages = stages;
   const size_t smem = 1024 + stages * stage_bytes + fwd_smem_tail_bytes();
 
-  REHR_SET_MAX_SMEM_ONCE(conv_tapped_gemm_kernel, 227 * 1024);
+  const bool rc = p.range != nullptr;
+  if (rc)
+    REHR_SET_MAX_SMEM_ONCE(conv_tapped_gemm_kernel<true>, 227 * 1024);
+  else
+    REHR_SET_MAX_SMEM_ONCE(conv_tapped_gemm_kernel<false>, 227 * 1024);
   const int total_tiles = p.tiles[0] * p.tiles[1] * p.tiles[2] * p.tiles[3] * p.n_tiles;
   // split-K when the output tiles cannot fill the machine and there is a long K loop to share
   const int kblocks = p.num_taps * p.cin_chunks;
@@ -886,14 +900,20 @@ int launch_tapped_gemm(const TapPlan& plan, const rehr_tensor& in, const void* w
   p.ksplit = ksplit;
   p.partial = ksplit > 1 ? reinterpret_cast<float*>(ws) : nullptr;
   const int grid = std::min(total_tiles * ksplit, sm_count());
-  conv_tapped_gemm_kernel<<<grid, kFwdThreads, smem, stream>>>(p);
+  if (rc)
+    conv_tapped_gemm_kernel<true><<<grid, kFwdThreads, smem, stream>>>(p);
+  else
+    conv_tapped_gemm_kernel<false><<<grid, kFwdThreads, smem, stream>>>(p);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
     g_last_cuda_error = (int)e;
     return REHR_CUDA_ERROR;
   }
   if (ksplit > 1) {
-    conv_splitk_finish_kernel<<<dim3(total_tiles, BN / 16), 128, 0, stream>>>(p);
+    if (rc)
+      conv_splitk_finish_kernel<true><<<dim3(total_tiles, BN / 16), 128, 0, stream>>>(p);
+    else
+      conv_splitk_finish_kernel<false><<<dim3(total_tiles, BN / 16), 128, 0, stream>>>(p);
     e = cudaGetLastError();
     if (e != cudaSuccess) {
       g_last_cuda_error = (int)e;

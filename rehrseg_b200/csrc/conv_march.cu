@@ -70,6 +70,7 @@ struct alignas(64) MarchParams {
   int out_f32;
   int out_f16;  // 16-bit output format (rehr_dtype of y) when !out_f32
   int in_f16;   // MMA operand format: of x and of the packed weights (one format per tcgen05.mma)
+  RangeSlot* range;  // fp16 saturation record of the stored values (rehr_range_sink), null = not checked
   long long out_ld;
   const float* bias;
   int act;
@@ -122,7 +123,9 @@ __device__ __forceinline__ bool elect_one_sync() {
 #ifndef REHR_MARCH_MAXNREG
 #define REHR_MARCH_MAXNREG 255
 #endif
-template <int BKT, int CHUNKS, int CT, int KS>
+// RC: the fp16 saturation check of the stored values (p.range != null) is compiled in; the unchecked instantiation is the kernel
+// without it (with a run-time test instead, this register-bound epilogue ran up to a quarter slower with the check off).
+template <int BKT, int CHUNKS, int CT, int KS, bool RC>
 __global__ void __launch_bounds__(kMarchThreads) __maxnreg__(KS > 0 ? REHR_MARCH_MAXNREG : 0) conv_march_kernel(const __grid_constant__ MarchParams p) {
   constexpr int R = MarchGeo<KS>::R;
   constexpr int kHaloW = MarchGeo<KS>::kHaloW;
@@ -382,6 +385,7 @@ __global__ void __launch_bounds__(kMarchThreads) __maxnreg__(KS > 0 ? REHR_MARCH
 #pragma unroll
             for (int i = 0; i < kW; ++i) f[i] = march_act(f[i], p.act, p.slope);
             const int cc = cbase + c0;
+            if constexpr (RC) range_check<kW>(p.range, f, nvalid);
             if (nvalid < kW) {
               if (p.out_f32) {
                 float* o = reinterpret_cast<float*>(p.out) + obase + cc;
@@ -592,6 +596,7 @@ int launch_march(const rehr_tensor& x, const void* w_march, const float* bias, c
   p.out = y.ptr;
   p.out_f32 = y_is_f32;
   p.out_f16 = y.dtype == REHR_F16;
+  p.range = range_target(!y_is_f32 && p.out_f16);
   p.in_f16 = x.dtype == REHR_F16;
   p.out_ld = y.ld;
   p.o_pw = y.ld;
@@ -650,8 +655,13 @@ int launch_march(const rehr_tensor& x, const void* w_march, const float* bias, c
 
 template <int BKT, int CHUNKS, int CT, int KS>
 static int launch_variant(const MarchPlan& pl, cudaStream_t stream) {
-  REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS>), 227 * 1024);
-  conv_march_kernel<BKT, CHUNKS, CT, KS><<<pl.grid, kMarchThreads, pl.smem, stream>>>(pl.p);
+  if (pl.p.range != nullptr) {
+    REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS, true>), 227 * 1024);
+    conv_march_kernel<BKT, CHUNKS, CT, KS, true><<<pl.grid, kMarchThreads, pl.smem, stream>>>(pl.p);
+  } else {
+    REHR_SET_MAX_SMEM_ONCE((conv_march_kernel<BKT, CHUNKS, CT, KS, false>), 227 * 1024);
+    conv_march_kernel<BKT, CHUNKS, CT, KS, false><<<pl.grid, kMarchThreads, pl.smem, stream>>>(pl.p);
+  }
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }

@@ -317,10 +317,12 @@ struct ApplyArgs {
   __nv_bfloat16* out2;   // MODE 0 only: optional second copy of the activation in the other 16-bit format (may be null)
   long long ld_o2;
   int out2_f16;
+  RangeSlot* range;      // MODE 0 only: fp16 saturation record of out (rehr_range_sink), null = not checked
 };
 
 // MODE 0: a = lrelu(gamma*xhat + beta).  MODE 1: dy = gamma*rstd*(g - S1/V - xhat*S2/V).
-template <int MODE>
+// RC (MODE 0): the fp16 saturation check of a (a.range != null) is compiled in; the unchecked instantiation has no trace of it.
+template <int MODE, bool RC = false>
 __global__ void __launch_bounds__(256, MODE == 1 ? 4 : 1) in_apply_kernel(const ApplyArgs a) {
   extern __shared__ float sh[];  // MODE0: scale, shift ; MODE1: mean, rstd, gamma, beta, m1, m2
   const int n = blockIdx.y;
@@ -392,6 +394,7 @@ __global__ void __launch_bounds__(256, MODE == 1 ? 4 : 1) in_apply_kernel(const 
           o[i] = sh[2 * C + c] * sh[C + c] * (gi - sh[4 * C + c] - xh * sh[5 * C + c]);
         }
       }
+      if constexpr (RC) range_check<8>(a.range, o);
       *reinterpret_cast<uint4*>(a.out + vox * a.ld_o + g * 8) = float_to_x16x8(o, a.out_f16);
       if (MODE == 0 && a.out2 != nullptr) *reinterpret_cast<uint4*>(a.out2 + vox * a.ld_o2 + g * 8) = float_to_x16x8(o, a.out2_f16);
     }
@@ -405,7 +408,14 @@ static int launch_in_apply(const ApplyArgs& a, int N, cudaStream_t st) {
   int gx = grid_for(items, 256, 8);
   gx = std::max(1, gx / std::max(1, N));
   dim3 grid(gx, N);
-  in_apply_kernel<MODE><<<grid, 256, smem, st>>>(a);
+  bool checked = false;
+  if constexpr (MODE == 0) {
+    if (a.range != nullptr) {
+      in_apply_kernel<0, true><<<grid, 256, smem, st>>>(a);
+      checked = true;
+    }
+  }
+  if (!checked) in_apply_kernel<MODE, false><<<grid, 256, smem, st>>>(a);
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }
@@ -635,7 +645,7 @@ static int channel_sum_blocks(const rehr_tensor* x) {
 // =================================================================================================
 __global__ void __launch_bounds__(256) upsample_d_kernel(const __nv_bfloat16* x, long long ldx, __nv_bfloat16* y,
                                                          long long ldy, int N, int D, int OD, long long HW, int C, int x_f16,
-                                                         int y_f16) {
+                                                         int y_f16, RangeSlot* range) {
   const int groups = C / 8;
   const long long items = (long long)N * OD * HW * groups;
   const float scale = OD > 1 ? (float)(D - 1) / (float)(OD - 1) : 0.f;
@@ -655,6 +665,7 @@ __global__ void __launch_bounds__(256) upsample_d_kernel(const __nv_bfloat16* x,
     x16x8_to_float(*reinterpret_cast<const uint4*>(x + ((n * D + i1) * HW + hw) * ldx + g * 8), b, x_f16);
 #pragma unroll
     for (int i = 0; i < 8; ++i) o[i] = l0 * a[i] + l1 * b[i];
+    if (range != nullptr) range_check<8>(range, o);
     *reinterpret_cast<uint4*>(y + ((n * OD + od) * HW + hw) * ldy + g * 8) = float_to_x16x8(o, y_f16);
   }
 }
@@ -663,7 +674,8 @@ __global__ void __launch_bounds__(256) upsample_d_kernel(const __nv_bfloat16* x,
 // from DRAM ~3.4 times at the C4 shape (profiles/r02_ncu_families_raw.txt: 450 MB read for a 134 MB input).  Indices and weights come
 // from the same float expressions, evaluated per output plane, so the results are bit-identical.
 __global__ void __launch_bounds__(256) upsample_d_src_kernel(const __nv_bfloat16* x, long long ldx, __nv_bfloat16* y, long long ldy,
-                                                             int N, int D, int OD, long long HW, int C, int x_f16, int y_f16) {
+                                                             int N, int D, int OD, long long HW, int C, int x_f16, int y_f16,
+                                                             RangeSlot* range) {
   const int groups = C / 8;
   const long long items = (long long)N * D * HW * groups;
   const float scale = OD > 1 ? (float)(D - 1) / (float)(OD - 1) : 0.f;
@@ -695,6 +707,7 @@ __global__ void __launch_bounds__(256) upsample_d_src_kernel(const __nv_bfloat16
       const float l1 = src - (float)i0, l0 = 1.f - l1;
 #pragma unroll
       for (int i = 0; i < 8; ++i) o[i] = l0 * a[i] + l1 * b[i];
+      if (range != nullptr) range_check<8>(range, o);
       *reinterpret_cast<uint4*>(y + ((n * OD + od) * HW + hw) * ldy + g * 8) = float_to_x16x8(o, y_f16);
     }
   }
@@ -784,7 +797,7 @@ __global__ void __launch_bounds__(256) ndhwc_to_ncdhw_kernel(const unsigned shor
 // 16-bit -> 16-bit format conversion of a (pitched) channels-last tensor: the bf16 twin of an fp16 forward activation that a
 // weight-gradient GEMM needs as its operand (its other operand, the gradient, is bf16 and one MMA takes one format)
 __global__ void __launch_bounds__(256) convert16_kernel(const __nv_bfloat16* x, long long ldx, int x_f16, __nv_bfloat16* y,
-                                                        long long ldy, int y_f16, long long vox_total, int C) {
+                                                        long long ldy, int y_f16, long long vox_total, int C, RangeSlot* range) {
   const int groups = C / 8;
   const long long items = vox_total * groups;
   for (long long it = blockIdx.x * (long long)blockDim.x + threadIdx.x; it < items; it += (long long)gridDim.x * blockDim.x) {
@@ -792,6 +805,7 @@ __global__ void __launch_bounds__(256) convert16_kernel(const __nv_bfloat16* x, 
     const long long vox = it / groups;
     float f[8];
     x16x8_to_float(__ldcs(reinterpret_cast<const uint4*>(x + vox * ldx + g * 8)), f, x_f16);
+    if (range != nullptr) range_check<8>(range, f);
     *reinterpret_cast<uint4*>(y + vox * ldy + g * 8) = float_to_x16x8(f, y_f16);
   }
 }
@@ -1602,6 +1616,7 @@ int rehr_instnorm_lrelu_apply(const rehr_tensor* y, const float* mean, const flo
   p.out = reinterpret_cast<__nv_bfloat16*>(a->ptr);
   p.y_f16 = y->dtype == REHR_F16;
   p.out_f16 = a->dtype == REHR_F16;
+  p.range = range_target(p.out_f16 || (a2 && a2->dtype == REHR_F16));
   if (a2) {
     p.out2 = reinterpret_cast<__nv_bfloat16*>(a2->ptr);
     p.ld_o2 = a2->ld;
@@ -1757,14 +1772,15 @@ int rehr_upsample_linear_d(const rehr_tensor* x, const rehr_tensor* y, rehr_stre
     const long long items = (long long)x->n * x->d * HW * (x->c / 8);
     upsample_d_src_kernel<<<grid_for(items, 256, 8), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const __nv_bfloat16*>(x->ptr), x->ld, reinterpret_cast<__nv_bfloat16*>(y->ptr), y->ld, x->n, x->d, y->d, HW, x->c,
-        x->dtype == REHR_F16, y->dtype == REHR_F16);
+        x->dtype == REHR_F16, y->dtype == REHR_F16, range_target(y->dtype == REHR_F16));
     REHR_CHECK_LAUNCH();
     return REHR_OK;
   }
   const long long items = (long long)y->n * y->d * HW * (y->c / 8);
   upsample_d_kernel<<<grid_for(items, 256, 8), 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const __nv_bfloat16*>(x->ptr), x->ld,
                                                                            reinterpret_cast<__nv_bfloat16*>(y->ptr), y->ld, x->n, x->d,
-                                                                           y->d, HW, x->c, x->dtype == REHR_F16, y->dtype == REHR_F16);
+                                                                           y->d, HW, x->c, x->dtype == REHR_F16, y->dtype == REHR_F16,
+                                                                           range_target(y->dtype == REHR_F16));
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }
@@ -1804,7 +1820,7 @@ int rehr_convert16(const rehr_tensor* src, const rehr_tensor* dst, rehr_stream s
   const long long vox = (long long)src->n * voxels_per_sample(src);
   convert16_kernel<<<grid_for(vox * (src->c / 8), 256, 8), 256, 0, (cudaStream_t)stream>>>(
       reinterpret_cast<const __nv_bfloat16*>(src->ptr), src->ld, src->dtype == REHR_F16, reinterpret_cast<__nv_bfloat16*>(dst->ptr), dst->ld,
-      dst->dtype == REHR_F16, vox, src->c);
+      dst->dtype == REHR_F16, vox, src->c, range_target(dst->dtype == REHR_F16));
   REHR_CHECK_LAUNCH();
   return REHR_OK;
 }

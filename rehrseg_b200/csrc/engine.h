@@ -64,6 +64,11 @@ struct PackJob {
 bool pack_recording();          // this thread is between rehr_pack_batch_begin and rehr_pack_batch_launch
 int pack_record(PackJob job);   // append (fills total / runs / nblocks)
 
+// fp16 saturation sink (rehr_range_sink, ptx.cuh range_check): the slot a launch wrapper hands its kernel, or null when this
+// thread has no sink set or the store the wrapper launches is not fp16 -- a null slot means the kernel checks nothing.
+struct RangeSlot;
+RangeSlot* range_target(int out_f16);
+
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is a PER-DEVICE setting: a process that drives several GPUs must apply it on
 // each of them, so the "already done" flag lives per device (index = cudaGetDevice()).
 static constexpr int kMaxDevices = 64;

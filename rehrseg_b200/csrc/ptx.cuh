@@ -185,6 +185,54 @@ __device__ __forceinline__ float2 unpack16x2(uint32_t u, int fp16) {
 }
 __device__ __forceinline__ float unpack16(unsigned short u, int fp16) { return unpack16x2((uint32_t)u, fp16).x; }
 
+// One slot of the saturation record (layout shared with rehrseg_b200/rangecheck.py: 16 bytes, count then max bits).
+struct RangeSlot {
+  unsigned long long count;
+  unsigned int max_bits;
+  unsigned int pad;
+};
+
+// fp16 saturation record (rehr_range_sink): a value saturates when it is at least the smallest magnitude round-to-nearest
+// would take to inf, or NaN -- on the bits of |v|: >= those of 65520.f (NaN sorts above inf).  The check only observes; the
+// stores are unchanged.  Per warp, one ballot on the largest |v| of each lane decides; only when some lane saw a saturated value
+// are the values counted and ONE atomic pair per warp issued (lane counts added, largest |v| bits as atomicMax).
+static constexpr uint32_t kRangeSatBits = 0x477FF000u;  // __float_as_uint(65520.f)
+__device__ __forceinline__ uint32_t range_abs_bits(float v) { return __float_as_uint(v) & 0x7FFFFFFFu; }
+__device__ __forceinline__ void range_fold(float v, uint32_t& cnt, uint32_t& mbits) {
+  const uint32_t b = range_abs_bits(v);
+  if (b >= kRangeSatBits) {
+    ++cnt;
+    mbits = max(mbits, b);
+  }
+}
+__device__ __forceinline__ void range_flush(RangeSlot* s, uint32_t cnt, uint32_t mbits) {
+  const uint32_t mask = __activemask();
+  if (__ballot_sync(mask, cnt != 0u) == 0u) return;
+  const uint32_t total = __reduce_add_sync(mask, cnt);
+  const uint32_t m = __reduce_max_sync(mask, mbits);
+  uint32_t lane;
+  asm("mov.u32 %0, %%laneid;" : "=r"(lane));
+  if (lane == (uint32_t)(__ffs(mask) - 1)) {
+    atomicAdd(&s->count, (unsigned long long)total);
+    atomicMax(&s->max_bits, m);
+  }
+}
+// the first `n` of K values about to be stored (fast path: one max per value and a ballot)
+template <int K>
+__device__ __forceinline__ void range_check(RangeSlot* s, const float* f, int n = K) {
+  uint32_t m = 0;
+#pragma unroll
+  for (int i = 0; i < K; ++i)
+    if (i < n) m = max(m, range_abs_bits(f[i]));
+  const uint32_t mask = __activemask();
+  if (__ballot_sync(mask, m >= kRangeSatBits) == 0u) return;
+  uint32_t cnt = 0, mbits = 0;
+#pragma unroll
+  for (int i = 0; i < K; ++i)
+    if (i < n) range_fold(f[i], cnt, mbits);
+  range_flush(s, cnt, mbits);
+}
+
 }  // namespace rehr
 
 namespace rehr {

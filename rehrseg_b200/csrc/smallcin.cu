@@ -37,6 +37,7 @@ struct SmallCinArgs {
   int act;
   float slope;
   int y_f16;           // storage format of y (rehr_dtype)
+  RangeSlot* range;    // fp16 saturation record of y (rehr_range_sink), null = not checked
 };
 
 // weights in smem as [cin*T][cout] (cout fastest) so that a thread's 16 channels are 4 float4 broadcasts.
@@ -108,6 +109,7 @@ __global__ void __launch_bounds__(256) smallcin_fwd_kernel(const SmallCinArgs a)
         if (a.act == REHR_ACT_LRELU) z = z > 0.f ? z : z * a.slope;
         f[i] = z;
       }
+      if (a.range != nullptr) range_check<kScCoutPerThread>(a.range, f);
       uint32_t* l2 = reinterpret_cast<uint32_t*>(&lo);
       uint32_t* h2 = reinterpret_cast<uint32_t*>(&hi);
 #pragma unroll
@@ -124,7 +126,9 @@ __global__ void __launch_bounds__(256) smallcin_fwd_kernel(const SmallCinArgs a)
           if (a.act == REHR_ACT_RELU) z = z > 0.f ? z : 0.f;
           if (a.act == REHR_ACT_LRELU) z = z > 0.f ? z : z * a.slope;
           reinterpret_cast<unsigned short*>(o)[i] = pack16(z, a.y_f16);
+          acc[i] = z;
         }
+      if (a.range != nullptr) range_check<kScCoutPerThread>(a.range, acc, a.cout - c0);
     }
   }
 }
@@ -202,6 +206,7 @@ __global__ void __launch_bounds__(256) smallcin_fwd_k3c32_kernel(const SmallCinA
           }
       const long long v = (((long long)nn * a.od + oz) * a.oh + oy) * a.ow + ox;
       uint4* o = reinterpret_cast<uint4*>(a.y + v * a.ldy);
+      uint32_t cnt = 0, mbits = 0;
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         uint4 u;
@@ -212,9 +217,11 @@ __global__ void __launch_bounds__(256) smallcin_fwd_k3c32_kernel(const SmallCinA
           if (a.act == REHR_ACT_RELU) { z0 = z0 > 0.f ? z0 : 0.f; z1 = z1 > 0.f ? z1 : 0.f; }
           if (a.act == REHR_ACT_LRELU) { z0 = z0 > 0.f ? z0 : z0 * a.slope; z1 = z1 > 0.f ? z1 : z1 * a.slope; }
           h2[i] = pack16x2(z0, z1, a.y_f16);
+          if (a.range != nullptr) { range_fold(z0, cnt, mbits); range_fold(z1, cnt, mbits); }
         }
         o[j] = u;
       }
+      if (a.range != nullptr) range_flush(a.range, cnt, mbits);
     }
   }
 }
@@ -600,6 +607,7 @@ int rehr_conv3d_smallcin_fwd(const rehr_conv_desc* desc, const float* x_ncdhw, i
   a.act = act;
   a.slope = slope;
   a.y_f16 = y->dtype == REHR_F16;
+  a.range = range_target(a.y_f16);
   const bool k3 = desc->kd == 3 && desc->kh == 3 && desc->kw == 3 && desc->sd == 1 && desc->sh == 1 && desc->sw == 1 &&
                   desc->pd == 1 && desc->ph == 1 && desc->pw == 1;
   // planar stem of anisotropic plans: k = (1,3,3), stride 1, pad (0,1,1)

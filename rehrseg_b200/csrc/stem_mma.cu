@@ -33,6 +33,7 @@ struct StemArgs {
   float slope;
   int planar;           // 1: k = (1,3,3), pad (0,1,1) (the stem of anisotropic plans): 9 taps, one staged plane
   int y_f16;            // forward: storage format of y (rehr_dtype); the weight gradient's dY is always bf16
+  RangeSlot* range;     // forward: fp16 saturation record of y (rehr_range_sink), null = not checked
 };
 
 __device__ __forceinline__ void mma_bf16_16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
@@ -171,6 +172,15 @@ __global__ void __launch_bounds__(256, 3) stem_fwd_mma_kernel(const StemArgs a) 
         }
         *reinterpret_cast<uint32_t*>(mine + g * kStemRowPad + (nt * 8 + 2 * t) * 2) = pack16x2(acc[nt][0], acc[nt][1], a.y_f16);
         *reinterpret_cast<uint32_t*>(mine + (g + 8) * kStemRowPad + (nt * 8 + 2 * t) * 2) = pack16x2(acc[nt][2], acc[nt][3], a.y_f16);
+      }
+      if (a.range != nullptr) {  // the voxels x0 + g and x0 + g + 8 that are stored below
+        uint32_t cnt = 0, mbits = 0;
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) {
+          if (x0 + g < a.wd) { range_fold(acc[nt][0], cnt, mbits); range_fold(acc[nt][1], cnt, mbits); }
+          if (x0 + g + 8 < a.wd) { range_fold(acc[nt][2], cnt, mbits); range_fold(acc[nt][3], cnt, mbits); }
+        }
+        range_flush(a.range, cnt, mbits);
       }
       __syncwarp();
 #pragma unroll
@@ -357,6 +367,7 @@ int launch_stem_fwd_mma(const float* x, const float* w, const float* bias, __nv_
   StemArgs a;
   a.planar = planar;
   a.y_f16 = y_f16;
+  a.range = range_target(y_f16);
   a.x = x; a.w = w; a.bias = bias; a.y = y; a.ldy = ldy; a.ws = nullptr;
   a.n = n; a.d = d; a.h = h; a.wd = wd; a.act = act; a.slope = slope;
   const size_t smem = stem_smem_bytes(wd, false);
@@ -376,6 +387,7 @@ int launch_stem_wgrad_mma(const float* x, const __nv_bfloat16* dy, long long ldd
   StemArgs a;
   a.planar = planar;
   a.y_f16 = 0;
+  a.range = nullptr;
   a.x = x; a.w = nullptr; a.bias = nullptr; a.y = const_cast<__nv_bfloat16*>(dy); a.ldy = lddy; a.ws = ws;
   a.n = n; a.d = d; a.h = h; a.wd = wd; a.act = 0; a.slope = 0.f;
   const size_t smem = stem_smem_bytes(wd, true);

@@ -92,6 +92,48 @@ class _timed:
 
 
 # --------------------------------------------------------------------------------------------------
+# opt-in fp16 saturation check (rangecheck.RangeCheck): the active check, or None.  `_sink(kind)` wraps one fp16-producing
+# launch of the SegModel forward; with no check active it does nothing and the kernels get a null slot.
+# --------------------------------------------------------------------------------------------------
+_range = None
+
+
+class _sink:
+    __slots__ = ("kind",)
+
+    def __init__(self, kind: str):
+        self.kind = kind
+
+    def __enter__(self):
+        if _range is not None:
+            _range.arm(self.kind)
+        return self
+
+    def __exit__(self, *exc):
+        if _range is not None:
+            _range.disarm()
+        return False
+
+
+class range_owner:
+    """Labels the fp16 stores issued inside the block with `module` (seg_model's conv blocks, transposed convs, sr_head)."""
+    __slots__ = ("module", "prev")
+
+    def __init__(self, module):
+        self.module = module
+
+    def __enter__(self):
+        if _range is not None:
+            self.prev, _range.owner = _range.owner, self.module
+        return self
+
+    def __exit__(self, *exc):
+        if _range is not None:
+            _range.owner = self.prev
+        return False
+
+
+# --------------------------------------------------------------------------------------------------
 # 16-bit storage formats
 # --------------------------------------------------------------------------------------------------
 # Gradients (and every FLAVR activation) are bf16.  The forward activations of the InstanceNorm'ed SegModel path are stored in
@@ -776,14 +818,16 @@ class ConvNormAct(torch.autograd.Function):
             stats = torch.empty((n, tiles, cout, 2), dtype=torch.float32, device=dev)
             # NB the conv bias is NOT added: a per-channel constant is removed exactly by the InstanceNorm that follows
             # (mean shifts by the same constant, variance is unchanged), so lrelu(IN(conv+b)) == lrelu(IN(conv)).
-            check(lib().rehr_conv3d_smallcin_fwd(C.byref(desc), ptr(xs), n, cin, d, h, w, ptr(_f32(weight)), None,
-                                                 C.byref(yt), ACT_NONE, 0.0, ptr(stats), stream_ptr()), "smallcin_fwd")
+            with _sink("y"):
+                check(lib().rehr_conv3d_smallcin_fwd(C.byref(desc), ptr(xs), n, cin, d, h, w, ptr(_f32(weight)), None,
+                                                     C.byref(yt), ACT_NONE, 0.0, ptr(stats), stream_ptr()), "smallcin_fwd")
             _count(2)
             x_saved = xs
         else:
             xc = as_cl(x)
             x_saved = bf_twin(x) if train else None   # bf16 operand of this layer's weight gradient
-            y, stats, tiles = conv3d_raw(xc, weight, None, kernel, stride, padding, want_stats=True, x_h=is_h(x), y_h=True)
+            with _sink("y"):
+                y, stats, tiles = conv3d_raw(xc, weight, None, kernel, stride, padding, want_stats=True, x_h=is_h(x), y_h=True)
         n = y.shape[0]
         vox = y.shape[1] * y.shape[2] * y.shape[3]
         mean = torch.empty((n, cout), dtype=torch.float32, device=dev)
@@ -799,8 +843,9 @@ class ConvNormAct(torch.autograd.Function):
         a2 = alloc(y.shape) if want_twin else None
         yt, at = rt(y, True), rt(a, a_h)
         a2t = rt(a2, False) if a2 is not None else None
-        check(lib().rehr_instnorm_lrelu_apply(C.byref(yt), ptr(mean), ptr(rstd), ptr(g32), ptr(b32), float(slope), C.byref(at),
-                                              C.byref(a2t) if a2t is not None else None, stream_ptr()), "instnorm_lrelu_apply")
+        with _sink("a"):
+            check(lib().rehr_instnorm_lrelu_apply(C.byref(yt), ptr(mean), ptr(rstd), ptr(g32), ptr(b32), float(slope), C.byref(at),
+                                                  C.byref(a2t) if a2t is not None else None, stream_ptr()), "instnorm_lrelu_apply")
         _count(2)
         ctx.save_for_backward(x_saved, weight, gamma, beta, y, mean, rstd)
         ctx.skip_key = (a.untyped_storage().data_ptr(), a.storage_offset()) if cat_room else None
@@ -1099,26 +1144,27 @@ class ConvTranspose(torch.autograd.Function):
             y = torch.empty((n, od, oh, ow, cout), dtype=torch.bfloat16, device=x.device)
         xt, yt = rt(x, x_h), rt(y, x_h)
         twin_done = False
-        if lib().rehr_convtranspose3d_fused_supported(C.byref(desc), cin, cout):
-            wp = _packed(weight, "tconv_fused", h=x_h)  # [T][Cout][Cin]
-            tw = getattr(skip, "_rehr_bf", None) if (skip is not None and x_h and train) else None
-            if tw is not None and getattr(tw, "_rehr_cat", None) == skip._rehr_cat:
-                # the bf16 twin of the up-sampled half goes straight into the twin's [up | skip] buffer from the same epilogue
-                full2 = whole(tw)
-                y2t = rt(full2[..., :cout], False)
-                check(lib().rehr_convtranspose3d_fused_fwd2(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt),
-                                                            C.byref(y2t), act, float(slope), stream_ptr()), "convtranspose3d_fused_fwd2")
-                twin_done = True
-                path_hits["tconv_twin_from_epilogue"] += 1
+        with _sink("up"):
+            if lib().rehr_convtranspose3d_fused_supported(C.byref(desc), cin, cout):
+                wp = _packed(weight, "tconv_fused", h=x_h)  # [T][Cout][Cin]
+                tw = getattr(skip, "_rehr_bf", None) if (skip is not None and x_h and train) else None
+                if tw is not None and getattr(tw, "_rehr_cat", None) == skip._rehr_cat:
+                    # the bf16 twin of the up-sampled half goes straight into the twin's [up | skip] buffer from the same epilogue
+                    full2 = whole(tw)
+                    y2t = rt(full2[..., :cout], False)
+                    check(lib().rehr_convtranspose3d_fused_fwd2(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt),
+                                                                C.byref(y2t), act, float(slope), stream_ptr()), "convtranspose3d_fused_fwd2")
+                    twin_done = True
+                    path_hits["tconv_twin_from_epilogue"] += 1
+                else:
+                    check(lib().rehr_convtranspose3d_fused_fwd(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt), act,
+                                                               float(slope), stream_ptr()), "convtranspose3d_fused_fwd")
+                _count()
             else:
-                check(lib().rehr_convtranspose3d_fused_fwd(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt), act,
-                                                           float(slope), stream_ptr()), "convtranspose3d_fused_fwd")
-            _count()
-        else:
-            wp = _packed(weight, "dgrad", h=x_h)  # [Cout][T][Cin]
-            check(lib().rehr_convtranspose3d_fwd(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt), act,
-                                                 float(slope), stream_ptr()), "convtranspose3d_fwd")
-            _count(stride[0] * stride[1] * stride[2])
+                wp = _packed(weight, "dgrad", h=x_h)  # [Cout][T][Cin]
+                check(lib().rehr_convtranspose3d_fwd(C.byref(desc), C.byref(xt), ptr(wp), ptr(_f32(bias)), C.byref(yt), act,
+                                                     float(slope), stream_ptr()), "convtranspose3d_fwd")
+                _count(stride[0] * stride[1] * stride[2])
         if x_h and train and not twin_done:
             # bf16 twin of the result for the weight-gradient GEMM of the consumer: the skip half already has one (written by
             # the skip's normalise pass), the up-sampled half is converted here
@@ -1264,7 +1310,8 @@ class UpsampleD(torch.autograd.Function):
         n, d, h, w, c = x.shape
         y = torch.empty((n, out_d, h, w, c), dtype=torch.bfloat16, device=x.device)   # bf16: the sr_head has no InstanceNorm
         xt, yt = rt(x, x_h), rt(y)
-        check(lib().rehr_upsample_linear_d(C.byref(xt), C.byref(yt), stream_ptr()), "upsample_linear_d")
+        with _sink("sr_up"):
+            check(lib().rehr_upsample_linear_d(C.byref(xt), C.byref(yt), stream_ptr()), "upsample_linear_d")
         _count()
         ctx.in_shape = tuple(x.shape)
         return y

@@ -16,9 +16,13 @@ _graph_cache: "weakref.WeakKeyDictionary" = weakref.WeakKeyDictionary()  # modul
 
 class GraphedForward:
     """`g = GraphedForward(module, example)`; `g(x)` copies x into the static input, replays the captured forward and
-    returns the STATIC output tensors (valid until the next call -- consume or copy them first)."""
+    returns the STATIC output tensors (valid until the next call -- consume or copy them first).
 
-    def __init__(self, module, example: torch.Tensor, warmup: int = 2):
+    `range_check=True` captures the forward inside a `rangecheck.RangeCheck(module)`: the graph starts with a memset that zeroes
+    its slots, so after each replay `g.range_report()` lists the fp16 saturation of that replay alone (no host synchronisation
+    until the report is asked for)."""
+
+    def __init__(self, module, example: torch.Tensor, warmup: int = 2, range_check: bool = False):
         if not example.is_cuda:
             raise ValueError("GraphedForward needs a CUDA example input")
         from . import functional as Fn
@@ -31,8 +35,17 @@ class GraphedForward:
         torch.cuda.current_stream(example.device).wait_stream(side)
         torch.cuda.synchronize(example.device)
         self.graph = torch.cuda.CUDAGraph()
+        self.range = None
+        if range_check:
+            from .rangecheck import RangeCheck
+            self.range = RangeCheck(module, device=example.device)
         with torch.no_grad(), torch.cuda.graph(self.graph):
-            self.static_out = module(self.static_in)
+            if self.range is None:
+                self.static_out = module(self.static_in)
+            else:
+                self.range.reset()
+                with self.range:
+                    self.static_out = module(self.static_in)
         # The captured kernels bake in the addresses of the packed 16-bit weight copies made during the warm-up.  Their only
         # other owner is functional's weight cache, which anyone may clear (GraphedTrainStep, bench.py): hold them here so a
         # replay can never read freed memory.  (The module itself is NOT kept: graphed() keys its cache on it weakly.)
@@ -45,13 +58,19 @@ class GraphedForward:
         self.graph.replay()
         return self.static_out
 
+    def range_report(self):
+        """fp16 saturation records of the last replay (rangecheck.RangeCheck.report); needs range_check=True."""
+        if self.range is None:
+            raise ValueError("GraphedForward was captured without range_check=True")
+        return self.range.report()
 
-def graphed(module, example: torch.Tensor) -> GraphedForward:
+
+def graphed(module, example: torch.Tensor, range_check: bool = False) -> GraphedForward:
     """Cached GraphedForward for (module, input shape).  The capture bakes in the packed bf16 copies of the weights, so it is
     reused only while every parameter still has the version and storage it had at capture time (an optimiser step or a
     load_state_dict invalidates it)."""
     params = list(module.parameters())
-    shape_key = (tuple(example.shape), example.dtype)
+    shape_key = (tuple(example.shape), example.dtype) + (("range_check",) if range_check else ())
     sig = (tuple(p._version for p in params), tuple(p.data_ptr() for p in params))
     per_module = _graph_cache.get(module)
     if per_module is None:
@@ -61,7 +80,7 @@ def graphed(module, example: torch.Tensor) -> GraphedForward:
         return hit[1]
     for k in [k for k, v in per_module.items() if v[0] != sig]:
         del per_module[k]                         # captures of older weights (any shape) are dead: release their memory
-    g = GraphedForward(module, example)
+    g = GraphedForward(module, example, range_check=range_check)
     per_module[shape_key] = (sig, g)              # one capture per input shape (single tiles, pairs of mirror variants, ...)
     return g
 
@@ -88,9 +107,13 @@ class GraphedTrainStep:
     gradients become final, and as soon as the last gradient of a bucket has been written the bucket is all-reduced (AVG, one
     coalesced NCCL launch over the gradients themselves: no gather / scatter copies) on a communication stream that the compute
     stream joins after the backward pass.  Every rank issues the same collectives in the same (autograd) order.
+
+    `range_check=True`: the step is captured inside a `rangecheck.RangeCheck(model)` whose slots a memset at the start of the
+    graph zeroes; `step.range_report()` then lists the fp16 saturation of the last replay's forward pass.
     """
 
-    def __init__(self, model, loss_fn, example_inputs, warmup: int = 2, before_step=None, dp_group=None, dp_buckets: int = 6):
+    def __init__(self, model, loss_fn, example_inputs, warmup: int = 2, before_step=None, dp_group=None, dp_buckets: int = 6,
+                 range_check: bool = False):
         self.model, self.loss_fn, self.before_step = model, loss_fn, before_step
         self._dp = None
         if dp_group is not None and dp_group is not False:
@@ -120,9 +143,18 @@ class GraphedTrainStep:
         # thread_local: the NCCL watchdog thread of torch.distributed polls events while this thread captures
         from . import functional as Fn
         cap = torch.cuda.Stream(device=dev, priority=Fn.SIDE_PRIORITY)
+        self.range = None
+        if range_check:
+            from .rangecheck import RangeCheck
+            self.range = RangeCheck(model, device=dev)
         l0 = Fn.launches()
         with torch.cuda.graph(self.graph, stream=cap, capture_error_mode="thread_local" if self._dp is not None else "global"):
-            self.loss = self._eager()
+            if self.range is None:
+                self.loss = self._eager()
+            else:
+                self.range.reset()
+                with self.range:
+                    self.loss = self._eager()
         self.engine_launches = Fn.launches() - l0      # engine kernels one replay issues (ATen / NCCL nodes not counted)
         self.grads = [p.grad for p in self.params]     # static gradient tensors (None for parameters the loss does not reach)
         # the captured pack kernels write the cached 16-bit weight copies in place: keep them alive with the graph
@@ -238,6 +270,12 @@ class GraphedTrainStep:
         for dst, src in zip(self.static_inputs, inputs):
             if src is not dst:
                 dst.copy_(src, non_blocking=non_blocking)
+
+    def range_report(self):
+        """fp16 saturation records of the last replay (rangecheck.RangeCheck.report); needs range_check=True."""
+        if self.range is None:
+            raise ValueError("GraphedTrainStep was captured without range_check=True")
+        return self.range.report()
 
     def replay(self):
         self.graph.replay()

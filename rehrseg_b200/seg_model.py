@@ -74,8 +74,9 @@ def run_conv_block(block: nn.Module, x: torch.Tensor, first: bool = False, cat_r
             raise RehrError("only InstanceNorm (no running stats) is implemented (train_all.py:485-486)")
         if act == ACT_RELU:
             slope = 0.0
-        return F_.conv_norm_act(x, conv.weight, conv.bias, norm.weight, norm.bias, k, s, p, eps=norm.eps, slope=slope,
-                                small_cin=small, cat_room=cat_room)
+        with F_.range_owner(block):
+            return F_.conv_norm_act(x, conv.weight, conv.bias, norm.weight, norm.bias, k, s, p, eps=norm.eps, slope=slope,
+                                    small_cin=small, cat_room=cat_room)
     if small:
         raise RehrError("small-Cin stem without InstanceNorm: use rehrseg_b200.flavr for the FLAVR stem")
     return F_.conv_act(x, conv.weight, conv.bias, k, s, p, act=act, slope=slope)
@@ -114,12 +115,15 @@ def run_transpconv(tc: nn.ConvTranspose3d, x: torch.Tensor, skip: torch.Tensor =
         raise RehrError("output_padding is not implemented")
     k, s, p = _triple(tc.kernel_size), _triple(tc.stride), _triple(tc.padding)
     if skip is None:
-        return F_.conv_transpose(x, tc.weight, tc.bias, k, s, p)
+        with F_.range_owner(tc):
+            return F_.conv_transpose(x, tc.weight, tc.bias, k, s, p)
     room = F_.concat_room_of(skip)
     if room is not None and room == (2 * tc.out_channels, tc.out_channels):
-        return F_.conv_transpose(x, tc.weight, tc.bias, k, s, p, skip=skip)
+        with F_.range_owner(tc):
+            return F_.conv_transpose(x, tc.weight, tc.bias, k, s, p, skip=skip)
     # no concat room (a caller-built skip): plain copy; fp16 payloads concatenate bit-wise, their bf16 twins likewise
-    up = F_.conv_transpose(x, tc.weight, tc.bias, k, s, p)
+    with F_.range_owner(tc):
+        up = F_.conv_transpose(x, tc.weight, tc.bias, k, s, p)
     if F_.is_h(up) != F_.is_h(skip):
         raise RehrError("run_transpconv: up-sampled tensor and skip use different 16-bit storage formats")
     cat = torch.cat((up, skip), dim=4)
@@ -161,7 +165,8 @@ def _seg_layer(layer: nn.Module, x: torch.Tensor) -> torch.Tensor:
 
 def sr_head_forward(sr_head: nn.Sequential, features: torch.Tensor, upscale: int) -> torch.Tensor:
     """F.interpolate(features, (upscale,1,1), trilinear, align_corners=True) -> sr_head (models/seg_model.py:204-205)."""
-    x = F_.upsample_linear_d(features, int(features.shape[1] * upscale))
+    with F_.range_owner(sr_head):
+        x = F_.upsample_linear_d(features, int(features.shape[1] * upscale))
     mods = list(sr_head)
     i = 0
     while i < len(mods):

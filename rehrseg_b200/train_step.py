@@ -241,7 +241,8 @@ class GraphedJointStep:
 
     def __init__(self, model_seg: nn.Module, example_batch: Sequence[torch.Tensor], loss_obj_lr_seg: nn.Module,
                  loss_obj_hr_seg: nn.Module, model_sr: Optional[nn.Module] = None, distiller: Optional[nn.Module] = None,
-                 enable_uncertainty: bool = True, dp_group=None, teacher_keys: Optional[Sequence[int]] = None):
+                 enable_uncertainty: bool = True, dp_group=None, teacher_keys: Optional[Sequence[int]] = None,
+                 range_check: bool = False):
         from .graphs import GraphedTrainStep
         device = next(model_seg.parameters()).device
         model_seg.train()
@@ -273,7 +274,11 @@ class GraphedJointStep:
             return loss
 
         self.module = _JointGraphModule(model_seg, distiller if distill else None, model_sr if distill else None)
-        self.step = GraphedTrainStep(self.module, loss_fn, tuple(example_batch), dp_group=dp_group)
+        self.step = GraphedTrainStep(self.module, loss_fn, tuple(example_batch), dp_group=dp_group, range_check=range_check)
+
+    def range_report(self):
+        """fp16 saturation of the last replay's student forward (`range_check=True`; names are prefixed `model_seg.`)."""
+        return self.step.range_report()
 
     def __call__(self, batch: Sequence[torch.Tensor]) -> dict:
         self.step.load(*batch)
@@ -373,7 +378,7 @@ class GraphedSRStep:
 
     def __init__(self, model: nn.Module, example_batch: Sequence[torch.Tensor], loss_obj: Optional[nn.Module] = None,
                  loss_seg: Optional[nn.Module] = None, slice_separation: int = 4, num_slices: int = 4, enable_uncertainty: bool = False,
-                 fused_loss: Optional[nn.Module] = None, dp_group=None):
+                 fused_loss: Optional[nn.Module] = None, dp_group=None, range_check: bool = False):
         from .graphs import GraphedTrainStep
         if fused_loss is None and (loss_obj is None or loss_seg is None):
             raise ValueError("GraphedSRStep needs either fused_loss or both loss_obj and loss_seg")
@@ -381,7 +386,12 @@ class GraphedSRStep:
         def loss_fn(out, patches_hr):
             return _sr_loss(out, patches_hr, loss_obj, loss_seg, slice_separation, num_slices, enable_uncertainty, fused_loss)
 
-        self.step = GraphedTrainStep(model, loss_fn, tuple(example_batch), dp_group=dp_group)
+        self.step = GraphedTrainStep(model, loss_fn, tuple(example_batch), dp_group=dp_group, range_check=range_check)
+
+    def range_report(self):
+        """fp16 saturation records of the last replay (`range_check=True`).  The FLAVR network stores its activations in bf16,
+        so its report is empty."""
+        return self.step.range_report()
 
     def __call__(self, batch: Sequence[torch.Tensor]) -> dict:
         self.step.load(*batch)
